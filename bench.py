@@ -4,10 +4,12 @@
 
   python bench.py --gpus N --steps K --warmup W            our CUDA path (one rank per GPU under torchrun)
   python bench.py --impl reference --steps K --warmup W    the reference algorithm on the host cores
+  python bench.py ... --dump-outputs DIR                   also write the last timed step's results as DIR/<name>.npy
 
 A step is one pass of the hot path over this rank's shard of the synthetic catalogue
 (BASELINE.json configs[1]: 10 000 DR12Q-shaped quasars per GPU, single-DLA model, k = 20,
-10 000 samples, 3 Lyman lines).  Prints ONE JSON line on rank 0.
+10 000 samples, 3 Lyman lines).  The inputs are seeded, so two builds given the same arguments see the same
+catalogue and their dumped outputs can be compared array by array.  Prints ONE JSON line on rank 0.
 """
 import argparse
 import json
@@ -20,6 +22,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # the source tree may be read-only: leave no bytecode caches in it
 sys.path.insert(0, ROOT)
 
 METRIC = "qso_spectra_per_sec_10k_dla_samples"
@@ -163,6 +166,25 @@ def spot_check(proc, model, samples, prior, spectra, timed_out, nq, threads):
     return nq / dt, dt, block
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out, path):
+    """Write the arrays a caller of the timed path receives (CUDA tensors, one row per quasar) as path/<name>.npy in
+    float64; map_inds (int64 sample indices < 2^53) converts exactly.  When all rows together exceed
+    DUMP_LIMIT_BYTES, a fixed seeded sample of rows is written instead, with its row numbers in sampled_quasars.npy."""
+    host = {name: t.cpu().numpy().astype(np.float64) for name, t in out.items()}
+    Q = len(next(iter(host.values())))
+    keep = DUMP_LIMIT_BYTES // (sum(a[:1].nbytes for a in host.values()) + 8)   # + 8: the row number
+    os.makedirs(path, exist_ok=True)
+    if Q > keep:
+        rows = np.sort(np.random.default_rng(0).choice(Q, size=keep, replace=False))
+        host = {name: a[rows] for name, a in host.items()}
+        host["sampled_quasars"] = rows.astype(np.float64)
+    for name, a in host.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -180,7 +202,14 @@ def main():
     ap.add_argument("--strong-steps", type=int, default=1,
                     help="timed passes of the strong-scaling leg (configs[2]: 162 861 quasars split over the ranks); 0 = skip")
     ap.add_argument("--catalog-quasars", type=int, default=162861, help="size of the full catalogue (configs[2])")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the results of the last one (rank 0's shard) as DIR/<name>.npy, "
+                         "float64, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the CUDA path")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -253,6 +282,8 @@ def main():
     ms, out, launches, k_ms, k_n = timed_device(proc, dtens, args.steps)
     clocks = sampler.stop() if sampler else None
     value = world * Q * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
 
     # ---- end to end through the public API: pinned host buffers in, host results out, every step
     hnp = {k: v.numpy() for k, v in host.items()}

@@ -7,7 +7,6 @@ import math
 import os
 
 import numpy as np
-import pytest
 
 from oracle import process_qsos_oracle as O
 from oracle import ref as R
@@ -52,8 +51,17 @@ def test_voigt_matches_golden_reference_vectors(golden_dir):
         assert np.max(np.abs(a - g["profile_%d" % i])) <= 4 * ULP
 
 
-@pytest.mark.skipif(not R.have_ref(), reason="oracle/_ref/voigt_ref.so not built (needs /root/reference)")
-def test_voigt_matches_compiled_reference():
+def test_voigt_matches_compiled_reference(golden_dir):
+    """Both restatements (Python and oracle/c) against the reference's own voigt.c: the profiles the compiled reference
+    computed on the stored cases (tests/golden/voigt_reference.npz, written by tests/golden/make_golden.py), and, where
+    oracle/_ref/voigt_ref.so has been built from the reference's source, 20 random profiles computed now."""
+    g = np.load(os.path.join(golden_dir, "voigt_reference.npz"))
+    for i, (z, N, nl) in enumerate(g["cases"]):
+        lam = g["lambdas"] if z < 3.5 else g["lambdas_hi"]
+        for voigt in (O.voigt, R.c_voigt):
+            assert np.max(np.abs(voigt(lam, z, N, int(nl)) - g["profile_%d" % i])) <= 4 * ULP, (voigt.__name__, i)
+    if not R.have_ref():
+        return
     lam = boss_grid()
     rng = np.random.default_rng(0)
     for _ in range(20):
