@@ -103,6 +103,12 @@ SYMBOLS = {
                            + [ctypes.POINTER(GpdlaPreloadParams), ctypes.c_int64] + [ctypes.c_void_p] * 7),
     "gpdla_preload_qsos_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64] + [ctypes.c_void_p] * 7
                                   + [ctypes.POINTER(GpdlaPreloadParams), ctypes.c_int64] + [ctypes.c_void_p] * 8),
+    "gpdla_training_set": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64] + [ctypes.c_void_p] * 7
+                           + [ctypes.c_int32, ctypes.c_double, ctypes.c_double] + [ctypes.c_void_p] * 6),
+    "gpdla_training_set_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64] + [ctypes.c_void_p] * 7
+                                  + [ctypes.c_int32, ctypes.c_double, ctypes.c_double] + [ctypes.c_void_p] * 7),
+    "gpdla_pairwise_covariance": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int32] + [ctypes.c_void_p] * 3),
+    "gpdla_pairwise_covariance_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int32] + [ctypes.c_void_p] * 4),
 }
 
 _lib = None

@@ -18,7 +18,7 @@ from typing import Dict, Optional, Sequence
 import numpy as np
 
 from . import _lib
-from .params import DEFAULT, Parameters
+from .params import DEFAULT, Parameters, lya_wavelength
 
 RESULT_NAMES = ["min_z_dlas", "max_z_dlas", "log_priors_no_dla", "log_priors_dla", "log_likelihoods_no_dla",
                 "log_likelihoods_dla", "log_posteriors_no_dla", "log_posteriors_dla", "model_posteriors",
@@ -408,7 +408,8 @@ def objective(x, centered_rest_fluxes, lya_1pzs, rest_noise_variances, device: i
 
 class TrainingObjective:
     """The training matrices of learn_qso_model.m:36-75 resident on one GPU; ``ev(x) -> (f, g)`` evaluates
-    objective.m for a parameter vector (what minFunc calls at learn_qso_model.m:97-99), uploading only ``x``."""
+    objective.m for a parameter vector (what minFunc calls at learn_qso_model.m:97-99), uploading only ``x``.
+    The matrices are host arrays (uploaded once) or contiguous float64 CUDA tensors on ``device`` (used in place)."""
 
     def __init__(self, centered_rest_fluxes, lya_1pzs, rest_noise_variances, k: int, device: int = 0,
                  num_forest_lines: int = 0, all_transition_wavelengths=None, all_oscillator_strengths=None):
@@ -418,10 +419,21 @@ class TrainingObjective:
         self._lib = _lib.load()
         self._torch = torch
         self.dev = torch.device("cuda", device)
-        self.N, self.P = np.shape(centered_rest_fluxes)
         self.k = int(k)
-        up = lambda a: torch.from_numpy(_f64(a)).to(self.dev)
-        self.y, self.z1, self.nv = up(centered_rest_fluxes), up(lya_1pzs), up(rest_noise_variances)
+        cuda_in = [torch.is_tensor(a) and a.is_cuda for a in (centered_rest_fluxes, lya_1pzs, rest_noise_variances)]
+        if any(cuda_in):
+            # device-resident matrices (e.g. from training_set_device) are kept as they are, without a copy
+            mats = (centered_rest_fluxes, lya_1pzs, rest_noise_variances)
+            if not all(cuda_in) or any(a.dtype != torch.float64 or not a.is_contiguous() or a.device != self.dev
+                                       or a.dim() != 2 or a.shape != mats[0].shape for a in mats):
+                raise ValueError("CUDA training matrices must be three contiguous float64 tensors of one (N, P) shape "
+                                 "on %s" % self.dev)
+            self.N, self.P = tuple(centered_rest_fluxes.shape)
+            self.y, self.z1, self.nv = mats
+        else:
+            self.N, self.P = np.shape(centered_rest_fluxes)
+            up = lambda a: torch.from_numpy(_f64(a)).to(self.dev)
+            self.y, self.z1, self.nv = up(centered_rest_fluxes), up(lya_1pzs), up(rest_noise_variances)
         self.nx = self.P * (self.k + 1) + 3
         self.x = torch.empty(self.nx, dtype=torch.float64, device=self.dev)
         self.g = torch.empty(self.nx, dtype=torch.float64, device=self.dev)
@@ -459,6 +471,170 @@ def learn_qso_model(centered_rest_fluxes, lya_1pzs, rest_noise_variances, initia
     finally:
         ev.close()
     return res.x, float(res.fun), res
+
+
+# ---------------------------------------------------------------- training set + PCA initialisation
+def rest_wavelengths(params: Parameters = DEFAULT) -> np.ndarray:
+    """The model grid min_lambda:dlambda:max_lambda (learn_qso_model.m:29): 911.75:0.25:1215.75, 1217 exact values."""
+    n = int(round((params.max_lambda - params.min_lambda) / params.dlambda)) + 1
+    return params.min_lambda + params.dlambda * np.arange(n)
+
+
+def _check_observed(num_observed: np.ndarray, rest: np.ndarray):
+    """nanmean / nanstd of a rest pixel need two observations (learn_qso_model.m:71-95)."""
+    few = np.flatnonzero(num_observed < 2)
+    if few.size:
+        p = int(few[0])
+        raise ValueError("rest wavelength %.2f A is observed in %d training spectra; every rest pixel needs at least 2 "
+                         "(%d pixels fall short)" % (rest[p], int(num_observed[p]), few.size))
+
+
+def _initial_x(cov: np.ndarray, std_dev: np.ndarray, k: int, rest: np.ndarray, params: Parameters) -> np.ndarray:
+    """learn_qso_model.m:82-95: the top-k principal axes of the pairwise covariance scaled by sqrt(latent), pca's sign
+    convention (largest |entry| of each axis positive, first on ties), then log nanstd and the initial c_0, tau_0, beta:
+    ``initial_x = [initial_M(:); initial_log_omega; log c_0; log tau_0; log beta]``.  The P x P eigendecomposition runs
+    on the host (numpy eigh)."""
+    P = cov.shape[0]
+    if not 1 <= k < P:
+        raise ValueError("k must lie in [1, %d)" % P)
+    bad = np.argwhere(np.isnan(cov))
+    if bad.size:
+        p, q = bad[0]
+        raise ValueError("pairwise covariance is undefined at rest wavelengths %.2f / %.2f A: fewer than 2 training "
+                         "spectra observe both" % (rest[p], rest[q]))
+    latent, coeff = np.linalg.eigh(cov)
+    order = np.arange(P)[::-1][:k]                                     # descending
+    latent, coeff = latent[order], coeff[:, order]
+    if np.any(latent <= 0):
+        raise ValueError("the top %d eigenvalues of the pairwise covariance must be positive (smallest: %.3e)"
+                         % (k, latent.min()))
+    big = np.argmax(np.abs(coeff), axis=0)
+    coeff = coeff * np.where(coeff[big, np.arange(k)] < 0, -1.0, 1.0)
+    initial_M = coeff * np.sqrt(latent)
+    return np.concatenate([initial_M.T.ravel(), np.log(std_dev),
+                           [np.log(params.initial_c_0), np.log(params.initial_tau_0), np.log(params.initial_beta)]])
+
+
+def pairwise_covariance(X, device: int = 0):
+    """The covariance ``pca(X, 'rows', 'pairwise')`` decomposes (learn_qso_model.m:82-95) on the GPU: ``X`` [N x P]
+    with NaN = not observed -> ``(cov, counts)``, [P x P] each; ``cov`` is NaN where fewer than 2 rows observe a pair."""
+    import torch
+    lib = _lib.load()
+    X = _f64(X)
+    if X.ndim != 2:
+        raise ValueError("X must be a 2-D (N, P) array")
+    N, P = X.shape
+    cov, counts = np.empty((P, P)), np.empty((P, P), dtype=np.int32)
+    vp = lambda a: ctypes.c_void_p(a.ctypes.data)
+    with torch.cuda.device(device):
+        _lib.check(lib.gpdla_pairwise_covariance(N, P, vp(X), vp(cov), vp(counts)))
+    return cov, counts
+
+
+def training_set(spectra: Dict, k: int, params: Parameters = DEFAULT, device: int = 0) -> Dict[str, np.ndarray]:
+    """The training matrices of learn_qso_model.m:36-75 and the PCA starting point of :82-95 on the GPU, host arrays in
+    and out.  ``spectra``: the ragged lists of ``preload_qsos`` or the padded planes (``wavelengths``, ``flux``,
+    ``noise_variance``, ``pixel_mask``, ``lengths``), plus ``z_qsos``, for the training selection.  Returns
+    ``rest_wavelengths``, ``lya_1pzs``, ``centered_rest_fluxes``, ``rest_noise_variances`` ([N x P]), ``mu``,
+    ``std_dev``, ``num_observed`` ([P]) and ``initial_x`` -- the arguments of ``learn_qso_model``."""
+    import torch
+    lib = _lib.load()
+    sp = pad_spectra(spectra)
+    W, F, V = _f64(sp["wavelengths"]), _f64(sp["flux"]), _f64(sp["noise_variance"])
+    Mk = np.ascontiguousarray(sp["pixel_mask"], dtype=np.uint8)
+    lengths = np.ascontiguousarray(sp["lengths"], dtype=np.int32).ravel()
+    z = _f64(sp["z_qsos"]).ravel()
+    _check_planes(W, F, V, Mk, lengths, z)
+    N, L_max = W.shape
+    rest = rest_wavelengths(params)
+    P = rest.size
+    out = dict(rest_wavelengths=rest, lya_1pzs=np.empty((N, P)), centered_rest_fluxes=np.empty((N, P)),
+               rest_noise_variances=np.empty((N, P)), mu=np.empty(P), std_dev=np.empty(P),
+               num_observed=np.full(P, np.iinfo(np.int32).max, dtype=np.int32))
+    vp = lambda a: ctypes.c_void_p(a.ctypes.data)
+    cov, counts = np.empty((P, P)), np.empty((P, P), dtype=np.int32)
+    with torch.cuda.device(device):
+        rc = lib.gpdla_training_set(N, L_max, vp(W), vp(F), vp(V), vp(Mk), vp(lengths), vp(z), vp(rest), P,
+                                    lya_wavelength, float(params.max_noise_variance), vp(out["lya_1pzs"]),
+                                    vp(out["centered_rest_fluxes"]), vp(out["rest_noise_variances"]), vp(out["mu"]),
+                                    vp(out["std_dev"]), vp(out["num_observed"]))
+        if rc == _lib.GPDLA_ERR_INVALID:
+            _check_observed(out["num_observed"], rest)
+        _lib.check(rc)
+        _lib.check(lib.gpdla_pairwise_covariance(N, P, vp(out["centered_rest_fluxes"]), vp(cov), vp(counts)))
+    out["initial_x"] = _initial_x(cov, out["std_dev"], int(k), rest, params)
+    return out
+
+
+def training_set_device(wavelengths, flux, noise_variance, pixel_mask, lengths, z_qsos, k: int,
+                        params: Parameters = DEFAULT) -> Dict:
+    """Device-resident ``training_set``: the CUDA tensors ``preload_qsos_device`` returns (float64 [N x L_max] planes,
+    uint8 mask, int32 lengths -- a negative or zero length gives an all-NaN row -- and float64 ``z_qsos``) in, the same
+    names as CUDA tensors out (``initial_x`` on the host).  Only the [P x P] covariance, ``std_dev`` and
+    ``num_observed`` cross to the host, for the eigendecomposition."""
+    import torch
+    lib = _lib.load()
+    dev = wavelengths.device
+    N, L_max = wavelengths.shape
+    for t, dt in ((wavelengths, torch.float64), (flux, torch.float64), (noise_variance, torch.float64),
+                  (pixel_mask, torch.uint8), (lengths, torch.int32), (z_qsos, torch.float64)):
+        if not (t.is_cuda and t.device == dev and t.dtype == dt and t.is_contiguous()):
+            raise ValueError("training_set_device takes contiguous CUDA tensors on one device: float64 planes, uint8 "
+                             "pixel_mask, int32 lengths, float64 z_qsos")
+    if any(t.shape != wavelengths.shape for t in (flux, noise_variance, pixel_mask)) or \
+            lengths.shape != (N,) or z_qsos.shape != (N,):
+        raise ValueError("wavelengths, flux, noise_variance and pixel_mask must share one (N, L_max) shape and lengths, "
+                         "z_qsos have one entry per spectrum")
+    rest = rest_wavelengths(params)
+    P = rest.size
+    f64 = dict(dtype=torch.float64, device=dev)
+    out = dict(rest_wavelengths=torch.from_numpy(rest).to(dev), lya_1pzs=torch.empty((N, P), **f64),
+               centered_rest_fluxes=torch.empty((N, P), **f64), rest_noise_variances=torch.empty((N, P), **f64),
+               mu=torch.empty(P, **f64), std_dev=torch.empty(P, **f64),
+               num_observed=torch.empty(P, dtype=torch.int32, device=dev))
+    cov = torch.empty((P, P), **f64)
+    counts = torch.empty((P, P), dtype=torch.int32, device=dev)
+    ptr = lambda t: ctypes.c_void_p(t.data_ptr())
+    with torch.cuda.device(dev):
+        stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _lib.check(lib.gpdla_training_set_device(
+            N, L_max, ptr(wavelengths), ptr(flux), ptr(noise_variance), ptr(pixel_mask), ptr(lengths), ptr(z_qsos),
+            ptr(out["rest_wavelengths"]), P, lya_wavelength, float(params.max_noise_variance), ptr(out["lya_1pzs"]),
+            ptr(out["centered_rest_fluxes"]), ptr(out["rest_noise_variances"]), ptr(out["mu"]), ptr(out["std_dev"]),
+            ptr(out["num_observed"]), stream))
+        _lib.check(lib.gpdla_pairwise_covariance_device(N, P, ptr(out["centered_rest_fluxes"]), ptr(cov), ptr(counts),
+                                                        stream))
+        num_observed = out["num_observed"].cpu().numpy()
+        _check_observed(num_observed, rest)
+        out["initial_x"] = _initial_x(cov.cpu().numpy(), out["std_dev"].cpu().numpy(), int(k), rest, params)
+    return out
+
+
+def learn_qso_model_from_spectra(spectra: Dict, k: int, params: Parameters = DEFAULT, max_iter: int = 2000,
+                                 device: int = 0) -> Dict:
+    """learn_qso_model.m:36-110 from preprocessed training spectra (ragged or padded, plus ``z_qsos``): the training
+    set and PCA starting point (``training_set_device``), L-BFGS on the GPU objective (``learn_qso_model``) and the
+    unpacking of :101-110.  Returns the model ``DLAProcessor`` takes -- ``rest_wavelengths``, ``mu``, ``M`` (P x k),
+    ``log_omega``, ``log_c_0``, ``log_tau_0``, ``log_beta`` -- plus ``initial_x``, ``log_likelihood`` (the objective
+    value at the optimum, the negative log-likelihood that learn_qso_model.m stores under this name) and the SciPy
+    ``result``."""
+    import torch
+    sp = pad_spectra(spectra)
+    W, F, V = _f64(sp["wavelengths"]), _f64(sp["flux"]), _f64(sp["noise_variance"])
+    Mk = np.ascontiguousarray(sp["pixel_mask"], dtype=np.uint8)
+    lengths = np.ascontiguousarray(sp["lengths"], dtype=np.int32).ravel()
+    z = _f64(sp["z_qsos"]).ravel()
+    _check_planes(W, F, V, Mk, lengths, z)
+    dev = torch.device("cuda", device)
+    up = lambda a: torch.from_numpy(a).to(dev)
+    ts = training_set_device(up(W), up(F), up(V), up(Mk), up(lengths), up(z), k, params)
+    x, f, res = learn_qso_model(ts["centered_rest_fluxes"], ts["lya_1pzs"], ts["rest_noise_variances"],
+                                ts["initial_x"], k, max_iter, device)
+    P = ts["mu"].numel()
+    return dict(rest_wavelengths=ts["rest_wavelengths"].cpu().numpy(), mu=ts["mu"].cpu().numpy(),
+                M=np.ascontiguousarray(x[:P * k].reshape(k, P).T), log_omega=x[P * k:P * (k + 1)].copy(),
+                log_c_0=float(x[-3]), log_tau_0=float(x[-2]), log_beta=float(x[-1]),
+                initial_x=ts["initial_x"], log_likelihood=f, result=res)
 
 
 def matlab_default_rand(n: int) -> np.ndarray:

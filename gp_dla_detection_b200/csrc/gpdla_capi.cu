@@ -19,6 +19,7 @@
 #include "gpdla_i8_kernels.cuh"
 #include "gpdla_preload.cuh"
 #include "gpdla_objective.cuh"
+#include "gpdla_training.cuh"
 #include "gpdla_rest_table.h"
 
 using namespace gpdla;
@@ -1550,6 +1551,211 @@ int gpdla_objective(int64_t num_quasars, int32_t num_pixels, int32_t k, const do
                     const double* lya_1pzs, const double* rest_noise_variances, const double* x, double* f, double* g) {
   return gpdla_objective_lyseries(num_quasars, num_pixels, k, centered_rest_fluxes, lya_1pzs, rest_noise_variances, 0, nullptr,
                                   nullptr, x, f, g);
+}
+
+// ---- training set + pairwise covariance (learn_qso_model.m:36-95) ----
+
+// rows of X per split of the covariance: a function of N alone, so that the summation order (and the bits) do not depend
+// on the device; up to 8 splits give 210 x 8 CTAs for the 1217-pixel grid
+static int64_t cov_rows_per_split(int64_t N) {
+  const int64_t nsplit = std::min<int64_t>(8, std::max<int64_t>(1, (N + 2047) / 2048));
+  return std::max<int64_t>(COV_CHUNK, ((N + nsplit - 1) / nsplit + COV_CHUNK - 1) / COV_CHUNK * COV_CHUNK);
+}
+
+// one column statistic of an [N x P] matrix: fixed row blocks, then their sum in block order
+static int column_stat(double* X, int64_t N, int P, int mode, const double* centre, double* out, int32_t* count,
+                       cudaStream_t st) {
+  const int nblocks = (int)((N + COL_ROWS - 1) / COL_ROWS);
+  double* psum = nullptr;
+  int32_t* pcnt = nullptr;
+  if (nblocks > 0) {
+    CUDA_TRY(cudaMallocAsync(&psum, (size_t)nblocks * P * (sizeof(double) + sizeof(int32_t)), st), g_err);
+    pcnt = reinterpret_cast<int32_t*>(psum + (size_t)nblocks * P);
+    column_partial_kernel<<<dim3((P + COL_THREADS - 1) / COL_THREADS, nblocks), COL_THREADS, 0, st>>>(X, N, P, mode, centre,
+                                                                                                     psum, pcnt);
+  }
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) {
+    column_finish_kernel<<<(P + 127) / 128, 128, 0, st>>>(psum, pcnt, nblocks, P, mode, out, count);
+    e = cudaGetLastError();
+  }
+  if (psum) {                                     // freed on the error path too
+    const cudaError_t ef = cudaFreeAsync(psum, st);
+    if (e == cudaSuccess) e = ef;
+  }
+  if (e != cudaSuccess) { g_err = std::string("column_stat: ") + cudaGetErrorString(e); return GPDLA_ERR_CUDA; }
+  return GPDLA_OK;
+}
+
+int gpdla_training_set_device(int64_t N, int64_t L_max, const double* wavelengths, const double* flux,
+                              const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                              const double* z_qsos, const double* rest_wavelengths, int32_t num_pixels,
+                              double lya_wavelength, double max_noise_variance, double* lya_1pzs,
+                              double* centered_rest_fluxes, double* rest_noise_variances, double* mu, double* std_dev,
+                              int32_t* num_observed, void* stream) {
+  if (N < 0 || N > INT32_MAX || L_max < 1 || num_pixels < 1 || !rest_wavelengths || !mu || !std_dev || !num_observed ||
+      !(lya_wavelength > 0.0) ||
+      (N > 0 && (!wavelengths || !flux || !noise_variance || !pixel_mask || !lengths || !z_qsos || !lya_1pzs ||
+                 !centered_rest_fluxes || !rest_noise_variances))) {
+    g_err = "gpdla_training_set_device: invalid arguments";
+    return GPDLA_ERR_INVALID;
+  }
+  const size_t smem = training_set_smem_bytes(L_max);
+  int dev = 0, optin = 0;
+  CUDA_TRY(cudaGetDevice(&dev), g_err);
+  CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev), g_err);
+  if (smem > (size_t)optin) {
+    g_err = "gpdla_training_set_device: L_max = " + std::to_string(L_max) + " does not fit in shared memory (at most " +
+            std::to_string(optin / 32) + " pixels)";
+    return GPDLA_ERR_INVALID;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  if (N > 0) {
+    TrainingArgs a;
+    a.wavelengths = wavelengths; a.flux = flux; a.noise_variance = noise_variance; a.pixel_mask = pixel_mask;
+    a.lengths = lengths; a.z_qsos = z_qsos; a.rest = rest_wavelengths; a.N = N; a.L_max = L_max; a.P = num_pixels;
+    a.lya_wavelength = lya_wavelength; a.max_noise_variance = max_noise_variance;
+    a.lya_1pzs = lya_1pzs; a.rest_fluxes = centered_rest_fluxes; a.rest_noise_variances = rest_noise_variances;
+    CUDA_TRY(cudaFuncSetAttribute(training_set_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), g_err);
+    training_set_kernel<<<(unsigned)N, TS_THREADS, smem, st>>>(a);
+    CUDA_TRY(cudaGetLastError(), g_err);
+  }
+  int rc;
+  // mu = nanmean(rest_fluxes), centred in place (:71-75); std_dev = nanstd of the centred fluxes (:82-95), whose own
+  // nanmean is kept in std_dev until the last pass overwrites it
+  if ((rc = column_stat(centered_rest_fluxes, N, num_pixels, COL_MEAN, nullptr, mu, num_observed, st))) return rc;
+  if ((rc = column_stat(centered_rest_fluxes, N, num_pixels, COL_CENTRE, mu, std_dev, nullptr, st))) return rc;
+  if ((rc = column_stat(centered_rest_fluxes, N, num_pixels, COL_SQDEV, std_dev, std_dev, nullptr, st))) return rc;
+  return GPDLA_OK;
+}
+
+int gpdla_training_set(int64_t N, int64_t L_max, const double* wavelengths, const double* flux,
+                       const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                       const double* z_qsos, const double* rest_wavelengths, int32_t num_pixels, double lya_wavelength,
+                       double max_noise_variance, double* lya_1pzs, double* centered_rest_fluxes,
+                       double* rest_noise_variances, double* mu, double* std_dev, int32_t* num_observed) {
+  if (N < 0 || N > INT32_MAX || L_max < 1 || num_pixels < 1 || !rest_wavelengths || !mu || !std_dev || !num_observed ||
+      (N > 0 && (!wavelengths || !flux || !noise_variance || !pixel_mask || !lengths || !z_qsos || !lya_1pzs ||
+                 !centered_rest_fluxes || !rest_noise_variances))) {
+    g_err = "gpdla_training_set: invalid arguments";
+    return GPDLA_ERR_INVALID;
+  }
+  for (int64_t i = 0; i < N; ++i)
+    if (lengths[i] < 0 || lengths[i] > L_max) {
+      g_err = "gpdla_training_set: lengths[" + std::to_string(i) + "] = " + std::to_string(lengths[i]) +
+              " is outside [0, L_max = " + std::to_string(L_max) + "]";
+      return GPDLA_ERR_INVALID;
+    }
+  for (int32_t p = 1; p < num_pixels; ++p)
+    if (!(rest_wavelengths[p] > rest_wavelengths[p - 1])) {
+      g_err = "gpdla_training_set: rest_wavelengths must be strictly increasing (entry " + std::to_string(p) + ")";
+      return GPDLA_ERR_INVALID;
+    }
+  const size_t NL = (size_t)N * L_max, NP = (size_t)N * num_pixels, P = (size_t)num_pixels;
+  const size_t bytes = 3 * NL * 8 + NL + N * (4 + 8) + P * 8 + 3 * NP * 8 + 2 * P * 8 + P * 4 + 256;
+  char* base = nullptr;
+  CUDA_TRY(cudaMalloc(&base, bytes), g_err);
+  char* ptr = base;
+  auto take = [&](size_t n) { char* r = ptr; ptr += (n + 15) / 16 * 16; return r; };
+  double* d_w = (double*)take(NL * 8); double* d_f = (double*)take(NL * 8); double* d_v = (double*)take(NL * 8);
+  double* d_z = (double*)take((size_t)N * 8); double* d_rest = (double*)take(P * 8);
+  double* d_lya = (double*)take(NP * 8); double* d_y = (double*)take(NP * 8); double* d_nv = (double*)take(NP * 8);
+  double* d_mu = (double*)take(P * 8); double* d_sd = (double*)take(P * 8);
+  int32_t* d_len = (int32_t*)take((size_t)N * 4); int32_t* d_cnt = (int32_t*)take(P * 4);
+  uint8_t* d_m = (uint8_t*)take(NL);
+  cudaError_t e = cudaSuccess;
+  auto up = [&](void* d, const void* h, size_t n) { if (e == cudaSuccess && n) e = cudaMemcpy(d, h, n, cudaMemcpyHostToDevice); };
+  auto down = [&](void* h, const void* d, size_t n) { if (e == cudaSuccess && n) e = cudaMemcpy(h, d, n, cudaMemcpyDeviceToHost); };
+  up(d_w, wavelengths, NL * 8); up(d_f, flux, NL * 8); up(d_v, noise_variance, NL * 8); up(d_m, pixel_mask, NL);
+  up(d_len, lengths, (size_t)N * 4); up(d_z, z_qsos, (size_t)N * 8); up(d_rest, rest_wavelengths, P * 8);
+  int rc = GPDLA_ERR_CUDA;
+  if (e == cudaSuccess) {
+    rc = gpdla_training_set_device(N, L_max, d_w, d_f, d_v, d_m, d_len, d_z, d_rest, num_pixels, lya_wavelength,
+                                   max_noise_variance, d_lya, d_y, d_nv, d_mu, d_sd, d_cnt, nullptr);
+    if (rc == GPDLA_OK) {
+      down(lya_1pzs, d_lya, NP * 8); down(centered_rest_fluxes, d_y, NP * 8); down(rest_noise_variances, d_nv, NP * 8);
+      down(mu, d_mu, P * 8); down(std_dev, d_sd, P * 8); down(num_observed, d_cnt, P * 4);
+      if (e == cudaSuccess) {
+        for (int32_t p = 0; p < num_pixels; ++p)
+          if (num_observed[p] < 2) {
+            char buf[256];
+            snprintf(buf, sizeof buf, "gpdla_training_set: rest pixel %d (%.2f A) is observed in %d spectra, fewer than 2",
+                     p, rest_wavelengths[p], num_observed[p]);
+            g_err = buf;
+            rc = GPDLA_ERR_INVALID;
+            break;
+          }
+      }
+    }
+  }
+  if (e != cudaSuccess) { g_err = cudaGetErrorString(e); rc = GPDLA_ERR_CUDA; }
+  cudaFree(base);
+  return rc;
+}
+
+int gpdla_pairwise_covariance_device(int64_t N, int32_t P, const double* X, double* cov, int32_t* counts, void* stream) {
+  if (N < 0 || N > INT32_MAX || P < 1 || !cov || !counts || (N > 0 && !X)) {
+    g_err = "gpdla_pairwise_covariance_device: invalid arguments";
+    return GPDLA_ERR_INVALID;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const int tiles_1d = (P + COV_TILE - 1) / COV_TILE;
+  const int ntile = tiles_1d * (tiles_1d + 1) / 2;
+  const int64_t rps = cov_rows_per_split(N);
+  const int nsplit = (int)std::max<int64_t>(1, (N + rps - 1) / rps);
+  const size_t tile_elems = (size_t)nsplit * ntile * COV_TILE * COV_TILE;
+  double* mean = nullptr;
+  CUDA_TRY(cudaMallocAsync(&mean, (size_t)P * (8 + 4) + tile_elems * (8 + 4) + 64, st), g_err);   // mean, counts, partials
+  int32_t* mcount = reinterpret_cast<int32_t*>(mean + P);
+  double* psum = mean + ((size_t)P + (P + 1) / 2 + 1) / 2 * 2;   // 16-byte aligned: the tile kernel stores double2
+  int32_t* pcnt = reinterpret_cast<int32_t*>(psum + tile_elems);
+  int rc = column_stat(const_cast<double*>(X), N, P, COL_MEAN, nullptr, mean, mcount, st);   // COL_MEAN only reads X
+  cudaError_t e = cudaSuccess;
+  if (rc == GPDLA_OK) {
+    CovArgs a;
+    a.X = X; a.mean = mean; a.N = N; a.P = P; a.ntile = ntile; a.rows_per_split = rps; a.psum = psum; a.pcnt = pcnt;
+    pairwise_cov_tile_kernel<<<dim3(ntile, nsplit), COV_THREADS, 0, st>>>(a);
+    e = cudaGetLastError();
+    if (e == cudaSuccess) {
+      const int64_t PP = (int64_t)P * P;
+      pairwise_cov_finish_kernel<<<(unsigned)((PP + 255) / 256), 256, 0, st>>>(psum, pcnt, nsplit, ntile, P, cov, counts);
+      e = cudaGetLastError();
+    }
+  }
+  const cudaError_t ef = cudaFreeAsync(mean, st);  // freed on the error paths too
+  if (rc != GPDLA_OK) return rc;
+  if (e == cudaSuccess) e = ef;
+  if (e != cudaSuccess) {
+    g_err = std::string("gpdla_pairwise_covariance_device: ") + cudaGetErrorString(e);
+    return GPDLA_ERR_CUDA;
+  }
+  return GPDLA_OK;
+}
+
+int gpdla_pairwise_covariance(int64_t N, int32_t P, const double* X, double* cov, int32_t* counts) {
+  if (N < 0 || N > INT32_MAX || P < 1 || !cov || !counts || (N > 0 && !X)) {
+    g_err = "gpdla_pairwise_covariance: invalid arguments";
+    return GPDLA_ERR_INVALID;
+  }
+  const size_t NP = (size_t)N * P, PP = (size_t)P * P;
+  char* base = nullptr;
+  CUDA_TRY(cudaMalloc(&base, NP * 8 + PP * 12 + 64), g_err);
+  double* d_x = (double*)base;
+  double* d_c = d_x + NP;
+  int32_t* d_n = (int32_t*)(d_c + PP);
+  cudaError_t e = cudaSuccess;
+  if (NP) e = cudaMemcpy(d_x, X, NP * 8, cudaMemcpyHostToDevice);
+  int rc = GPDLA_ERR_CUDA;
+  if (e == cudaSuccess) {
+    rc = gpdla_pairwise_covariance_device(N, P, d_x, d_c, d_n, nullptr);
+    if (rc == GPDLA_OK) {
+      e = cudaMemcpy(cov, d_c, PP * 8, cudaMemcpyDeviceToHost);
+      if (e == cudaSuccess) e = cudaMemcpy(counts, d_n, PP * 4, cudaMemcpyDeviceToHost);
+    }
+  }
+  if (e != cudaSuccess) { g_err = cudaGetErrorString(e); rc = GPDLA_ERR_CUDA; }
+  cudaFree(base);
+  return rc;
 }
 
 }  // extern "C"

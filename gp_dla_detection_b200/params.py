@@ -35,6 +35,10 @@ class Parameters:
     z_qso_cut: float = 2.15                           # :25
     loading_min_lambda: float = 910.0                 # :15
     loading_max_lambda: float = 1217.0                # :16
+    max_noise_variance: float = 1.0 ** 2              # next to k: noisier interpolated pixels leave the training set
+    initial_c_0: float = 0.1                          # :40  starting point of the null-model fit
+    initial_tau_0: float = 0.0023                     # :41
+    initial_beta: float = 3.65                        # :42
 
 
 DEFAULT = Parameters()

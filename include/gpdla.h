@@ -227,6 +227,38 @@ int gpdla_objective_device(int64_t num_quasars, int32_t num_pixels, int32_t k, c
                            const double* lya_1pzs, const double* rest_noise_variances, const double* x, double* f,
                            double* g, void* stream);
 
+/* ---- GP training set on the device: learn_qso_model.m:36-75 (+ the nanstd of :82-95) ----
+ * Inputs are the training spectra in the padded [N x L_max] form of gpdla_process_qsos (observed wavelengths, flux,
+ * noise variance, pixel mask, lengths, z_qsos) and the model grid rest_wavelengths [num_pixels] (strictly increasing).
+ * Per spectrum: emitted wavelengths lambda / (1 + z); flux and noise variance NaN where masked; each of
+ * 1 + (lambda - lya_wavelength) / lya_wavelength, flux and noise variance linearly interpolated (interp1) onto the grid,
+ * NaN outside the spectrum or next to a NaN; every grid point whose interpolated noise variance exceeds
+ * max_noise_variance set to NaN in all three outputs (:66-69).  Outputs: lya_1pzs, centered_rest_fluxes (rest fluxes
+ * minus mu), rest_noise_variances, [N x num_pixels] row-major; per rest pixel mu = nanmean of the rest fluxes,
+ * num_observed = their non-NaN count, std_dev = nanstd (n - 1) of the centred fluxes.  A spectrum with lengths < 2 gives
+ * an all-NaN row.  The host entry checks lengths in [0, L_max] and the grid, and returns GPDLA_ERR_INVALID (outputs
+ * written) if a rest pixel is observed fewer than 2 times.  Context-free; the _device entry is asynchronous on `stream`
+ * and works on the current device. */
+int gpdla_training_set(int64_t N, int64_t L_max, const double* wavelengths, const double* flux,
+                       const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                       const double* z_qsos, const double* rest_wavelengths, int32_t num_pixels,
+                       double lya_wavelength, double max_noise_variance,
+                       double* lya_1pzs, double* centered_rest_fluxes, double* rest_noise_variances,
+                       double* mu, double* std_dev, int32_t* num_observed);
+int gpdla_training_set_device(int64_t N, int64_t L_max, const double* wavelengths, const double* flux,
+                              const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                              const double* z_qsos, const double* rest_wavelengths, int32_t num_pixels,
+                              double lya_wavelength, double max_noise_variance,
+                              double* lya_1pzs, double* centered_rest_fluxes, double* rest_noise_variances,
+                              double* mu, double* std_dev, int32_t* num_observed, void* stream);
+/* The covariance pca(X, 'rows', 'pairwise') decomposes (learn_qso_model.m:82-95): X [N x P] row-major, NaN = not
+ * observed; X~ = X - nanmean(X) column-wise; cov[p, q] = sum over the rows observed in both columns of X~_rp X~_rq,
+ * divided by (counts[p, q] - 1), NaN where counts < 2.  cov, counts: [P x P] row-major, symmetric.  FP64 tensor cores;
+ * every sum has a fixed order, so repeated calls return the same bits.  Context-free; the _device entry is asynchronous on
+ * `stream`. */
+int gpdla_pairwise_covariance(int64_t N, int32_t P, const double* X, double* cov, int32_t* counts);
+int gpdla_pairwise_covariance_device(int64_t N, int32_t P, const double* X, double* cov, int32_t* counts, void* stream);
+
 /* voigt.c:253-304: profile has num_points - 6 entries.  Host buffers; runs on the current device. */
 int gpdla_voigt(const double* lambdas, int64_t num_points, double z, double N, int32_t num_lines, double* profile);
 /* Batched, device buffers: profile[s, :] = voigt(lambdas, z[s], N[s], num_lines), [S x (num_points-6)] */
