@@ -109,6 +109,14 @@ SYMBOLS = {
                                   + [ctypes.c_int32, ctypes.c_double, ctypes.c_double] + [ctypes.c_void_p] * 7),
     "gpdla_pairwise_covariance": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int32] + [ctypes.c_void_p] * 3),
     "gpdla_pairwise_covariance_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int32] + [ctypes.c_void_p] * 4),
+    "gpdla_training_set_lyseries": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64] + [ctypes.c_void_p] * 7
+                                    + [ctypes.c_int32, ctypes.c_double, ctypes.c_double, ctypes.c_int32]
+                                    + [ctypes.c_void_p] * 7),
+    "gpdla_training_set_lyseries_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64] + [ctypes.c_void_p] * 7
+                                           + [ctypes.c_int32, ctypes.c_double, ctypes.c_double, ctypes.c_int32]
+                                           + [ctypes.c_void_p] * 8),
+    "gpdla_row_nanmedian_fill": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int32] + [ctypes.c_void_p] * 2),
+    "gpdla_row_nanmedian_fill_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int32] + [ctypes.c_void_p] * 3),
 }
 
 _lib = None

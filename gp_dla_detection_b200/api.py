@@ -18,7 +18,8 @@ from typing import Dict, Optional, Sequence
 import numpy as np
 
 from . import _lib
-from .params import DEFAULT, Parameters, lya_wavelength
+from . import params as _params
+from .params import DEFAULT, MULTI, Parameters, lya_wavelength
 
 RESULT_NAMES = ["min_z_dlas", "max_z_dlas", "log_priors_no_dla", "log_priors_dla", "log_likelihoods_no_dla",
                 "log_likelihoods_dla", "log_posteriors_no_dla", "log_posteriors_dla", "model_posteriors",
@@ -461,11 +462,15 @@ class TrainingObjective:
 
 
 def learn_qso_model(centered_rest_fluxes, lya_1pzs, rest_noise_variances, initial_x, k: int, max_iter: int = 2000,
-                    device: int = 0):
+                    device: int = 0, num_forest_lines: int = 0, all_transition_wavelengths=None,
+                    all_oscillator_strengths=None):
     """The optimisation of learn_qso_model.m:97-99 (minFunc L-BFGS there, SciPy's L-BFGS-B here) with the objective and
-    gradient evaluated on the GPU.  Returns ``(x, f, scipy_result)``; M = x[:P k].reshape(k, P).T etc. (:101-110)."""
+    gradient evaluated on the GPU.  Returns ``(x, f, scipy_result)``; M = x[:P k].reshape(k, P).T etc. (:101-110).
+    ``num_forest_lines > 0`` with the two Lyman-series tables fits objective_lyseries.m instead
+    (learn_qso_model_meanflux.m:140-142)."""
     from scipy.optimize import minimize
-    ev = TrainingObjective(centered_rest_fluxes, lya_1pzs, rest_noise_variances, k, device)
+    ev = TrainingObjective(centered_rest_fluxes, lya_1pzs, rest_noise_variances, k, device, num_forest_lines,
+                           all_transition_wavelengths, all_oscillator_strengths)
     try:
         res = minimize(lambda v: ev(v), _f64(initial_x), jac=True, method="L-BFGS-B", options={"maxiter": max_iter})
     finally:
@@ -630,6 +635,143 @@ def learn_qso_model_from_spectra(spectra: Dict, k: int, params: Parameters = DEF
     ts = training_set_device(up(W), up(F), up(V), up(Mk), up(lengths), up(z), k, params)
     x, f, res = learn_qso_model(ts["centered_rest_fluxes"], ts["lya_1pzs"], ts["rest_noise_variances"],
                                 ts["initial_x"], k, max_iter, device)
+    P = ts["mu"].numel()
+    return dict(rest_wavelengths=ts["rest_wavelengths"].cpu().numpy(), mu=ts["mu"].cpu().numpy(),
+                M=np.ascontiguousarray(x[:P * k].reshape(k, P).T), log_omega=x[P * k:P * (k + 1)].copy(),
+                log_c_0=float(x[-3]), log_tau_0=float(x[-2]), log_beta=float(x[-1]),
+                initial_x=ts["initial_x"], log_likelihood=f, result=res)
+
+
+# ---------------------------------------------------------------- the multi-DLA (mean-flux) model's training set
+def _check_forest_lines(num_forest_lines) -> int:
+    nl = int(num_forest_lines)
+    if not 0 <= nl <= _lib.MAX_LINES:
+        raise ValueError("num_forest_lines must lie in [0, %d]" % _lib.MAX_LINES)
+    return nl
+
+
+def row_nanmedian_fill(X, device: int = 0) -> np.ndarray:
+    """A copy of ``X`` [N x P] with each row's NaNs replaced by that row's nanmedian (MATLAB's median, ``meanof`` for an
+    even count) on the GPU; an all-NaN row stays NaN.  The matrix learn_qso_model_meanflux.m decomposes with
+    ``pca(..., 'rows', 'complete')``."""
+    import torch
+    lib = _lib.load()
+    X = _f64(X)
+    if X.ndim != 2:
+        raise ValueError("X must be a 2-D (N, P) array")
+    N, P = X.shape
+    out = np.empty((N, P))
+    with torch.cuda.device(device):
+        _lib.check(lib.gpdla_row_nanmedian_fill(N, P, ctypes.c_void_p(X.ctypes.data), ctypes.c_void_p(out.ctypes.data)))
+    return out
+
+
+def training_set_meanflux(spectra: Dict, k: int, params: Parameters = MULTI, num_forest_lines: int = 31,
+                          device: int = 0) -> Dict[str, np.ndarray]:
+    """The training matrices and PCA starting point of multi_dlas/learn_qso_model_meanflux.m on the GPU, host arrays in
+    and out: ``training_set`` with the Lyman-series mean-flux suppression (Kim et al. 2007, fixed prev_tau_0 = 0.0023,
+    prev_beta = 3.65, the first ``num_forest_lines`` members) divided out of the rest fluxes and noise variances, the
+    noise ceiling ``params.max_noise_variance`` (``MULTI``: 3^2), and the PCA of the row-nanmedian-filled centred fluxes
+    (``pca(..., 'rows', 'complete')``).  Returns the names ``training_set`` returns plus ``lya_absorption`` [N x P]."""
+    import torch
+    lib = _lib.load()
+    nl = _check_forest_lines(num_forest_lines)
+    sp = pad_spectra(spectra)
+    W, F, V = _f64(sp["wavelengths"]), _f64(sp["flux"]), _f64(sp["noise_variance"])
+    Mk = np.ascontiguousarray(sp["pixel_mask"], dtype=np.uint8)
+    lengths = np.ascontiguousarray(sp["lengths"], dtype=np.int32).ravel()
+    z = _f64(sp["z_qsos"]).ravel()
+    _check_planes(W, F, V, Mk, lengths, z)
+    N, L_max = W.shape
+    rest = rest_wavelengths(params)
+    P = rest.size
+    out = dict(rest_wavelengths=rest, lya_1pzs=np.empty((N, P)), centered_rest_fluxes=np.empty((N, P)),
+               rest_noise_variances=np.empty((N, P)), lya_absorption=np.empty((N, P)), mu=np.empty(P),
+               std_dev=np.empty(P), num_observed=np.full(P, np.iinfo(np.int32).max, dtype=np.int32))
+    vp = lambda a: ctypes.c_void_p(a.ctypes.data)
+    filled = np.empty((N, P))
+    cov, counts = np.empty((P, P)), np.empty((P, P), dtype=np.int32)
+    with torch.cuda.device(device):
+        rc = lib.gpdla_training_set_lyseries(N, L_max, vp(W), vp(F), vp(V), vp(Mk), vp(lengths), vp(z), vp(rest), P,
+                                             lya_wavelength, float(params.max_noise_variance), nl, vp(out["lya_1pzs"]),
+                                             vp(out["centered_rest_fluxes"]), vp(out["rest_noise_variances"]),
+                                             vp(out["lya_absorption"]), vp(out["mu"]), vp(out["std_dev"]),
+                                             vp(out["num_observed"]))
+        if rc == _lib.GPDLA_ERR_INVALID:
+            _check_observed(out["num_observed"], rest)
+        _lib.check(rc)
+        _lib.check(lib.gpdla_row_nanmedian_fill(N, P, vp(out["centered_rest_fluxes"]), vp(filled)))
+        _lib.check(lib.gpdla_pairwise_covariance(N, P, vp(filled), vp(cov), vp(counts)))
+    out["initial_x"] = _initial_x(cov, out["std_dev"], int(k), rest, params)
+    return out
+
+
+def training_set_meanflux_device(wavelengths, flux, noise_variance, pixel_mask, lengths, z_qsos, k: int,
+                                 params: Parameters = MULTI, num_forest_lines: int = 31) -> Dict:
+    """Device-resident ``training_set_meanflux``: the CUDA tensors ``preload_qsos_device`` returns in, the same names as
+    CUDA tensors out (``initial_x`` on the host).  The filled copy lives only for the covariance; only the [P x P]
+    covariance, ``std_dev`` and ``num_observed`` cross to the host."""
+    import torch
+    lib = _lib.load()
+    nl = _check_forest_lines(num_forest_lines)
+    dev = wavelengths.device
+    N, L_max = wavelengths.shape
+    for t, dt in ((wavelengths, torch.float64), (flux, torch.float64), (noise_variance, torch.float64),
+                  (pixel_mask, torch.uint8), (lengths, torch.int32), (z_qsos, torch.float64)):
+        if not (t.is_cuda and t.device == dev and t.dtype == dt and t.is_contiguous()):
+            raise ValueError("training_set_meanflux_device takes contiguous CUDA tensors on one device: float64 planes, "
+                             "uint8 pixel_mask, int32 lengths, float64 z_qsos")
+    if any(t.shape != wavelengths.shape for t in (flux, noise_variance, pixel_mask)) or \
+            lengths.shape != (N,) or z_qsos.shape != (N,):
+        raise ValueError("wavelengths, flux, noise_variance and pixel_mask must share one (N, L_max) shape and lengths, "
+                         "z_qsos have one entry per spectrum")
+    rest = rest_wavelengths(params)
+    P = rest.size
+    f64 = dict(dtype=torch.float64, device=dev)
+    out = dict(rest_wavelengths=torch.from_numpy(rest).to(dev), lya_1pzs=torch.empty((N, P), **f64),
+               centered_rest_fluxes=torch.empty((N, P), **f64), rest_noise_variances=torch.empty((N, P), **f64),
+               lya_absorption=torch.empty((N, P), **f64), mu=torch.empty(P, **f64), std_dev=torch.empty(P, **f64),
+               num_observed=torch.empty(P, dtype=torch.int32, device=dev))
+    filled = torch.empty((N, P), **f64)
+    cov = torch.empty((P, P), **f64)
+    counts = torch.empty((P, P), dtype=torch.int32, device=dev)
+    ptr = lambda t: ctypes.c_void_p(t.data_ptr())
+    with torch.cuda.device(dev):
+        stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _lib.check(lib.gpdla_training_set_lyseries_device(
+            N, L_max, ptr(wavelengths), ptr(flux), ptr(noise_variance), ptr(pixel_mask), ptr(lengths), ptr(z_qsos),
+            ptr(out["rest_wavelengths"]), P, lya_wavelength, float(params.max_noise_variance), nl, ptr(out["lya_1pzs"]),
+            ptr(out["centered_rest_fluxes"]), ptr(out["rest_noise_variances"]), ptr(out["lya_absorption"]),
+            ptr(out["mu"]), ptr(out["std_dev"]), ptr(out["num_observed"]), stream))
+        _lib.check(lib.gpdla_row_nanmedian_fill_device(N, P, ptr(out["centered_rest_fluxes"]), ptr(filled), stream))
+        _lib.check(lib.gpdla_pairwise_covariance_device(N, P, ptr(filled), ptr(cov), ptr(counts), stream))
+        num_observed = out["num_observed"].cpu().numpy()
+        _check_observed(num_observed, rest)
+        out["initial_x"] = _initial_x(cov.cpu().numpy(), out["std_dev"].cpu().numpy(), int(k), rest, params)
+    return out
+
+
+def learn_qso_model_meanflux_from_spectra(spectra: Dict, k: int, params: Parameters = MULTI, max_iter: int = 2000,
+                                          device: int = 0) -> Dict:
+    """multi_dlas/learn_qso_model_meanflux.m from preprocessed training spectra (ragged or padded, plus ``z_qsos``): the
+    mean-flux training set and its PCA starting point (``training_set_meanflux_device``), L-BFGS on the GPU
+    objective_lyseries with 31 Lyman-series members, and the unpacking of learn_qso_model.m:101-110.  Returns the model
+    ``process_qsos_multiple_dlas_meanflux`` / ``DLAProcessor.process_multi`` load plus ``initial_x``,
+    ``log_likelihood`` and the SciPy ``result``, as ``learn_qso_model_from_spectra`` does."""
+    import torch
+    sp = pad_spectra(spectra)
+    W, F, V = _f64(sp["wavelengths"]), _f64(sp["flux"]), _f64(sp["noise_variance"])
+    Mk = np.ascontiguousarray(sp["pixel_mask"], dtype=np.uint8)
+    lengths = np.ascontiguousarray(sp["lengths"], dtype=np.int32).ravel()
+    z = _f64(sp["z_qsos"]).ravel()
+    _check_planes(W, F, V, Mk, lengths, z)
+    dev = torch.device("cuda", device)
+    up = lambda a: torch.from_numpy(a).to(dev)
+    nl = _params.num_forest_lines
+    ts = training_set_meanflux_device(up(W), up(F), up(V), up(Mk), up(lengths), up(z), k, params, nl)
+    x, f, res = learn_qso_model(ts["centered_rest_fluxes"], ts["lya_1pzs"], ts["rest_noise_variances"],
+                                ts["initial_x"], k, max_iter, device, nl, _params.all_transition_wavelengths,
+                                _params.all_oscillator_strengths)
     P = ts["mu"].numel()
     return dict(rest_wavelengths=ts["rest_wavelengths"].cpu().numpy(), mu=ts["mu"].cpu().numpy(),
                 M=np.ascontiguousarray(x[:P * k].reshape(k, P).T), log_omega=x[P * k:P * (k + 1)].copy(),

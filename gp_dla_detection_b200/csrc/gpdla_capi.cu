@@ -73,6 +73,22 @@ void fill_line_constants(LineConstants* lc) {
   lc->inv_s2s = 1.0 / (sqrt(2.0) * kSigma);
 }
 
+// Lyman-series forest data of the multi-DLA mean-flux suppression: the one table both inference (c_forest) and the
+// mean-flux training set (TrainingArgs::forest) read
+void fill_forest_constants(ForestConstants* fc, int num_forest_lines) {
+  fc->num_forest_lines = num_forest_lines;                // set_parameters_multi.m:76
+  fc->prev_beta = 3.65;                                   // ...meanflux.m:37
+  const double prev_tau_0 = 0.0023;                       // ...meanflux.m:36
+  const double lya_wavelength = 1215.6701, lya_oscillator_strength = 0.416400;
+  for (int l = 0; l < MAX_LINES; ++l) fc->wavelength[l] = kLyman[l].wavelength_cm * 1e8;   // set_parameters_multi.m:77-109
+  for (int l = 0; l < MAX_LINES; ++l) {
+    // tau_0 * lambda_l * f_l / (lambda_1 * f_1) without the tau_0                         ...meanflux.m:255-256
+    fc->tau_ratio[l] = fc->wavelength[l] * kLyman[l].f / (fc->wavelength[0] * kLyman[0].f);
+    // prev_tau_0 * f_l / f_lya * lambda_l / lya_wavelength                               ...meanflux.m:271-273
+    fc->kim_tau[l] = prev_tau_0 * kLyman[l].f / lya_oscillator_strength * fc->wavelength[l] / lya_wavelength;
+  }
+}
+
 thread_local std::string g_err;   // errors of the context-free entry points
 
 #define CUDA_TRY(expr, errstr)                                                              \
@@ -188,17 +204,7 @@ int upload_device_constants(std::string& err) {
   CUDA_TRY(cudaMemcpyToSymbol(c_lines, &lc, sizeof lc), err);
   {  // Lyman-series forest data of the multi-DLA mean-flux suppression
     ForestConstants fc;
-    fc.num_forest_lines = MAX_LINES;                       // set_parameters_multi.m:76
-    fc.prev_beta = 3.65;                                   // ...meanflux.m:37
-    const double prev_tau_0 = 0.0023;                      // ...meanflux.m:36
-    const double lya_wavelength = 1215.6701, lya_oscillator_strength = 0.416400;
-    for (int l = 0; l < MAX_LINES; ++l) fc.wavelength[l] = kLyman[l].wavelength_cm * 1e8;   // set_parameters_multi.m:77-109
-    for (int l = 0; l < MAX_LINES; ++l) {
-      // tau_0 * lambda_l * f_l / (lambda_1 * f_1) without the tau_0                         ...meanflux.m:255-256
-      fc.tau_ratio[l] = fc.wavelength[l] * kLyman[l].f / (fc.wavelength[0] * kLyman[0].f);
-      // prev_tau_0 * f_l / f_lya * lambda_l / lya_wavelength                               ...meanflux.m:271-273
-      fc.kim_tau[l] = prev_tau_0 * kLyman[l].f / lya_oscillator_strength * fc.wavelength[l] / lya_wavelength;
-    }
+    fill_forest_constants(&fc, MAX_LINES);
     CUDA_TRY(cudaMemcpyToSymbol(c_forest, &fc, sizeof fc), err);
   }
   {  // three-line wing tables in velocity units (see tau_sum_3_wing)
@@ -1587,26 +1593,30 @@ static int column_stat(double* X, int64_t N, int P, int mode, const double* cent
   return GPDLA_OK;
 }
 
-int gpdla_training_set_device(int64_t N, int64_t L_max, const double* wavelengths, const double* flux,
-                              const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
-                              const double* z_qsos, const double* rest_wavelengths, int32_t num_pixels,
-                              double lya_wavelength, double max_noise_variance, double* lya_1pzs,
-                              double* centered_rest_fluxes, double* rest_noise_variances, double* mu, double* std_dev,
-                              int32_t* num_observed, void* stream) {
+// The plain (learn_qso_model.m) and the Lyman-series (learn_qso_model_meanflux.m) training set share their checks,
+// buffers and reductions; num_forest_lines < 0 selects the plain kernel, 0..31 the mean-flux one.
+static int training_set_device_impl(const char* fn, int64_t N, int64_t L_max, const double* wavelengths,
+                                    const double* flux, const double* noise_variance, const uint8_t* pixel_mask,
+                                    const int32_t* lengths, const double* z_qsos, const double* rest_wavelengths,
+                                    int32_t num_pixels, double lya_wavelength, double max_noise_variance,
+                                    int32_t num_forest_lines, double* lya_1pzs, double* centered_rest_fluxes,
+                                    double* rest_noise_variances, double* lya_absorption, double* mu, double* std_dev,
+                                    int32_t* num_observed, void* stream) {
   if (N < 0 || N > INT32_MAX || L_max < 1 || num_pixels < 1 || !rest_wavelengths || !mu || !std_dev || !num_observed ||
-      !(lya_wavelength > 0.0) ||
+      !(lya_wavelength > 0.0) || num_forest_lines > MAX_LINES ||
       (N > 0 && (!wavelengths || !flux || !noise_variance || !pixel_mask || !lengths || !z_qsos || !lya_1pzs ||
                  !centered_rest_fluxes || !rest_noise_variances))) {
-    g_err = "gpdla_training_set_device: invalid arguments";
+    g_err = std::string(fn) + ": invalid arguments";
     return GPDLA_ERR_INVALID;
   }
-  const size_t smem = training_set_smem_bytes(L_max);
+  const bool lyseries = num_forest_lines >= 0;
+  const size_t smem = training_set_smem_bytes(L_max, lyseries);
   int dev = 0, optin = 0;
   CUDA_TRY(cudaGetDevice(&dev), g_err);
   CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev), g_err);
   if (smem > (size_t)optin) {
-    g_err = "gpdla_training_set_device: L_max = " + std::to_string(L_max) + " does not fit in shared memory (at most " +
-            std::to_string(optin / 32) + " pixels)";
+    g_err = std::string(fn) + ": L_max = " + std::to_string(L_max) + " does not fit in shared memory (at most " +
+            std::to_string(optin / (smem / L_max)) + " pixels)";
     return GPDLA_ERR_INVALID;
   }
   cudaStream_t st = (cudaStream_t)stream;
@@ -1616,8 +1626,16 @@ int gpdla_training_set_device(int64_t N, int64_t L_max, const double* wavelength
     a.lengths = lengths; a.z_qsos = z_qsos; a.rest = rest_wavelengths; a.N = N; a.L_max = L_max; a.P = num_pixels;
     a.lya_wavelength = lya_wavelength; a.max_noise_variance = max_noise_variance;
     a.lya_1pzs = lya_1pzs; a.rest_fluxes = centered_rest_fluxes; a.rest_noise_variances = rest_noise_variances;
-    CUDA_TRY(cudaFuncSetAttribute(training_set_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), g_err);
-    training_set_kernel<<<(unsigned)N, TS_THREADS, smem, st>>>(a);
+    fill_forest_constants(&a.forest, lyseries ? num_forest_lines : 0);
+    for (int l = 0; l < MAX_LINES; ++l) a.lya_over_wavelength[l] = lya_wavelength / a.forest.wavelength[l];
+    a.lya_absorption = lya_absorption;
+    if (lyseries) {
+      CUDA_TRY(cudaFuncSetAttribute(training_set_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), g_err);
+      training_set_kernel<true><<<(unsigned)N, TS_THREADS, smem, st>>>(a);
+    } else {
+      CUDA_TRY(cudaFuncSetAttribute(training_set_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), g_err);
+      training_set_kernel<false><<<(unsigned)N, TS_THREADS, smem, st>>>(a);
+    }
     CUDA_TRY(cudaGetLastError(), g_err);
   }
   int rc;
@@ -1629,30 +1647,34 @@ int gpdla_training_set_device(int64_t N, int64_t L_max, const double* wavelength
   return GPDLA_OK;
 }
 
-int gpdla_training_set(int64_t N, int64_t L_max, const double* wavelengths, const double* flux,
-                       const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
-                       const double* z_qsos, const double* rest_wavelengths, int32_t num_pixels, double lya_wavelength,
-                       double max_noise_variance, double* lya_1pzs, double* centered_rest_fluxes,
-                       double* rest_noise_variances, double* mu, double* std_dev, int32_t* num_observed) {
+static int training_set_host_impl(const char* fn, int64_t N, int64_t L_max, const double* wavelengths,
+                                  const double* flux, const double* noise_variance, const uint8_t* pixel_mask,
+                                  const int32_t* lengths, const double* z_qsos, const double* rest_wavelengths,
+                                  int32_t num_pixels, double lya_wavelength, double max_noise_variance,
+                                  int32_t num_forest_lines, double* lya_1pzs, double* centered_rest_fluxes,
+                                  double* rest_noise_variances, double* lya_absorption, double* mu, double* std_dev,
+                                  int32_t* num_observed) {
   if (N < 0 || N > INT32_MAX || L_max < 1 || num_pixels < 1 || !rest_wavelengths || !mu || !std_dev || !num_observed ||
+      num_forest_lines > MAX_LINES ||
       (N > 0 && (!wavelengths || !flux || !noise_variance || !pixel_mask || !lengths || !z_qsos || !lya_1pzs ||
                  !centered_rest_fluxes || !rest_noise_variances))) {
-    g_err = "gpdla_training_set: invalid arguments";
+    g_err = std::string(fn) + ": invalid arguments";
     return GPDLA_ERR_INVALID;
   }
   for (int64_t i = 0; i < N; ++i)
     if (lengths[i] < 0 || lengths[i] > L_max) {
-      g_err = "gpdla_training_set: lengths[" + std::to_string(i) + "] = " + std::to_string(lengths[i]) +
+      g_err = std::string(fn) + ": lengths[" + std::to_string(i) + "] = " + std::to_string(lengths[i]) +
               " is outside [0, L_max = " + std::to_string(L_max) + "]";
       return GPDLA_ERR_INVALID;
     }
   for (int32_t p = 1; p < num_pixels; ++p)
     if (!(rest_wavelengths[p] > rest_wavelengths[p - 1])) {
-      g_err = "gpdla_training_set: rest_wavelengths must be strictly increasing (entry " + std::to_string(p) + ")";
+      g_err = std::string(fn) + ": rest_wavelengths must be strictly increasing (entry " + std::to_string(p) + ")";
       return GPDLA_ERR_INVALID;
     }
   const size_t NL = (size_t)N * L_max, NP = (size_t)N * num_pixels, P = (size_t)num_pixels;
-  const size_t bytes = 3 * NL * 8 + NL + N * (4 + 8) + P * 8 + 3 * NP * 8 + 2 * P * 8 + P * 4 + 256;
+  const size_t NA = lya_absorption ? NP : 0;
+  const size_t bytes = 3 * NL * 8 + NL + N * (4 + 8) + P * 8 + (3 * NP + NA) * 8 + 2 * P * 8 + P * 4 + 256;
   char* base = nullptr;
   CUDA_TRY(cudaMalloc(&base, bytes), g_err);
   char* ptr = base;
@@ -1660,6 +1682,7 @@ int gpdla_training_set(int64_t N, int64_t L_max, const double* wavelengths, cons
   double* d_w = (double*)take(NL * 8); double* d_f = (double*)take(NL * 8); double* d_v = (double*)take(NL * 8);
   double* d_z = (double*)take((size_t)N * 8); double* d_rest = (double*)take(P * 8);
   double* d_lya = (double*)take(NP * 8); double* d_y = (double*)take(NP * 8); double* d_nv = (double*)take(NP * 8);
+  double* d_abs = lya_absorption ? (double*)take(NA * 8) : nullptr;
   double* d_mu = (double*)take(P * 8); double* d_sd = (double*)take(P * 8);
   int32_t* d_len = (int32_t*)take((size_t)N * 4); int32_t* d_cnt = (int32_t*)take(P * 4);
   uint8_t* d_m = (uint8_t*)take(NL);
@@ -1670,17 +1693,19 @@ int gpdla_training_set(int64_t N, int64_t L_max, const double* wavelengths, cons
   up(d_len, lengths, (size_t)N * 4); up(d_z, z_qsos, (size_t)N * 8); up(d_rest, rest_wavelengths, P * 8);
   int rc = GPDLA_ERR_CUDA;
   if (e == cudaSuccess) {
-    rc = gpdla_training_set_device(N, L_max, d_w, d_f, d_v, d_m, d_len, d_z, d_rest, num_pixels, lya_wavelength,
-                                   max_noise_variance, d_lya, d_y, d_nv, d_mu, d_sd, d_cnt, nullptr);
+    rc = training_set_device_impl(fn, N, L_max, d_w, d_f, d_v, d_m, d_len, d_z, d_rest, num_pixels, lya_wavelength,
+                                  max_noise_variance, num_forest_lines, d_lya, d_y, d_nv, d_abs, d_mu, d_sd, d_cnt,
+                                  nullptr);
     if (rc == GPDLA_OK) {
       down(lya_1pzs, d_lya, NP * 8); down(centered_rest_fluxes, d_y, NP * 8); down(rest_noise_variances, d_nv, NP * 8);
+      if (d_abs) down(lya_absorption, d_abs, NA * 8);
       down(mu, d_mu, P * 8); down(std_dev, d_sd, P * 8); down(num_observed, d_cnt, P * 4);
       if (e == cudaSuccess) {
         for (int32_t p = 0; p < num_pixels; ++p)
           if (num_observed[p] < 2) {
             char buf[256];
-            snprintf(buf, sizeof buf, "gpdla_training_set: rest pixel %d (%.2f A) is observed in %d spectra, fewer than 2",
-                     p, rest_wavelengths[p], num_observed[p]);
+            snprintf(buf, sizeof buf, "%s: rest pixel %d (%.2f A) is observed in %d spectra, fewer than 2",
+                     fn, p, rest_wavelengths[p], num_observed[p]);
             g_err = buf;
             rc = GPDLA_ERR_INVALID;
             break;
@@ -1690,6 +1715,97 @@ int gpdla_training_set(int64_t N, int64_t L_max, const double* wavelengths, cons
   }
   if (e != cudaSuccess) { g_err = cudaGetErrorString(e); rc = GPDLA_ERR_CUDA; }
   cudaFree(base);
+  return rc;
+}
+
+int gpdla_training_set_device(int64_t N, int64_t L_max, const double* wavelengths, const double* flux,
+                              const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                              const double* z_qsos, const double* rest_wavelengths, int32_t num_pixels,
+                              double lya_wavelength, double max_noise_variance, double* lya_1pzs,
+                              double* centered_rest_fluxes, double* rest_noise_variances, double* mu, double* std_dev,
+                              int32_t* num_observed, void* stream) {
+  return training_set_device_impl("gpdla_training_set_device", N, L_max, wavelengths, flux, noise_variance, pixel_mask,
+                                  lengths, z_qsos, rest_wavelengths, num_pixels, lya_wavelength, max_noise_variance, -1,
+                                  lya_1pzs, centered_rest_fluxes, rest_noise_variances, nullptr, mu, std_dev,
+                                  num_observed, stream);
+}
+
+int gpdla_training_set(int64_t N, int64_t L_max, const double* wavelengths, const double* flux,
+                       const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                       const double* z_qsos, const double* rest_wavelengths, int32_t num_pixels, double lya_wavelength,
+                       double max_noise_variance, double* lya_1pzs, double* centered_rest_fluxes,
+                       double* rest_noise_variances, double* mu, double* std_dev, int32_t* num_observed) {
+  return training_set_host_impl("gpdla_training_set", N, L_max, wavelengths, flux, noise_variance, pixel_mask, lengths,
+                                z_qsos, rest_wavelengths, num_pixels, lya_wavelength, max_noise_variance, -1, lya_1pzs,
+                                centered_rest_fluxes, rest_noise_variances, nullptr, mu, std_dev, num_observed);
+}
+
+int gpdla_training_set_lyseries_device(int64_t N, int64_t L_max, const double* wavelengths, const double* flux,
+                                       const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                                       const double* z_qsos, const double* rest_wavelengths, int32_t num_pixels,
+                                       double lya_wavelength, double max_noise_variance, int32_t num_forest_lines,
+                                       double* lya_1pzs, double* centered_rest_fluxes, double* rest_noise_variances,
+                                       double* lya_absorption, double* mu, double* std_dev, int32_t* num_observed,
+                                       void* stream) {
+  if (num_forest_lines < 0 || num_forest_lines > MAX_LINES) {
+    g_err = "gpdla_training_set_lyseries_device: num_forest_lines = " + std::to_string(num_forest_lines) +
+            " is outside [0, 31]";
+    return GPDLA_ERR_INVALID;
+  }
+  return training_set_device_impl("gpdla_training_set_lyseries_device", N, L_max, wavelengths, flux, noise_variance,
+                                  pixel_mask, lengths, z_qsos, rest_wavelengths, num_pixels, lya_wavelength,
+                                  max_noise_variance, num_forest_lines, lya_1pzs, centered_rest_fluxes,
+                                  rest_noise_variances, lya_absorption, mu, std_dev, num_observed, stream);
+}
+
+int gpdla_training_set_lyseries(int64_t N, int64_t L_max, const double* wavelengths, const double* flux,
+                                const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                                const double* z_qsos, const double* rest_wavelengths, int32_t num_pixels,
+                                double lya_wavelength, double max_noise_variance, int32_t num_forest_lines,
+                                double* lya_1pzs, double* centered_rest_fluxes, double* rest_noise_variances,
+                                double* lya_absorption, double* mu, double* std_dev, int32_t* num_observed) {
+  if (num_forest_lines < 0 || num_forest_lines > MAX_LINES) {
+    g_err = "gpdla_training_set_lyseries: num_forest_lines = " + std::to_string(num_forest_lines) +
+            " is outside [0, 31]";
+    return GPDLA_ERR_INVALID;
+  }
+  return training_set_host_impl("gpdla_training_set_lyseries", N, L_max, wavelengths, flux, noise_variance, pixel_mask,
+                                lengths, z_qsos, rest_wavelengths, num_pixels, lya_wavelength, max_noise_variance,
+                                num_forest_lines, lya_1pzs, centered_rest_fluxes, rest_noise_variances, lya_absorption,
+                                mu, std_dev, num_observed);
+}
+
+int gpdla_row_nanmedian_fill_device(int64_t N, int32_t P, const double* X, double* out, void* stream) {
+  if (N < 0 || N > INT32_MAX || P < 1 || P > MED_MAX_P || !out || (N > 0 && !X)) {
+    g_err = "gpdla_row_nanmedian_fill_device: invalid arguments (N >= 0, 1 <= P <= " + std::to_string(MED_MAX_P) + ")";
+    return GPDLA_ERR_INVALID;
+  }
+  if (N == 0) return GPDLA_OK;
+  const int S = median_sort_size(P);
+  const size_t smem = (size_t)S * sizeof(uint64_t);
+  CUDA_TRY(cudaFuncSetAttribute(row_nanmedian_fill_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), g_err);
+  row_nanmedian_fill_kernel<<<(unsigned)N, MED_THREADS, smem, (cudaStream_t)stream>>>(X, P, S, out);
+  CUDA_TRY(cudaGetLastError(), g_err);
+  return GPDLA_OK;
+}
+
+int gpdla_row_nanmedian_fill(int64_t N, int32_t P, const double* X, double* out) {
+  if (N < 0 || N > INT32_MAX || P < 1 || P > MED_MAX_P || !out || (N > 0 && !X)) {
+    g_err = "gpdla_row_nanmedian_fill: invalid arguments (N >= 0, 1 <= P <= " + std::to_string(MED_MAX_P) + ")";
+    return GPDLA_ERR_INVALID;
+  }
+  const size_t NP = (size_t)N * P;
+  if (NP == 0) return GPDLA_OK;
+  double* d_x = nullptr;
+  CUDA_TRY(cudaMalloc(&d_x, NP * 8), g_err);
+  cudaError_t e = cudaMemcpy(d_x, X, NP * 8, cudaMemcpyHostToDevice);
+  int rc = GPDLA_ERR_CUDA;
+  if (e == cudaSuccess) {
+    rc = gpdla_row_nanmedian_fill_device(N, P, d_x, d_x, nullptr);          // in place
+    if (rc == GPDLA_OK) e = cudaMemcpy(out, d_x, NP * 8, cudaMemcpyDeviceToHost);
+  }
+  if (e != cudaSuccess) { g_err = cudaGetErrorString(e); rc = GPDLA_ERR_CUDA; }
+  cudaFree(d_x);
   return rc;
 }
 

@@ -1,7 +1,10 @@
 // Training set of the GP null model on the device: learn_qso_model.m:36-75 (spectra -> lya_1pzs, centered_rest_fluxes,
 // rest_noise_variances, mu) and the statistics of its PCA initialisation, learn_qso_model.m:82-95 (nanstd of the
-// centred fluxes, the pairwise covariance that pca(X, 'rows', 'pairwise') decomposes).
-//   training_set_kernel         one CTA per spectrum: linear interpolation (interp1) onto the rest grid, noisy pixels
+// centred fluxes, the pairwise covariance that pca(X, 'rows', 'pairwise') decomposes); the multi-DLA model's variant,
+// learn_qso_model_meanflux.m, adds the Lyman-series mean-flux correction and fills NaNs by row medians before its PCA.
+//   training_set_kernel         one CTA per spectrum: linear interpolation (interp1) onto the rest grid, noisy pixels,
+//                               with LYSERIES also the Kim et al. mean-flux correction of flux and noise variance
+//   row_nanmedian_fill_kernel   one CTA per row: NaN -> the row's nanmedian (bitonic sort in shared memory)
 //   column_partial_kernel       per-column partial sums over fixed row blocks, then column_finish_kernel sums the blocks
 //   pairwise_cov_tile_kernel    lower-triangle 64 x 64 tiles of X~0' X~0 on FP64 DMMA, pairwise counts by popc
 //   pairwise_cov_finish_kernel  fixed-order sum of the row-split partials, / (n - 1), mirrored to the full P x P
@@ -25,22 +28,38 @@ struct TrainingArgs {
   int64_t N, L_max;
   int P;
   double lya_wavelength;         // set_parameters.m:5
-  double max_noise_variance;     // set_parameters.m (1^2)
+  double max_noise_variance;     // set_parameters.m (1^2), set_parameters_multi.m:37 (3^2)
   double* lya_1pzs;              // [N x P]
   double* rest_fluxes;           // [N x P], centred in place afterwards
   double* rest_noise_variances;  // [N x P]
+  // mean-flux correction (training_set_kernel<true> only): forest.num_forest_lines members, their wavelengths (A),
+  // Kim weights and prev_beta -- the table inference reads from c_forest, filled by the same host helper
+  ForestConstants forest;
+  double lya_over_wavelength[MAX_LINES];   // lya_wavelength / forest.wavelength[l], increasing in l
+  double* lya_absorption;        // [N x P] or nullptr
 };
 
 constexpr int TS_THREADS = 256;
 
-__host__ __device__ constexpr size_t training_set_smem_bytes(int64_t L_max) { return (size_t)L_max * 4 * sizeof(double); }
+// emitted wavelengths, 1 + z_lya, flux, noise variance; the Lyman-series variant also stages the observed wavelengths
+__host__ __device__ constexpr size_t training_set_smem_bytes(int64_t L_max, bool lyseries) {
+  return (size_t)L_max * (lyseries ? 5 : 4) * sizeof(double);
+}
 
 // interp1(x, v, r) on the interval [x_j, x_{j+1}], every operation rounded on its own (no FMA contraction)
 __device__ __forceinline__ double lerp_rn(double t, double v0, double v1) {
   return __dadd_rn(v0, __dmul_rn(t, __dsub_rn(v1, v0)));
 }
 
-__global__ void __launch_bounds__(TS_THREADS) training_set_kernel(TrainingArgs a) {
+// 1 + z_l = 1 + (lambda - lambda_l) / lambda_l at an observed wavelength, each operation rounded on its own
+__device__ __forceinline__ double one_plus_z_rn(double lam, double lambda_l) {
+  return __dadd_rn(1.0, __ddiv_rn(__dsub_rn(lam, lambda_l), lambda_l));
+}
+
+// LYSERIES = false: learn_qso_model.m:36-69.  LYSERIES = true: learn_qso_model_meanflux.m, the same interpolation and
+// noisy-pixel rule, then every kept pixel divided by the Kim et al. absorption exp(-sum_l kim_tau_l (1 + z_l)^prev_beta)
+template <bool LYSERIES>
+__global__ void __launch_bounds__(TS_THREADS) training_set_kernel(const __grid_constant__ TrainingArgs a) {
   extern __shared__ __align__(16) double ts_smem[];
   const int64_t i = blockIdx.x;
   const int L = (int)max((int64_t)0, min((int64_t)a.lengths[i], a.L_max));
@@ -48,6 +67,7 @@ __global__ void __launch_bounds__(TS_THREADS) training_set_kernel(TrainingArgs a
   double* sw = sx + a.L_max;         // 1 + (lambda - lya) / lya
   double* sf = sw + a.L_max;         // flux, NaN where masked
   double* sv = sf + a.L_max;         // noise variance, NaN where masked
+  double* sl = sv + a.L_max;         // observed wavelengths (LYSERIES)
   const double opz = __dadd_rn(1.0, a.z_qsos[i]);
   const double lya = a.lya_wavelength;
   const int64_t row = i * a.L_max;
@@ -58,6 +78,7 @@ __global__ void __launch_bounds__(TS_THREADS) training_set_kernel(TrainingArgs a
     sw[j] = __dadd_rn(1.0, __ddiv_rn(__dsub_rn(lam, lya), lya));
     sf[j] = m ? __longlong_as_double(0x7ff8000000000000ll) : a.flux[row + j];
     sv[j] = m ? __longlong_as_double(0x7ff8000000000000ll) : a.noise_variance[row + j];
+    if (LYSERIES) sl[j] = lam;
   }
   __syncthreads();
   const double qnan = __longlong_as_double(0x7ff8000000000000ll);
@@ -65,6 +86,7 @@ __global__ void __launch_bounds__(TS_THREADS) training_set_kernel(TrainingArgs a
   for (int p = threadIdx.x; p < a.P; p += TS_THREADS) {        // :52-64, then the noisy-pixel rule :66-69
     const double r = a.rest[p];
     double oz = qnan, of = qnan, ov = qnan;
+    double total = 0.0;                                        // nansum of the forest terms: 0 where nothing is observed
     if (L >= 2 && r >= sx[0] && r <= sx[L - 1]) {
       int lo = 0, hi = L - 1;                                  // largest j with x_j <= r
       while (lo < hi) {
@@ -77,6 +99,28 @@ __global__ void __launch_bounds__(TS_THREADS) training_set_kernel(TrainingArgs a
       of = lerp_rn(t, sf[j], sf[j + 1]);
       ov = lerp_rn(t, sv[j], sv[j + 1]);
       if (ov > a.max_noise_variance) { oz = qnan; of = qnan; ov = qnan; }
+      else if (LYSERIES) {
+        // sum_l kim_tau_l (1 + z_l)^prev_beta in ascending l; a member below Lya counts where 1 + z_l <= 1 + z_qso.  A
+        // failing indicator makes the term +0.0, which leaves the sum's bits alone, so its pow is skipped.  Moreover
+        // 1 + z_l equals (1 + z_Lya) lya / lambda_l to a few ulp; where that estimate exceeds 1 + z_qso by a relative
+        // 1e-12 the indicator fails for certain, and, the estimate growing with l, for every later member too.  So the
+        // loop stops there, and most grid points evaluate one to three members exactly instead of all of them.
+        const double l0 = sl[j], l1 = sl[j + 1];
+        const double opz_safe = opz * (1.0 + 1e-12);
+        for (int l = 0; l < a.forest.num_forest_lines; ++l) {
+          if (l > 0 && oz * a.lya_over_wavelength[l] > opz_safe) break;
+          const double wl = a.forest.wavelength[l];
+          const double zl = lerp_rn(t, one_plus_z_rn(l0, wl), one_plus_z_rn(l1, wl));
+          if (l == 0 ? !isnan(zl) : zl <= opz)                 // NaN terms are skipped (nansum)
+            total = __dadd_rn(total, __dmul_rn(a.forest.kim_tau[l], pow(zl, a.forest.prev_beta)));
+        }
+      }
+    }
+    if (LYSERIES) {
+      const double absorption = exp(-total);
+      of = __ddiv_rn(of, absorption);                          // NaN stays NaN
+      ov = __ddiv_rn(ov, __dmul_rn(absorption, absorption));
+      if (a.lya_absorption) a.lya_absorption[out + p] = absorption;
     }
     a.lya_1pzs[out + p] = oz;
     a.rest_fluxes[out + p] = of;
@@ -127,6 +171,66 @@ __global__ void column_finish_kernel(const double* __restrict__ psum, const int3
   if (mode == COL_MEAN) { out[c] = n > 0 ? s / n : qnan; if (count) count[c] = n; }
   else if (mode == COL_CENTRE) out[c] = n > 0 ? s / n : qnan;
   else out[c] = n > 1 ? sqrt(s / (n - 1)) : qnan;
+}
+
+// ---- row medians: out[r, p] = X[r, p], or nanmedian(X[r, :]) where X[r, p] is NaN; an all-NaN row stays NaN.  One CTA per
+// row sorts the row's values as order-preserving integer keys (NaN and the padding up to a power of two last) with a
+// bitonic network in shared memory; no atomics, so the result does not depend on scheduling.
+constexpr int MED_THREADS = 512;
+constexpr int MED_MAX_P = 16384;               // 128 KB of keys
+
+__host__ __device__ inline int median_sort_size(int P) { int s = 1; while (s < P) s <<= 1; return s; }
+
+__device__ __forceinline__ uint64_t median_key(double v) {     // a < b  <=>  key(a) < key(b); -0 sorts before +0
+  const uint64_t b = (uint64_t)__double_as_longlong(v);
+  return isnan(v) ? ~0ull : (b >> 63) ? ~b : (b | 0x8000000000000000ull);
+}
+__device__ __forceinline__ double median_value(uint64_t k) {
+  return __longlong_as_double((long long)((k >> 63) ? (k & 0x7fffffffffffffffull) : ~k));
+}
+
+// MATLAB's median of an even count: meanof(a, b) = a + (b - a) / 2, or (a + b) / 2 where sign(a) ~= sign(b) (sign(0) = 0)
+// or either is infinite
+__device__ __forceinline__ double matlab_meanof(double a, double b) {
+  const int sa = (a > 0.0) - (a < 0.0), sb = (b > 0.0) - (b < 0.0);
+  if (sa != sb || isinf(a) || isinf(b)) return __ddiv_rn(__dadd_rn(a, b), 2.0);
+  return __dadd_rn(a, __ddiv_rn(__dsub_rn(b, a), 2.0));
+}
+
+__global__ void __launch_bounds__(MED_THREADS) row_nanmedian_fill_kernel(const double* X, int P, int S, double* out) {
+  extern __shared__ __align__(16) uint64_t med_keys[];
+  __shared__ int warp_count[MED_THREADS / 32];
+  const int64_t row = (int64_t)blockIdx.x * P;
+  int n = 0;
+  for (int p = threadIdx.x; p < S; p += MED_THREADS) {
+    uint64_t k = ~0ull;
+    if (p < P) { const double v = X[row + p]; if (!isnan(v)) { k = median_key(v); ++n; } }
+    med_keys[p] = k;
+  }
+  n = __reduce_add_sync(0xffffffffu, n);
+  if ((threadIdx.x & 31) == 0) warp_count[threadIdx.x >> 5] = n;
+  __syncthreads();
+  int count = 0;
+#pragma unroll
+  for (int w = 0; w < MED_THREADS / 32; ++w) count += warp_count[w];
+  double med = __longlong_as_double(0x7ff8000000000000ll);
+  if (count > 0 && count < P) {                  // a complete row has nothing to fill, an all-NaN row nothing to fill with
+    for (int k = 2; k <= S; k <<= 1)
+      for (int j = k >> 1; j > 0; j >>= 1) {
+        for (int e = threadIdx.x; e < S / 2; e += MED_THREADS) {
+          const int lo = 2 * e - (e & (j - 1)), hi = lo + j;      // the pairs (lo, lo + j) with bit j of lo clear
+          const uint64_t a = med_keys[lo], b = med_keys[hi];
+          if ((a > b) == ((lo & k) == 0)) { med_keys[lo] = b; med_keys[hi] = a; }
+        }
+        __syncthreads();
+      }
+    med = (count & 1) ? median_value(med_keys[count / 2])
+                      : matlab_meanof(median_value(med_keys[count / 2 - 1]), median_value(med_keys[count / 2]));
+  }
+  for (int p = threadIdx.x; p < P; p += MED_THREADS) {
+    const double v = X[row + p];
+    out[row + p] = isnan(v) ? med : v;
+  }
 }
 
 // ---- pairwise covariance C_pq = sum_{rows observed in both} X~_rp X~_rq / (n_pq - 1), X~ = X - nanmean(X)

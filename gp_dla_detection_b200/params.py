@@ -7,6 +7,8 @@ from __future__ import annotations
 
 from dataclasses import dataclass
 
+import numpy as np
+
 lya_wavelength = 1215.6701          # set_parameters.m:5   Lyman alpha transition wavelength (A)
 lyb_wavelength = 1025.7223          # :6
 lyman_limit = 911.7633              # :7
@@ -42,3 +44,21 @@ class Parameters:
 
 
 DEFAULT = Parameters()
+
+# ---- the multi-DLA / mean-flux model (multi_dlas/set_parameters_multi.m, learn_qso_model_meanflux.m)
+MULTI = Parameters(max_noise_variance=3.0 ** 2)      # set_parameters_multi.m:37; everything else as DEFAULT
+prev_tau_0 = 0.0023                                  # learn_qso_model_meanflux.m: Kim et al. (2007) mean-flux prior
+prev_beta = 3.65
+num_forest_lines = 31                                # set_parameters_multi.m:76
+# set_parameters_multi.m:77-109, Angstrom (the cm values of voigt.c times 1e8, as the library computes them)
+all_transition_wavelengths = np.array([
+    1.2156701e-05, 1.0257223e-05, 9.725368e-06, 9.497431e-06, 9.378035e-06, 9.307483e-06, 9.262257e-06,
+    9.231504e-06, 9.209631e-06, 9.193514e-06, 9.181294e-06, 9.171806e-06, 9.16429e-06, 9.15824e-06, 9.15329e-06,
+    9.14919e-06, 9.14576e-06, 9.14286e-06, 9.14039e-06, 9.13826e-06, 9.13641e-06, 9.13480e-06, 9.13339e-06,
+    9.13215e-06, 9.13104e-06, 9.13006e-06, 9.12918e-06, 9.12839e-06, 9.12768e-06, 9.12703e-06, 9.12645e-06]) * 1e8
+all_oscillator_strengths = np.array([                # :111-143
+    0.416400, 0.079120, 0.029000, 0.013940, 0.007799, 0.004814, 0.003183, 0.002216, 0.001605, 0.00120, 0.000921,
+    0.0007226, 0.000577, 0.000469, 0.000386, 0.000321, 0.000270, 0.000230, 0.000197, 0.000170, 0.000148, 0.000129,
+    0.000114, 0.000101, 0.000089, 0.000080, 0.000071, 0.000064, 0.000058, 0.000053, 0.000048])
+all_transition_wavelengths.flags.writeable = False
+all_oscillator_strengths.flags.writeable = False

@@ -259,6 +259,38 @@ int gpdla_training_set_device(int64_t N, int64_t L_max, const double* wavelength
 int gpdla_pairwise_covariance(int64_t N, int32_t P, const double* X, double* cov, int32_t* counts);
 int gpdla_pairwise_covariance_device(int64_t N, int32_t P, const double* X, double* cov, int32_t* counts, void* stream);
 
+/* ---- Training set of the multi-DLA (mean-flux) null model: multi_dlas/learn_qso_model_meanflux.m ----
+ * The gpdla_training_set arguments (max_noise_variance is 3^2 for this model, set_parameters_multi.m:37) plus
+ * num_forest_lines (0..31; 31 in the reference) and the nullable output lya_absorption [N x num_pixels].  After the
+ * interpolation and the noisy-pixel rule (applied to the noise variance before the correction), each of the first
+ * num_forest_lines Lyman-series members l gives 1 + z_l = interp1(x, 1 + (lambda - lambda_l) / lambda_l, r) with the same
+ * interval and weight; total = sum_l kim_tau_l (1 + z_l)^3.65 in ascending l, kim_tau_l = 0.0023 f_l / f_lya * lambda_l /
+ * lya_wavelength (the table the multi-DLA inference uses); the Lya term always counts, a term l >= 1 only where
+ * 1 + z_l <= 1 + z_qso; NaN terms are skipped, so lya_absorption = exp(-total) is 1 where nothing is observed.  Rest
+ * fluxes are divided by lya_absorption and rest noise variances by lya_absorption^2 before mu, the centring and std_dev;
+ * lya_1pzs is not corrected.  num_forest_lines = 0 gives the bits of gpdla_training_set.  Checks, errors and the
+ * GPDLA_ERR_INVALID of a rest pixel observed fewer than 2 times as gpdla_training_set. */
+int gpdla_training_set_lyseries(int64_t N, int64_t L_max, const double* wavelengths, const double* flux,
+                                const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                                const double* z_qsos, const double* rest_wavelengths, int32_t num_pixels,
+                                double lya_wavelength, double max_noise_variance, int32_t num_forest_lines,
+                                double* lya_1pzs, double* centered_rest_fluxes, double* rest_noise_variances,
+                                double* lya_absorption, double* mu, double* std_dev, int32_t* num_observed);
+int gpdla_training_set_lyseries_device(int64_t N, int64_t L_max, const double* wavelengths, const double* flux,
+                                       const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                                       const double* z_qsos, const double* rest_wavelengths, int32_t num_pixels,
+                                       double lya_wavelength, double max_noise_variance, int32_t num_forest_lines,
+                                       double* lya_1pzs, double* centered_rest_fluxes, double* rest_noise_variances,
+                                       double* lya_absorption, double* mu, double* std_dev, int32_t* num_observed,
+                                       void* stream);
+/* The matrix learn_qso_model_meanflux.m hands to pca(..., 'rows', 'complete'): out = X with each row's NaNs replaced by
+ * that row's nanmedian (MATLAB's median: for an even count meanof(a, b) = a + (b - a) / 2, or (a + b) / 2 when
+ * sign(a) ~= sign(b) or either is infinite).  An all-NaN row stays NaN, so every row of out is complete or all NaN and
+ * gpdla_pairwise_covariance of out is the covariance of its complete rows.  X, out: [N x P] row-major, 1 <= P <= 16384;
+ * out may alias X.  Deterministic (no atomics).  Context-free; the _device entry is asynchronous on `stream`. */
+int gpdla_row_nanmedian_fill(int64_t N, int32_t P, const double* X, double* out);
+int gpdla_row_nanmedian_fill_device(int64_t N, int32_t P, const double* X, double* out, void* stream);
+
 /* voigt.c:253-304: profile has num_points - 6 entries.  Host buffers; runs on the current device. */
 int gpdla_voigt(const double* lambdas, int64_t num_points, double z, double N, int32_t num_lines, double* profile);
 /* Batched, device buffers: profile[s, :] = voigt(lambdas, z[s], N[s], num_lines), [S x (num_points-6)] */
