@@ -117,6 +117,12 @@ SYMBOLS = {
                                            + [ctypes.c_void_p] * 8),
     "gpdla_row_nanmedian_fill": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int32] + [ctypes.c_void_p] * 2),
     "gpdla_row_nanmedian_fill_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int32] + [ctypes.c_void_p] * 3),
+    "gpdla_dla_statistics": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64] + [ctypes.c_void_p] * 8
+                             + [ctypes.c_int32, c_double_p, ctypes.c_int32, c_double_p, ctypes.c_double, ctypes.c_double,
+                                ctypes.c_void_p]),
+    "gpdla_dla_statistics_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64] + [ctypes.c_void_p] * 8
+                                    + [ctypes.c_int32, c_double_p, ctypes.c_int32, c_double_p, ctypes.c_double,
+                                       ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]),
 }
 
 _lib = None

@@ -98,6 +98,8 @@ class DLAProcessor:
                                              float(model["log_beta"])), self._ctx)
         off, lnhi, nhi = (_f64(samples[k]).ravel() for k in ("offset_samples", "log_nhi_samples", "nhi_samples"))
         self.num_dla_samples = int(off.size)
+        self._samples_host = (off, lnhi, nhi)
+        self._samples_device = None          # CUDA copies for statistics_device, made on its first call
         _lib.check(self._lib.gpdla_set_samples(self._ctx, _dp(off), _dp(lnhi), _dp(nhi), off.size), self._ctx)
         self.has_lls = "lls_nhi_samples" in samples and "Z_lls" in samples and "Z_dla" in samples
         if self.has_lls:   # multi_dlas/set_lls_parameters.m:55-71
@@ -253,6 +255,45 @@ class DLAProcessor:
             pixel_mask.data_ptr(), lengths.data_ptr(), z_qsos.data_ptr(), ctypes.byref(res),
             ctypes.c_void_p(stream)), self._ctx)
         return out
+
+    def statistics_device(self, out: Dict, z_edges, log_nhi_edges, select=None, sums=None,
+                          dla_log_nhi_min: float = _params.dla_log_nhi_min, omega_m: float = _params.omega_m):
+        """Population-statistics sums (``dla_statistics_sums``) of what ``process_device(...,
+        return_sample_log_likelihoods=True)`` returned, without the sample log-likelihoods leaving the GPU.  ``select``:
+        optional CUDA bool / uint8 tensor [Q]; ``sums``: a float64 CUDA tensor to add into (a new zero vector when None).
+        Returns the sums tensor; asynchronous on torch's current stream.  Uses device copies of this processor's samples,
+        made once."""
+        import torch
+        ll = out.get("sample_log_likelihoods_dla")
+        if ll is None:
+            raise ValueError("statistics_device needs process_device(..., return_sample_log_likelihoods=True)")
+        dev = ll.device
+        Q, S = ll.shape
+        if S != self.num_dla_samples:
+            raise ValueError("sample_log_likelihoods_dla has %d samples, this processor %d" % (S, self.num_dla_samples))
+        ze, ne = _stats_edges(z_edges, log_nhi_edges)
+        width = dla_statistics_width(ze.size - 1, ne.size - 1)
+        if self._samples_device is None:
+            self._samples_device = tuple(torch.from_numpy(a).to(dev) for a in self._samples_host)
+        if sums is None:
+            sums = torch.zeros(width, dtype=torch.float64, device=dev)
+        if not (sums.is_cuda and sums.device == dev and sums.dtype == torch.float64 and sums.is_contiguous()
+                and sums.numel() == width):
+            raise ValueError("sums must be a contiguous float64 CUDA tensor of %d entries on %s" % (width, dev))
+        sel = None
+        if select is not None:
+            sel = select.to(device=dev, dtype=torch.uint8).contiguous()
+            if sel.shape != (Q,):
+                raise ValueError("select must have one entry per quasar")
+        ptr = lambda t: None if t is None else ctypes.c_void_p(t.data_ptr())
+        off, lnhi, nhi = self._samples_device
+        with torch.cuda.device(dev):
+            stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+            _lib.check(self._lib.gpdla_dla_statistics_device(
+                Q, S, ptr(ll), ptr(out["p_dlas"]), ptr(out["min_z_dlas"]), ptr(out["max_z_dlas"]), ptr(sel), ptr(off),
+                ptr(lnhi), ptr(nhi), ze.size - 1, _dp(ze), ne.size - 1, _dp(ne), float(dla_log_nhi_min),
+                float(omega_m), ptr(sums), stream))
+        return sums
 
 
 def process_qsos(model: Dict, samples: Dict, spectra: Dict, prior: Dict, params: Parameters = DEFAULT,
@@ -777,6 +818,103 @@ def learn_qso_model_meanflux_from_spectra(spectra: Dict, k: int, params: Paramet
                 M=np.ascontiguousarray(x[:P * k].reshape(k, P).T), log_omega=x[P * k:P * (k + 1)].copy(),
                 log_c_0=float(x[-3]), log_tau_0=float(x[-2]), log_beta=float(x[-1]),
                 initial_x=ts["initial_x"], log_likelihood=f, result=res)
+
+
+# ---------------------------------------------------------------- population statistics (CDDF_analysis/calc_cddf.py)
+def dla_statistics_width(n_z: int, n_nhi: int) -> int:
+    """Length of the sums vector for n_z z bins and n_nhi log-N bins."""
+    return 2 * n_z * n_nhi + 5 * n_z + 1
+
+
+def dla_statistics_layout(n_z: int, n_nhi: int) -> Dict[str, tuple]:
+    """Names of the parts of the sums vector -> (start, shape): counts, counts_var [n_z, n_nhi]; dla, dla_var, nhi,
+    nhi_var, path [n_z]; num_quasars []."""
+    a, t = n_z * n_nhi, 2 * n_z * n_nhi
+    return dict(counts=(0, (n_z, n_nhi)), counts_var=(a, (n_z, n_nhi)), dla=(t, (n_z,)), dla_var=(t + n_z, (n_z,)),
+                nhi=(t + 2 * n_z, (n_z,)), nhi_var=(t + 3 * n_z, (n_z,)), path=(t + 4 * n_z, (n_z,)),
+                num_quasars=(t + 5 * n_z, ()))
+
+
+def unpack_dla_statistics(sums, n_z: int, n_nhi: int) -> Dict[str, np.ndarray]:
+    """The sums vector (host array or tensor) -> a dict of its parts as host arrays."""
+    v = np.asarray(sums.cpu().numpy() if hasattr(sums, "cpu") else sums, dtype=np.float64)
+    out = {}
+    for n, (start, shape) in dla_statistics_layout(n_z, n_nhi).items():
+        size = int(np.prod(shape))
+        out[n] = v[start:start + size].reshape(shape).copy() if shape else float(v[start])
+    return out
+
+
+def _stats_edges(z_edges, log_nhi_edges):
+    ze, ne = _f64(z_edges).ravel(), _f64(log_nhi_edges).ravel()
+    if ze.size < 2 or ne.size < 2:
+        raise ValueError("z_edges and log_nhi_edges need at least two entries (one bin)")
+    return ze, ne
+
+
+def dla_statistics_sums(results: Dict, samples: Dict, z_edges, log_nhi_edges, select=None, sums=None,
+                        dla_log_nhi_min: float = _params.dla_log_nhi_min, omega_m: float = _params.omega_m,
+                        device: int = 0) -> np.ndarray:
+    """The additive sums behind the column density distribution, dN/dX and Omega_DLA (CDDF_analysis/calc_cddf.py) of
+    one ``process`` / ``process_qsos`` result (host arrays, with ``sample_log_likelihoods_dla``) and the samples it was
+    run with, computed on the GPU.  Per quasar the normalised sample posterior is binned by z_dla (``z_edges``) and
+    log10 N_HI (``log_nhi_edges``), half-open bins; ``select`` [Q] (bool) drops quasars (SNR, z_qso or filter cuts).
+    Returns the float64 vector ``dla_statistics_layout`` describes -- ``sums`` (when given) plus this batch.  Sums of
+    disjoint quasar sets add; pass the total to ``finish_dla_statistics``.  Variances add across quasars, not across z
+    bins: a statistic over all z needs a single z bin."""
+    import torch
+    lib = _lib.load()
+    ze, ne = _stats_edges(z_edges, log_nhi_edges)
+    width = dla_statistics_width(ze.size - 1, ne.size - 1)
+    ll = _f64(results["sample_log_likelihoods_dla"])
+    if ll.ndim != 2:
+        raise ValueError("sample_log_likelihoods_dla must be (Q, S)")
+    Q, S = ll.shape
+    p, zlo, zhi = (_f64(results[n]).ravel() for n in ("p_dlas", "min_z_dlas", "max_z_dlas"))
+    off, lnhi, nhi = (_f64(samples[k]).ravel() for k in ("offset_samples", "log_nhi_samples", "nhi_samples"))
+    if p.size != Q or zlo.size != Q or zhi.size != Q or off.size != S or lnhi.size != S or nhi.size != S:
+        raise ValueError("results need Q entries per quasar and the samples S entries each (Q, S = %d, %d)" % (Q, S))
+    sel = None
+    if select is not None:
+        sel = np.ascontiguousarray(np.asarray(select).astype(np.uint8)).ravel()
+        if sel.size != Q:
+            raise ValueError("select must have one entry per quasar")
+    out = np.zeros(width) if sums is None else _f64(sums).ravel().copy()
+    if out.size != width:
+        raise ValueError("sums must have %d entries" % width)
+    vp = lambda a: None if a is None else ctypes.c_void_p(a.ctypes.data)
+    with torch.cuda.device(device):
+        _lib.check(lib.gpdla_dla_statistics(Q, S, vp(ll), vp(p), vp(zlo), vp(zhi), vp(sel), vp(off), vp(lnhi), vp(nhi),
+                                            ze.size - 1, _dp(ze), ne.size - 1, _dp(ne), float(dla_log_nhi_min),
+                                            float(omega_m), vp(out)))
+    return out
+
+
+def omega_dla_coefficient(hubble_h: float = _params.hubble_h) -> float:
+    """8 pi G m_H / (3 c H0) in cm^2: Omega_DLA = this x (sum of N_HI) / (absorption path).  HI only, no helium."""
+    H0 = 100.0 * hubble_h * 1e5 / _params.megaparsec                      # s^-1
+    return 8.0 * np.pi * _params.gravitational_constant * _params.hydrogen_mass / (3.0 * _params.speed_of_light_cgs * H0)
+
+
+def finish_dla_statistics(sums, z_edges, log_nhi_edges, hubble_h: float = _params.hubble_h) -> Dict[str, np.ndarray]:
+    """The statistics from the total sums (host): ``cddf`` f(N, X) = counts / (dN path) [n_z, n_nhi] in cm^2 per unit
+    absorption distance, ``dndx`` = dla / path and ``omega_dla`` = 8 pi G m_H / (3 c H0) nhi / path [n_z], each with
+    ``*_sigma`` = sqrt(variance) over the same factors, plus ``path_length`` (sum of dX per z bin), ``expected_counts``
+    (the Poisson-binomial mean of DLAs per cell) and ``num_quasars``.  Omega_m entered through the path the sums carry;
+    ``hubble_h`` sets H0 = 100 h km/s/Mpc.  Bins without path give NaN."""
+    ze, ne = _stats_edges(z_edges, log_nhi_edges)
+    n_z, n_nhi = ze.size - 1, ne.size - 1
+    t = unpack_dla_statistics(sums, n_z, n_nhi)
+    path = t["path"]
+    with np.errstate(divide="ignore", invalid="ignore"):
+        inv = np.where(path > 0, 1.0 / path, np.nan)
+        dn = 10.0 ** ne[1:] - 10.0 ** ne[:-1]
+        coef = omega_dla_coefficient(hubble_h)
+        return dict(cddf=t["counts"] / dn[None, :] * inv[:, None],
+                    cddf_sigma=np.sqrt(t["counts_var"]) / dn[None, :] * inv[:, None],
+                    dndx=t["dla"] * inv, dndx_sigma=np.sqrt(t["dla_var"]) * inv,
+                    omega_dla=coef * t["nhi"] * inv, omega_dla_sigma=coef * np.sqrt(np.maximum(t["nhi_var"], 0.0)) * inv,
+                    path_length=path, expected_counts=t["counts"], num_quasars=int(round(t["num_quasars"])))
 
 
 def matlab_default_rand(n: int) -> np.ndarray:

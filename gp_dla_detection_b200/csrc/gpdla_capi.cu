@@ -7,6 +7,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
 #include <map>
 #include <mutex>
 #include <numeric>
@@ -20,6 +21,7 @@
 #include "gpdla_preload.cuh"
 #include "gpdla_objective.cuh"
 #include "gpdla_training.cuh"
+#include "gpdla_statistics.cuh"
 #include "gpdla_rest_table.h"
 
 using namespace gpdla;
@@ -1870,6 +1872,159 @@ int gpdla_pairwise_covariance(int64_t N, int32_t P, const double* X, double* cov
     }
   }
   if (e != cudaSuccess) { g_err = cudaGetErrorString(e); rc = GPDLA_ERR_CUDA; }
+  cudaFree(base);
+  return rc;
+}
+
+// ---- population statistics of the single-DLA catalogue (CDDF_analysis/calc_cddf.py) ----
+
+// the checks both statistics entries make before any CUDA call
+static int stats_check(const char* fn, int64_t Q, int64_t S, const double* ll, const double* p_dlas,
+                       const double* min_z_dlas, const double* max_z_dlas, const double* offset_samples,
+                       const double* log_nhi_samples, const double* nhi_samples, int32_t n_z, const double* z_edges,
+                       int32_t n_nhi, const double* log_nhi_edges, double dla_log_nhi_min, double omega_m,
+                       const double* sums) {
+  auto fail = [&](const std::string& why) { g_err = std::string(fn) + ": " + why; return GPDLA_ERR_INVALID; };
+  if (Q < 0 || Q > INT32_MAX || S < 1 || S > INT32_MAX) return fail("Q must lie in [0, 2^31) and S in [1, 2^31)");
+  if (n_z < 1 || n_z > STAT_MAX_Z)
+    return fail("n_z = " + std::to_string(n_z) + " is outside [1, " + std::to_string(STAT_MAX_Z) + "]");
+  if (n_nhi < 1 || n_nhi > STAT_MAX_NHI)
+    return fail("n_nhi = " + std::to_string(n_nhi) + " is outside [1, " + std::to_string(STAT_MAX_NHI) + "]");
+  if (!z_edges || !log_nhi_edges || !sums || !offset_samples || !log_nhi_samples || !nhi_samples ||
+      (Q > 0 && (!ll || !p_dlas || !min_z_dlas || !max_z_dlas)))
+    return fail("a required array is NULL");
+  for (int pass = 0; pass < 2; ++pass) {
+    const double* e = pass ? log_nhi_edges : z_edges;
+    const int n = (pass ? n_nhi : n_z) + 1;
+    const char* name = pass ? "log_nhi_edges" : "z_edges";
+    for (int i = 0; i < n; ++i) {
+      if (!std::isfinite(e[i])) return fail(std::string(name) + "[" + std::to_string(i) + "] is not finite");
+      if (i > 0 && !(e[i] > e[i - 1])) return fail(std::string(name) + " must be strictly increasing (entry " + std::to_string(i) + ")");
+    }
+  }
+  if (!std::isfinite(dla_log_nhi_min)) return fail("dla_log_nhi_min is not finite");
+  if (!(omega_m > 0.0 && omega_m <= 1.0)) return fail("omega_m must lie in (0, 1]");
+  return GPDLA_OK;
+}
+
+int gpdla_dla_statistics_device(int64_t Q, int64_t S, const double* sample_log_likelihoods_dla, const double* p_dlas,
+                                const double* min_z_dlas, const double* max_z_dlas, const uint8_t* select,
+                                const double* offset_samples, const double* log_nhi_samples, const double* nhi_samples,
+                                int32_t n_z, const double* z_edges, int32_t n_nhi, const double* log_nhi_edges,
+                                double dla_log_nhi_min, double omega_m, double* sums, void* stream) {
+  const char* fn = "gpdla_dla_statistics_device";
+  int rc = stats_check(fn, Q, S, sample_log_likelihoods_dla, p_dlas, min_z_dlas, max_z_dlas, offset_samples,
+                       log_nhi_samples, nhi_samples, n_z, z_edges, n_nhi, log_nhi_edges, dla_log_nhi_min, omega_m, sums);
+  if (rc) return rc;
+  if (Q == 0) return GPDLA_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  // log-N classes: the intervals between the union of the bin edges and the DLA threshold
+  std::vector<double> bound(log_nhi_edges, log_nhi_edges + n_nhi + 1);
+  bound.push_back(dla_log_nhi_min);
+  std::sort(bound.begin(), bound.end());
+  bound.erase(std::unique(bound.begin(), bound.end()), bound.end());
+  const int m = (int)bound.size();
+  auto class_of = [&](double v) { return (int)(std::lower_bound(bound.begin(), bound.end(), v) - bound.begin()) + 1; };
+  StatsClassArgs ca;
+  ca.offset = offset_samples; ca.log_nhi = log_nhi_samples; ca.S = S; ca.nbound = m;
+  for (int k = 0; k < m; ++k) ca.bound[k] = bound[k];
+  StatsArgs a;
+  a.ll = sample_log_likelihoods_dla; a.p_dlas = p_dlas; a.min_z_dlas = min_z_dlas; a.max_z_dlas = max_z_dlas;
+  a.select = select; a.S = S; a.n_z = n_z; a.n_nhi = n_nhi; a.nbound = m; a.W = stats_width(n_z, n_nhi);
+  for (int e = 0; e <= n_z; ++e) a.z_edges[e] = z_edges[e];
+  for (int c = 0; c < n_nhi; ++c) {
+    a.nhi_class0[c] = (int16_t)class_of(log_nhi_edges[c]);
+    a.nhi_class1[c] = (int16_t)class_of(log_nhi_edges[c + 1]);
+  }
+  a.dla_class0 = class_of(dla_log_nhi_min);
+  a.omega_m = omega_m; a.omega_l = 1.0 - omega_m; a.x_coef = 2.0 / (3.0 * omega_m);
+  const int64_t W = a.W;
+  int dev = 0, optin = 0;
+  CUDA_TRY(cudaGetDevice(&dev), g_err);
+  CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev), g_err);
+  const bool staged = stats_smem_bytes(true, S, n_z, m) + STAT_THREADS / 32 * 8 + 64 <= (size_t)optin;
+  const size_t smem = stats_smem_bytes(staged, S, n_z, m);
+  // rows of per-quasar cell values are reduced over fixed COL_ROWS-row blocks; a chunk of quasars is a whole number of
+  // blocks, so the chunking (at most 256 MB of rows at a time) does not change the summation order
+  const int64_t nblocks = (Q + COL_ROWS - 1) / COL_ROWS;
+  const int64_t chunk = std::min(nblocks * COL_ROWS,
+                                 std::max<int64_t>(COL_ROWS, ((256ll << 20) / (W * 8)) / COL_ROWS * COL_ROWS));
+  const size_t bytes = (size_t)S * (4 + 8 + 4 + 4 + 8 + 8) + (size_t)(m + 2) * 4 + (size_t)chunk * W * 8 +
+                       (size_t)nblocks * W * (8 + 4) + 8 * 64;
+  char* base = nullptr;
+  CUDA_TRY(cudaMallocAsync(&base, bytes, st), g_err);
+  char* ptr = base;
+  auto take = [&](size_t n) { char* r = ptr; ptr += (n + 15) / 16 * 16; return r; };
+  double* sorted_offset = (double*)take(S * 8); double* sorted_nhi = (double*)take(S * 8);
+  uint64_t* key = (uint64_t*)take(S * 8);
+  double* rows = (double*)take((size_t)chunk * W * 8); double* psum = (double*)take((size_t)nblocks * W * 8);
+  int32_t* cls = (int32_t*)take(S * 4); int32_t* perm = (int32_t*)take(S * 4); int32_t* rank = (int32_t*)take(S * 4);
+  int32_t* class_start = (int32_t*)take((m + 2) * 4); int32_t* pcnt = (int32_t*)take((size_t)nblocks * W * 4);
+  ca.cls = cls; ca.key = key;
+  a.sorted_offset = sorted_offset; a.sorted_nhi = sorted_nhi; a.perm = perm; a.rank = rank; a.class_start = class_start;
+  a.rows = rows;
+  const unsigned sblocks = (unsigned)((S + STAT_THREADS - 1) / STAT_THREADS);
+  stats_class_kernel<<<sblocks, STAT_THREADS, 0, st>>>(ca);
+  stats_rank_kernel<<<sblocks, STAT_THREADS, 0, st>>>(cls, key, S, perm);
+  stats_gather_kernel<<<sblocks, STAT_THREADS, 0, st>>>(perm, cls, offset_samples, nhi_samples, S, m, sorted_offset,
+                                                        sorted_nhi, rank, class_start);
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess)
+    e = staged ? cudaFuncSetAttribute(dla_stats_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+               : cudaFuncSetAttribute(dla_stats_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  for (int64_t q0 = 0; q0 < Q && e == cudaSuccess; q0 += chunk) {
+    const int64_t nq = std::min(chunk, Q - q0);
+    a.q0 = q0;
+    if (staged) dla_stats_kernel<true><<<(unsigned)nq, STAT_THREADS, smem, st>>>(a);
+    else dla_stats_kernel<false><<<(unsigned)nq, STAT_THREADS, smem, st>>>(a);
+    const int64_t b0 = q0 / COL_ROWS;
+    column_partial_kernel<<<dim3((unsigned)((W + COL_THREADS - 1) / COL_THREADS), (unsigned)((nq + COL_ROWS - 1) / COL_ROWS)),
+                            COL_THREADS, 0, st>>>(rows, nq, (int)W, COL_MEAN, nullptr, psum + b0 * W, pcnt + b0 * W);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) {
+    stats_finish_kernel<<<(unsigned)((W + 127) / 128), 128, 0, st>>>(psum, (int)nblocks, W, sums);
+    e = cudaGetLastError();
+  }
+  const cudaError_t ef = cudaFreeAsync(base, st);   // freed on the error path too
+  if (e == cudaSuccess) e = ef;
+  if (e != cudaSuccess) { g_err = std::string(fn) + ": " + cudaGetErrorString(e); return GPDLA_ERR_CUDA; }
+  return GPDLA_OK;
+}
+
+int gpdla_dla_statistics(int64_t Q, int64_t S, const double* sample_log_likelihoods_dla, const double* p_dlas,
+                         const double* min_z_dlas, const double* max_z_dlas, const uint8_t* select,
+                         const double* offset_samples, const double* log_nhi_samples, const double* nhi_samples,
+                         int32_t n_z, const double* z_edges, int32_t n_nhi, const double* log_nhi_edges,
+                         double dla_log_nhi_min, double omega_m, double* sums) {
+  const char* fn = "gpdla_dla_statistics";
+  int rc = stats_check(fn, Q, S, sample_log_likelihoods_dla, p_dlas, min_z_dlas, max_z_dlas, offset_samples,
+                       log_nhi_samples, nhi_samples, n_z, z_edges, n_nhi, log_nhi_edges, dla_log_nhi_min, omega_m, sums);
+  if (rc) return rc;
+  const size_t QS = (size_t)Q * S, W = (size_t)stats_width(n_z, n_nhi), Sb = (size_t)S * 8;
+  const size_t bytes = QS * 8 + (size_t)Q * (3 * 8 + 1) + 3 * Sb + W * 8 + 6 * 64;
+  char* base = nullptr;
+  CUDA_TRY(cudaMalloc(&base, bytes), g_err);
+  char* ptr = base;
+  auto take = [&](size_t n) { char* r = ptr; ptr += (n + 15) / 16 * 16; return r; };
+  double* d_ll = (double*)take(QS * 8); double* d_p = (double*)take((size_t)Q * 8);
+  double* d_zlo = (double*)take((size_t)Q * 8); double* d_zhi = (double*)take((size_t)Q * 8);
+  double* d_off = (double*)take(Sb); double* d_lnhi = (double*)take(Sb); double* d_nhi = (double*)take(Sb);
+  double* d_sums = (double*)take(W * 8);
+  uint8_t* d_sel = select ? (uint8_t*)take((size_t)Q) : nullptr;
+  cudaError_t e = cudaSuccess;
+  auto up = [&](void* d, const void* h, size_t n) { if (e == cudaSuccess && n) e = cudaMemcpy(d, h, n, cudaMemcpyHostToDevice); };
+  up(d_ll, sample_log_likelihoods_dla, QS * 8); up(d_p, p_dlas, (size_t)Q * 8); up(d_zlo, min_z_dlas, (size_t)Q * 8);
+  up(d_zhi, max_z_dlas, (size_t)Q * 8); up(d_off, offset_samples, Sb); up(d_lnhi, log_nhi_samples, Sb);
+  up(d_nhi, nhi_samples, Sb); up(d_sums, sums, W * 8);
+  if (d_sel) up(d_sel, select, (size_t)Q);
+  rc = GPDLA_ERR_CUDA;
+  if (e == cudaSuccess) {
+    rc = gpdla_dla_statistics_device(Q, S, d_ll, d_p, d_zlo, d_zhi, d_sel, d_off, d_lnhi, d_nhi, n_z, z_edges, n_nhi,
+                                     log_nhi_edges, dla_log_nhi_min, omega_m, d_sums, nullptr);
+    if (rc == GPDLA_OK) e = cudaMemcpy(sums, d_sums, W * 8, cudaMemcpyDeviceToHost);
+  }
+  if (e != cudaSuccess) { g_err = std::string(fn) + ": " + cudaGetErrorString(e); rc = GPDLA_ERR_CUDA; }
   cudaFree(base);
   return rc;
 }

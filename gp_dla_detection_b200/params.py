@@ -62,3 +62,14 @@ all_oscillator_strengths = np.array([                # :111-143
     0.000114, 0.000101, 0.000089, 0.000080, 0.000071, 0.000064, 0.000058, 0.000053, 0.000048])
 all_transition_wavelengths.flags.writeable = False
 all_oscillator_strengths.flags.writeable = False
+
+# ---- population statistics of the single-DLA catalogue (CDDF_analysis/calc_cddf.py; api.dla_statistics_sums,
+# api.finish_dla_statistics).  Flat LambdaCDM with Omega_Lambda = 1 - omega_m and no radiation.  The defaults
+# omega_m = 0.3, hubble_h = 0.7 are this package's choice: they are not checked against calc_cddf.py.
+omega_m = 0.3
+hubble_h = 0.7                                       # H0 = 100 h km/s/Mpc
+dla_log_nhi_min = 20.3                               # a sample is a DLA where log10 N_HI >= this
+gravitational_constant = 6.67430e-8                  # cm^3 g^-1 s^-2, CODATA 2018
+speed_of_light_cgs = 2.99792458e10                   # cm/s
+hydrogen_mass = 1.6735575e-24                        # g, m_H (the hydrogen atom; no helium correction anywhere)
+megaparsec = 3.0856775814913673e24                   # cm

@@ -6,7 +6,8 @@ is a contiguous partition of the catalogue balanced by per-quasar cost (number o
 modelled window x samples); every rank (one process per GPU) runs the hot path on its block with
 no data-path collective, and ONE ``all_gather`` of fixed-width per-quasar records (NCCL over
 NVLink on GPUs, gloo in CPU tests) reassembles the catalogue.  ``sample_log_likelihoods_dla``
-(80 KB/quasar) stays sharded.
+(80 KB/quasar) stays sharded; ``dla_statistics_sharded`` reduces it to the population-statistics sums on the rank
+that produced it and gathers only those (a few KB).
 """
 from __future__ import annotations
 
@@ -114,3 +115,83 @@ def process_qsos_sharded(model: Dict, samples: Dict, spectra: Dict, prior: Dict,
     out = unpack_records(full)
     out["blocks"] = blocks
     return out
+
+
+def gather_sums(local: np.ndarray, device=None) -> np.ndarray:
+    """One all_gather of every rank's fixed-width sums vector, added in rank order: every rank gets the same bits."""
+    import torch
+    import torch.distributed as dist
+    world = dist.get_world_size()
+    buf = torch.from_numpy(np.ascontiguousarray(local, dtype=np.float64)).to(device or "cpu")
+    out = torch.empty(world * buf.numel(), dtype=torch.float64, device=buf.device)
+    dist.all_gather_into_tensor(out, buf)
+    parts = out.cpu().numpy().reshape(world, buf.numel())
+    total = parts[0].copy()
+    for r in range(1, world):
+        total += parts[r]
+    return total
+
+
+def dla_statistics_sharded(model: Dict, samples: Dict, spectra: Dict, prior: Dict, z_edges, log_nhi_edges,
+                           select=None, params=None, batch_quasars: int = 4096, dla_log_nhi_min: float = None,
+                           omega_m: float = None, hubble_h: float = None,
+                           compute: Callable[[Dict, np.ndarray, np.ndarray], np.ndarray] = None, device=None) -> Dict:
+    """Population statistics (``api.finish_dla_statistics``) of the whole catalogue on every rank.  Every rank calls
+    this with the FULL catalogue description (and ``select`` [Q], optional); rank r runs its cost-balanced block through
+    ``process_device`` in batches of ``batch_quasars`` and accumulates the sums on its GPU with ``statistics_device``;
+    one ``all_gather`` of the fixed-width vector follows, added in rank order.  The bits depend on the batch split and
+    the world size (they set the summation order); repeated runs with the same ones are identical.  ``compute(spectra,
+    select, sums) -> sums`` replaces the CUDA path of one rank (tests inject a CPU stand-in); the CUDA path keeps the
+    sums on the GPU between batches.  Returns the finished
+    dict plus ``sums`` and ``blocks``."""
+    import torch.distributed as dist
+    from . import params as P
+    from .api import dla_statistics_width, finish_dla_statistics
+    dla_log_nhi_min = P.dla_log_nhi_min if dla_log_nhi_min is None else dla_log_nhi_min
+    omega_m = P.omega_m if omega_m is None else omega_m
+    hubble_h = P.hubble_h if hubble_h is None else hubble_h
+    rank, world = dist.get_rank(), dist.get_world_size()
+    blocks = partition_by_cost(quasar_costs(spectra), world)
+    s, e = blocks[rank]
+    Q = len(spectra["z_qsos"])
+    sel = np.ones(Q, dtype=bool) if select is None else np.asarray(select, dtype=bool).ravel()
+    width = dla_statistics_width(len(z_edges) - 1, len(log_nhi_edges) - 1)
+    if compute is None:
+        compute = _device_statistics(model, samples, prior, params, z_edges, log_nhi_edges, dla_log_nhi_min, omega_m)
+    local = np.zeros(width)
+    for b0 in range(s, e, max(int(batch_quasars), 1)):
+        b1 = min(e, b0 + max(int(batch_quasars), 1))
+        local = compute(slice_spectra(spectra, b0, b1), sel[b0:b1], local)
+    if hasattr(local, "cpu"):
+        local = local.cpu().numpy()
+    total = gather_sums(np.asarray(local, dtype=np.float64), device=device)
+    out = finish_dla_statistics(total, z_edges, log_nhi_edges, hubble_h=hubble_h)
+    out["sums"] = total
+    out["blocks"] = blocks
+    return out
+
+
+def _device_statistics(model, samples, prior, params, z_edges, log_nhi_edges, dla_log_nhi_min, omega_m):
+    """The CUDA path of one rank: spectra -> process_device -> statistics_device into one device sums tensor."""
+    import os
+    import torch
+    from .api import DLAProcessor, pad_spectra
+    from .params import DEFAULT
+    dev = int(os.environ.get("LOCAL_RANK", 0))
+    proc = DLAProcessor(model, samples, prior, params or DEFAULT, device=dev)
+    state = {}
+
+    def compute(sp, sel, sums):
+        pad = pad_spectra(sp)
+        d = torch.device("cuda", dev)
+        up = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dtype=dt)).to(d)
+        if "sums" not in state:
+            state["sums"] = up(sums, np.float64)
+        out = proc.process_device(up(pad["wavelengths"], np.float64), up(pad["flux"], np.float64),
+                                  up(pad["noise_variance"], np.float64), up(pad["pixel_mask"], np.uint8),
+                                  up(pad["lengths"], np.int32), up(pad["z_qsos"], np.float64),
+                                  return_sample_log_likelihoods=True)
+        proc.statistics_device(out, z_edges, log_nhi_edges, select=up(sel, np.uint8), sums=state["sums"],
+                               dla_log_nhi_min=dla_log_nhi_min, omega_m=omega_m)
+        return state["sums"]
+    return compute

@@ -291,6 +291,34 @@ int gpdla_training_set_lyseries_device(int64_t N, int64_t L_max, const double* w
 int gpdla_row_nanmedian_fill(int64_t N, int32_t P, const double* X, double* out);
 int gpdla_row_nanmedian_fill_device(int64_t N, int32_t P, const double* X, double* out, void* stream);
 
+/* Population statistics of the single-DLA catalogue (the additive sums behind CDDF_analysis/calc_cddf.py: column density
+ * distribution, dN/dX, Omega_DLA; Bird, Garnett & Ho 2017) from one gpdla_process_qsos call's outputs with the same
+ * samples: sample_log_likelihoods_dla [Q x S], p_dlas, min_z_dlas, max_z_dlas [Q], the nullable uint8 mask `select`
+ * [Q], and offset_samples, log_nhi_samples, nhi_samples [S].  Quasar i contributes iff select[i] (default 1),
+ * isfinite(p_dlas[i]), max_z > min_z and its row's log-sum-exp is finite; w_ij is its normalised sample posterior,
+ * z_ij = min_z + (max_z - min_z) offset_j rounded as map_z_dlas, bins are half-open [lo, hi).  `sums` (in/out, float64,
+ * 2 n_z n_nhi + 5 n_z + 1 entries) is ADDED to, in this layout:
+ *   counts[n_z][n_nhi] = sum q, counts_var[n_z][n_nhi] = sum q(1-q), q = p sum_j w_j [z_j in b, log N_j in c]
+ *   dla[n_z] = sum d, dla_var[n_z] = sum d(1-d), d = p sum_j w_j [z_j in b, log N_j >= dla_log_nhi_min]
+ *   nhi[n_z] = sum e, nhi_var[n_z] = sum (e2 - e^2), e = p sum_j w_j N_j [...], e2 = p sum_j w_j N_j^2 [...]
+ *   path[n_z] = sum dX, flat LambdaCDM X(z) = 2 / (3 omega_m) sqrt(omega_m (1+z)^3 + 1 - omega_m), clipped to
+ *               [min_z, max_z] of each quasar;   num_quasars.
+ * Sums of disjoint sets of quasars add; variances add across quasars, never across z bins (one quasar's cells are
+ * exclusive), so an all-z statistic needs one z bin.  z_edges [n_z + 1], log_nhi_edges [n_nhi + 1]: host arrays,
+ * finite and strictly increasing; 1 <= n_z <= 64, 1 <= n_nhi <= 128, omega_m in (0, 1], else GPDLA_ERR_INVALID before
+ * any CUDA call.  No atomics: repeated calls give the same bits.  Context-free, on the current device; the _device entry
+ * takes device arrays and is asynchronous on `stream`, the other entry host arrays. */
+int gpdla_dla_statistics(int64_t Q, int64_t S, const double* sample_log_likelihoods_dla, const double* p_dlas,
+                         const double* min_z_dlas, const double* max_z_dlas, const uint8_t* select,
+                         const double* offset_samples, const double* log_nhi_samples, const double* nhi_samples,
+                         int32_t n_z, const double* z_edges, int32_t n_nhi, const double* log_nhi_edges,
+                         double dla_log_nhi_min, double omega_m, double* sums);
+int gpdla_dla_statistics_device(int64_t Q, int64_t S, const double* sample_log_likelihoods_dla, const double* p_dlas,
+                                const double* min_z_dlas, const double* max_z_dlas, const uint8_t* select,
+                                const double* offset_samples, const double* log_nhi_samples, const double* nhi_samples,
+                                int32_t n_z, const double* z_edges, int32_t n_nhi, const double* log_nhi_edges,
+                                double dla_log_nhi_min, double omega_m, double* sums, void* stream);
+
 /* voigt.c:253-304: profile has num_points - 6 entries.  Host buffers; runs on the current device. */
 int gpdla_voigt(const double* lambdas, int64_t num_points, double z, double N, int32_t num_lines, double* profile);
 /* Batched, device buffers: profile[s, :] = voigt(lambdas, z[s], N[s], num_lines), [S x (num_points-6)] */
