@@ -123,6 +123,13 @@ SYMBOLS = {
     "gpdla_dla_statistics_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64] + [ctypes.c_void_p] * 8
                                     + [ctypes.c_int32, c_double_p, ctypes.c_int32, c_double_p, ctypes.c_double,
                                        ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]),
+    "gpdla_multi_dla_statistics": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64, ctypes.c_int32] + [ctypes.c_void_p] * 9
+                                   + [ctypes.c_int32, c_double_p, ctypes.c_int32, c_double_p, ctypes.c_double,
+                                      ctypes.c_double, ctypes.c_void_p]),
+    "gpdla_multi_dla_statistics_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64, ctypes.c_int32]
+                                          + [ctypes.c_void_p] * 9
+                                          + [ctypes.c_int32, c_double_p, ctypes.c_int32, c_double_p, ctypes.c_double,
+                                             ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]),
 }
 
 _lib = None

@@ -256,6 +256,73 @@ class DLAProcessor:
             ctypes.c_void_p(stream)), self._ctx)
         return out
 
+    def process_multi_device(self, wavelengths, flux, noise_variance, pixel_mask, lengths, z_qsos, max_dlas: int = 4,
+                             base_sample_inds=None, return_samples: bool = False, out: Optional[Dict] = None) -> Dict:
+        """The device-resident twin of ``process_multi``: inputs as ``process_device`` takes them, CUDA tensors out, in
+        the C layout -- ``model_posteriors`` [Q, 2 + max_dlas], ``MAP_*`` [Q, max_dlas, max_dlas] and, with
+        ``return_samples``, ``sample_log_likelihoods_dla`` [Q, max_dlas, S], ``sample_log_likelihoods_lls`` [Q, S] and
+        ``base_sample_inds`` [Q, max_dlas - 1, S] (int32, 0-based).  ``base_sample_inds`` given as input (an int32 CUDA
+        tensor [Q, max_dlas - 1, S]) replaces the built-in resampling.  Asynchronous on torch's current stream."""
+        import torch
+        if not self.has_lls:
+            raise ValueError("samples must hold lls_nhi_samples, Z_lls and Z_dla for the multi-DLA path")
+        MD = int(max_dlas)
+        if not 1 <= MD <= 4:
+            raise ValueError("max_dlas must lie in [1, 4]")
+        Q, L_max = wavelengths.shape
+        dev = wavelengths.device
+        assert dev.type == "cuda" and dev.index == self.device
+        for t, dt in ((wavelengths, torch.float64), (flux, torch.float64), (noise_variance, torch.float64),
+                      (pixel_mask, torch.uint8), (lengths, torch.int32), (z_qsos, torch.float64)):
+            assert t.is_cuda and t.dtype == dt and t.is_contiguous()
+        S = self.num_dla_samples
+        if out is None:
+            shapes = dict(log_priors_dla=(Q, MD), log_likelihoods_dla=(Q, MD), log_posteriors_dla=(Q, MD),
+                          model_posteriors=(Q, MD + 2), MAP_z_dlas=(Q, MD, MD), MAP_log_nhis=(Q, MD, MD))
+            out = {n: torch.empty(shapes.get(n, (Q,)), dtype=torch.float64, device=dev)
+                   for n in _lib.MULTI_RESULT_FIELDS[:17]}
+            out["MAP_inds"] = torch.empty((Q, MD, MD), dtype=torch.int64, device=dev)
+            if return_samples:
+                out["sample_log_likelihoods_dla"] = torch.full((Q, MD, S), float("nan"), dtype=torch.float64, device=dev)
+                out["sample_log_likelihoods_lls"] = torch.full((Q, S), float("nan"), dtype=torch.float64, device=dev)
+                out["base_sample_inds"] = torch.zeros((Q, MD - 1, S), dtype=torch.int32, device=dev)
+        res = _lib.GpdlaMultiResults()
+        for n in _lib.MULTI_RESULT_FIELDS:
+            setattr(res, n, out[n].data_ptr() if n in out and out[n].numel() else None)
+        bin_ = None
+        if base_sample_inds is not None and MD > 1:
+            if not (base_sample_inds.is_cuda and base_sample_inds.dtype == torch.int32
+                    and tuple(base_sample_inds.shape) == (Q, MD - 1, S)):
+                raise ValueError("base_sample_inds must be an int32 CUDA tensor [Q, max_dlas - 1, S]")
+            # the device entry reads given indices with a stride of 3 S per quasar, as its workspace holds them
+            bin_ = torch.zeros((Q, 3, S), dtype=torch.int32, device=dev)
+            bin_[:, :MD - 1] = base_sample_inds
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(self._lib.gpdla_process_qsos_multi_device(
+            self._ctx, Q, L_max, wavelengths.data_ptr(), flux.data_ptr(), noise_variance.data_ptr(),
+            pixel_mask.data_ptr(), lengths.data_ptr(), z_qsos.data_ptr(), MD,
+            None if bin_ is None else bin_.data_ptr(), ctypes.byref(res), ctypes.c_void_p(stream)), self._ctx)
+        return out
+
+    def _stats_operands(self, dev, Q: int, S: int, width: int, select, sums):
+        """Device samples (copied once), the sums tensor to add into and the uint8 select mask of a statistics call."""
+        import torch
+        if S != self.num_dla_samples:
+            raise ValueError("sample_log_likelihoods_dla has %d samples, this processor %d" % (S, self.num_dla_samples))
+        if self._samples_device is None:
+            self._samples_device = tuple(torch.from_numpy(a).to(dev) for a in self._samples_host)
+        if sums is None:
+            sums = torch.zeros(width, dtype=torch.float64, device=dev)
+        if not (sums.is_cuda and sums.device == dev and sums.dtype == torch.float64 and sums.is_contiguous()
+                and sums.numel() == width):
+            raise ValueError("sums must be a contiguous float64 CUDA tensor of %d entries on %s" % (width, dev))
+        sel = None
+        if select is not None:
+            sel = select.to(device=dev, dtype=torch.uint8).contiguous()
+            if sel.shape != (Q,):
+                raise ValueError("select must have one entry per quasar")
+        return self._samples_device, sums, sel
+
     def statistics_device(self, out: Dict, z_edges, log_nhi_edges, select=None, sums=None,
                           dla_log_nhi_min: float = _params.dla_log_nhi_min, omega_m: float = _params.omega_m):
         """Population-statistics sums (``dla_statistics_sums``) of what ``process_device(...,
@@ -269,29 +336,49 @@ class DLAProcessor:
             raise ValueError("statistics_device needs process_device(..., return_sample_log_likelihoods=True)")
         dev = ll.device
         Q, S = ll.shape
-        if S != self.num_dla_samples:
-            raise ValueError("sample_log_likelihoods_dla has %d samples, this processor %d" % (S, self.num_dla_samples))
         ze, ne = _stats_edges(z_edges, log_nhi_edges)
-        width = dla_statistics_width(ze.size - 1, ne.size - 1)
-        if self._samples_device is None:
-            self._samples_device = tuple(torch.from_numpy(a).to(dev) for a in self._samples_host)
-        if sums is None:
-            sums = torch.zeros(width, dtype=torch.float64, device=dev)
-        if not (sums.is_cuda and sums.device == dev and sums.dtype == torch.float64 and sums.is_contiguous()
-                and sums.numel() == width):
-            raise ValueError("sums must be a contiguous float64 CUDA tensor of %d entries on %s" % (width, dev))
-        sel = None
-        if select is not None:
-            sel = select.to(device=dev, dtype=torch.uint8).contiguous()
-            if sel.shape != (Q,):
-                raise ValueError("select must have one entry per quasar")
+        (off, lnhi, nhi), sums, sel = self._stats_operands(dev, Q, S, dla_statistics_width(ze.size - 1, ne.size - 1),
+                                                           select, sums)
         ptr = lambda t: None if t is None else ctypes.c_void_p(t.data_ptr())
-        off, lnhi, nhi = self._samples_device
         with torch.cuda.device(dev):
             stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
             _lib.check(self._lib.gpdla_dla_statistics_device(
                 Q, S, ptr(ll), ptr(out["p_dlas"]), ptr(out["min_z_dlas"]), ptr(out["max_z_dlas"]), ptr(sel), ptr(off),
                 ptr(lnhi), ptr(nhi), ze.size - 1, _dp(ze), ne.size - 1, _dp(ne), float(dla_log_nhi_min),
+                float(omega_m), ptr(sums), stream))
+        return sums
+
+    def multi_statistics_device(self, out: Dict, z_edges, log_nhi_edges, select=None, sums=None,
+                                dla_log_nhi_min: float = _params.dla_log_nhi_min, omega_m: float = _params.omega_m):
+        """Population-statistics sums of the multi-DLA model (``multi_dla_statistics_sums``) of what
+        ``process_multi_device(..., return_samples=True)`` returned, without the per-sample arrays leaving the GPU.
+        ``select``: optional CUDA bool / uint8 tensor [Q]; ``sums``: a float64 CUDA tensor to add into (a new zero
+        vector when None).  Returns the sums tensor; asynchronous on torch's current stream.  Uses device copies of this
+        processor's samples, made once."""
+        import torch
+        ll = out.get("sample_log_likelihoods_dla")
+        if ll is None:
+            raise ValueError("multi_statistics_device needs process_multi_device(..., return_samples=True)")
+        dev = ll.device
+        Q, J, S = ll.shape
+        part = out.get("base_sample_inds")
+        if J > 1 and (part is None or tuple(part.shape) != (Q, J - 1, S) or part.dtype != torch.int32
+                      or not part.is_contiguous()):
+            raise ValueError("base_sample_inds must be a contiguous int32 tensor [Q, max_dlas - 1, S]")
+        if tuple(out["model_posteriors"].shape) != (Q, J + 2):
+            raise ValueError("model_posteriors must be [Q, 2 + max_dlas]")
+        if not all(out[n].is_contiguous() for n in ("sample_log_likelihoods_dla", "model_posteriors", "min_z_dlas",
+                                                    "max_z_dlas")):
+            raise ValueError("the arrays of process_multi_device must be contiguous")
+        ze, ne = _stats_edges(z_edges, log_nhi_edges)
+        (off, lnhi, nhi), sums, sel = self._stats_operands(dev, Q, S, dla_statistics_width(ze.size - 1, ne.size - 1),
+                                                           select, sums)
+        ptr = lambda t: None if t is None else ctypes.c_void_p(t.data_ptr())
+        with torch.cuda.device(dev):
+            stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+            _lib.check(self._lib.gpdla_multi_dla_statistics_device(
+                Q, S, J, ptr(ll), ptr(part if J > 1 else None), ptr(out["model_posteriors"]), ptr(out["min_z_dlas"]), ptr(out["max_z_dlas"]), ptr(sel),
+                ptr(off), ptr(lnhi), ptr(nhi), ze.size - 1, _dp(ze), ne.size - 1, _dp(ne), float(dla_log_nhi_min),
                 float(omega_m), ptr(sums), stream))
         return sums
 
@@ -889,6 +976,50 @@ def dla_statistics_sums(results: Dict, samples: Dict, z_edges, log_nhi_edges, se
                                             float(omega_m), vp(out)))
     return out
 
+
+def multi_dla_statistics_sums(results: Dict, samples: Dict, z_edges, log_nhi_edges, select=None, sums=None,
+                              dla_log_nhi_min: float = _params.dla_log_nhi_min, omega_m: float = _params.omega_m,
+                              device: int = 0) -> np.ndarray:
+    """``dla_statistics_sums`` for the multi-DLA model (Ho et al. 2021), computed on the GPU, from one
+    ``process_multi`` / ``process_qsos_multiple_dlas_meanflux`` result in the reference layout --
+    ``sample_log_likelihoods_dla`` (Q, S, J), ``base_sample_inds`` (Q, S, J-1), 0-based, ``model_posteriors``
+    (Q, 2 + J) -- and the samples it was run with.  Each quasar adds the exact mean and variance, under its model
+    mixture, of the number of absorbers per cell (and of the N_HI sum per z bin); a j-DLA sample places j absorbers,
+    the sub-DLA model none.  Same layout, ``select``, ``sums`` and finishing as ``dla_statistics_sums``."""
+    import torch
+    lib = _lib.load()
+    ze, ne = _stats_edges(z_edges, log_nhi_edges)
+    width = dla_statistics_width(ze.size - 1, ne.size - 1)
+    sll = np.asarray(results["sample_log_likelihoods_dla"], dtype=np.float64)
+    if sll.ndim != 3:
+        raise ValueError("sample_log_likelihoods_dla must be (Q, S, max_dlas)")
+    Q, S, J = sll.shape
+    ll = np.ascontiguousarray(np.transpose(sll, (0, 2, 1)))
+    part = None
+    if J > 1:
+        bsi = np.asarray(results["base_sample_inds"])
+        if bsi.shape != (Q, S, J - 1):
+            raise ValueError("base_sample_inds must be (Q, S, max_dlas - 1)")
+        part = np.ascontiguousarray(np.transpose(bsi, (0, 2, 1)), dtype=np.int32)
+    mp = _f64(results["model_posteriors"])
+    zlo, zhi = (_f64(results[n]).ravel() for n in ("min_z_dlas", "max_z_dlas"))
+    off, lnhi, nhi = (_f64(samples[k]).ravel() for k in ("offset_samples", "log_nhi_samples", "nhi_samples"))
+    if mp.shape != (Q, J + 2) or zlo.size != Q or zhi.size != Q or off.size != S or lnhi.size != S or nhi.size != S:
+        raise ValueError("results need Q entries per quasar and the samples S entries each (Q, S = %d, %d)" % (Q, S))
+    sel = None
+    if select is not None:
+        sel = np.ascontiguousarray(np.asarray(select).astype(np.uint8)).ravel()
+        if sel.size != Q:
+            raise ValueError("select must have one entry per quasar")
+    out = np.zeros(width) if sums is None else _f64(sums).ravel().copy()
+    if out.size != width:
+        raise ValueError("sums must have %d entries" % width)
+    vp = lambda a: None if a is None else ctypes.c_void_p(a.ctypes.data)
+    with torch.cuda.device(device):
+        _lib.check(lib.gpdla_multi_dla_statistics(Q, S, J, vp(ll), vp(part), vp(mp), vp(zlo), vp(zhi), vp(sel), vp(off),
+                                                  vp(lnhi), vp(nhi), ze.size - 1, _dp(ze), ne.size - 1, _dp(ne),
+                                                  float(dla_log_nhi_min), float(omega_m), vp(out)))
+    return out
 
 def omega_dla_coefficient(hubble_h: float = _params.hubble_h) -> float:
     """8 pi G m_H / (3 c H0) in cm^2: Omega_DLA = this x (sum of N_HI) / (absorption path).  HI only, no helium."""

@@ -1907,6 +1907,52 @@ static int stats_check(const char* fn, int64_t Q, int64_t S, const double* ll, c
   return GPDLA_OK;
 }
 
+// log-N class boundaries: the union of the bin edges and the DLA threshold, ascending and distinct
+static std::vector<double> stats_bounds(const double* log_nhi_edges, int32_t n_nhi, double dla_log_nhi_min) {
+  std::vector<double> bound(log_nhi_edges, log_nhi_edges + n_nhi + 1);
+  bound.push_back(dla_log_nhi_min);
+  std::sort(bound.begin(), bound.end());
+  bound.erase(std::unique(bound.begin(), bound.end()), bound.end());
+  return bound;
+}
+
+// the 1-based class whose lower boundary is v (v is one of the boundaries)
+static int stats_class_of(const std::vector<double>& bound, double v) {
+  return (int)(std::lower_bound(bound.begin(), bound.end(), v) - bound.begin()) + 1;
+}
+
+// Per-quasar rows of cell values -> sums.  launch(q0, nq, rows) enqueues the rows of quasars [q0, q0 + nq).  The rows
+// are reduced over fixed COL_ROWS-row blocks; a chunk of quasars is a whole number of blocks, so the chunking (at most
+// 256 MB of rows at a time) does not change the summation order.  The blocks are then added in order into `sums`.
+extern "C++" {
+template <class Launch>
+static cudaError_t stats_rows_to_sums(int64_t Q, int64_t W, double* sums, cudaStream_t st, Launch launch) {
+  const int64_t nblocks = (Q + COL_ROWS - 1) / COL_ROWS;
+  const int64_t chunk = std::min(nblocks * COL_ROWS,
+                                 std::max<int64_t>(COL_ROWS, ((256ll << 20) / (W * 8)) / COL_ROWS * COL_ROWS));
+  char* base = nullptr;
+  cudaError_t e = cudaMallocAsync(&base, (size_t)chunk * W * 8 + (size_t)nblocks * W * (8 + 4), st);
+  if (e != cudaSuccess) return e;
+  double* rows = (double*)base;
+  double* psum = rows + (size_t)chunk * W;
+  int32_t* pcnt = (int32_t*)(psum + (size_t)nblocks * W);
+  for (int64_t q0 = 0; q0 < Q && e == cudaSuccess; q0 += chunk) {
+    const int64_t nq = std::min(chunk, Q - q0);
+    launch(q0, nq, rows);
+    const int64_t b0 = q0 / COL_ROWS;
+    column_partial_kernel<<<dim3((unsigned)((W + COL_THREADS - 1) / COL_THREADS), (unsigned)((nq + COL_ROWS - 1) / COL_ROWS)),
+                            COL_THREADS, 0, st>>>(rows, nq, (int)W, COL_MEAN, nullptr, psum + b0 * W, pcnt + b0 * W);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) {
+    stats_finish_kernel<<<(unsigned)((W + 127) / 128), 128, 0, st>>>(psum, (int)nblocks, W, sums);
+    e = cudaGetLastError();
+  }
+  const cudaError_t ef = cudaFreeAsync(base, st);   // freed on the error path too
+  return e == cudaSuccess ? ef : e;
+}
+}  // extern "C++"
+
 int gpdla_dla_statistics_device(int64_t Q, int64_t S, const double* sample_log_likelihoods_dla, const double* p_dlas,
                                 const double* min_z_dlas, const double* max_z_dlas, const uint8_t* select,
                                 const double* offset_samples, const double* log_nhi_samples, const double* nhi_samples,
@@ -1919,12 +1965,8 @@ int gpdla_dla_statistics_device(int64_t Q, int64_t S, const double* sample_log_l
   if (Q == 0) return GPDLA_OK;
   cudaStream_t st = (cudaStream_t)stream;
   // log-N classes: the intervals between the union of the bin edges and the DLA threshold
-  std::vector<double> bound(log_nhi_edges, log_nhi_edges + n_nhi + 1);
-  bound.push_back(dla_log_nhi_min);
-  std::sort(bound.begin(), bound.end());
-  bound.erase(std::unique(bound.begin(), bound.end()), bound.end());
+  const std::vector<double> bound = stats_bounds(log_nhi_edges, n_nhi, dla_log_nhi_min);
   const int m = (int)bound.size();
-  auto class_of = [&](double v) { return (int)(std::lower_bound(bound.begin(), bound.end(), v) - bound.begin()) + 1; };
   StatsClassArgs ca;
   ca.offset = offset_samples; ca.log_nhi = log_nhi_samples; ca.S = S; ca.nbound = m;
   for (int k = 0; k < m; ++k) ca.bound[k] = bound[k];
@@ -1933,10 +1975,10 @@ int gpdla_dla_statistics_device(int64_t Q, int64_t S, const double* sample_log_l
   a.select = select; a.S = S; a.n_z = n_z; a.n_nhi = n_nhi; a.nbound = m; a.W = stats_width(n_z, n_nhi);
   for (int e = 0; e <= n_z; ++e) a.z_edges[e] = z_edges[e];
   for (int c = 0; c < n_nhi; ++c) {
-    a.nhi_class0[c] = (int16_t)class_of(log_nhi_edges[c]);
-    a.nhi_class1[c] = (int16_t)class_of(log_nhi_edges[c + 1]);
+    a.nhi_class0[c] = (int16_t)stats_class_of(bound, log_nhi_edges[c]);
+    a.nhi_class1[c] = (int16_t)stats_class_of(bound, log_nhi_edges[c + 1]);
   }
-  a.dla_class0 = class_of(dla_log_nhi_min);
+  a.dla_class0 = stats_class_of(bound, dla_log_nhi_min);
   a.omega_m = omega_m; a.omega_l = 1.0 - omega_m; a.x_coef = 2.0 / (3.0 * omega_m);
   const int64_t W = a.W;
   int dev = 0, optin = 0;
@@ -1944,25 +1986,17 @@ int gpdla_dla_statistics_device(int64_t Q, int64_t S, const double* sample_log_l
   CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev), g_err);
   const bool staged = stats_smem_bytes(true, S, n_z, m) + STAT_THREADS / 32 * 8 + 64 <= (size_t)optin;
   const size_t smem = stats_smem_bytes(staged, S, n_z, m);
-  // rows of per-quasar cell values are reduced over fixed COL_ROWS-row blocks; a chunk of quasars is a whole number of
-  // blocks, so the chunking (at most 256 MB of rows at a time) does not change the summation order
-  const int64_t nblocks = (Q + COL_ROWS - 1) / COL_ROWS;
-  const int64_t chunk = std::min(nblocks * COL_ROWS,
-                                 std::max<int64_t>(COL_ROWS, ((256ll << 20) / (W * 8)) / COL_ROWS * COL_ROWS));
-  const size_t bytes = (size_t)S * (4 + 8 + 4 + 4 + 8 + 8) + (size_t)(m + 2) * 4 + (size_t)chunk * W * 8 +
-                       (size_t)nblocks * W * (8 + 4) + 8 * 64;
+  const size_t bytes = (size_t)S * (4 + 8 + 4 + 4 + 8 + 8) + (size_t)(m + 2) * 4 + 8 * 64;
   char* base = nullptr;
   CUDA_TRY(cudaMallocAsync(&base, bytes, st), g_err);
   char* ptr = base;
   auto take = [&](size_t n) { char* r = ptr; ptr += (n + 15) / 16 * 16; return r; };
   double* sorted_offset = (double*)take(S * 8); double* sorted_nhi = (double*)take(S * 8);
   uint64_t* key = (uint64_t*)take(S * 8);
-  double* rows = (double*)take((size_t)chunk * W * 8); double* psum = (double*)take((size_t)nblocks * W * 8);
   int32_t* cls = (int32_t*)take(S * 4); int32_t* perm = (int32_t*)take(S * 4); int32_t* rank = (int32_t*)take(S * 4);
-  int32_t* class_start = (int32_t*)take((m + 2) * 4); int32_t* pcnt = (int32_t*)take((size_t)nblocks * W * 4);
+  int32_t* class_start = (int32_t*)take((m + 2) * 4);
   ca.cls = cls; ca.key = key;
   a.sorted_offset = sorted_offset; a.sorted_nhi = sorted_nhi; a.perm = perm; a.rank = rank; a.class_start = class_start;
-  a.rows = rows;
   const unsigned sblocks = (unsigned)((S + STAT_THREADS - 1) / STAT_THREADS);
   stats_class_kernel<<<sblocks, STAT_THREADS, 0, st>>>(ca);
   stats_rank_kernel<<<sblocks, STAT_THREADS, 0, st>>>(cls, key, S, perm);
@@ -1972,20 +2006,12 @@ int gpdla_dla_statistics_device(int64_t Q, int64_t S, const double* sample_log_l
   if (e == cudaSuccess)
     e = staged ? cudaFuncSetAttribute(dla_stats_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
                : cudaFuncSetAttribute(dla_stats_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  for (int64_t q0 = 0; q0 < Q && e == cudaSuccess; q0 += chunk) {
-    const int64_t nq = std::min(chunk, Q - q0);
-    a.q0 = q0;
-    if (staged) dla_stats_kernel<true><<<(unsigned)nq, STAT_THREADS, smem, st>>>(a);
-    else dla_stats_kernel<false><<<(unsigned)nq, STAT_THREADS, smem, st>>>(a);
-    const int64_t b0 = q0 / COL_ROWS;
-    column_partial_kernel<<<dim3((unsigned)((W + COL_THREADS - 1) / COL_THREADS), (unsigned)((nq + COL_ROWS - 1) / COL_ROWS)),
-                            COL_THREADS, 0, st>>>(rows, nq, (int)W, COL_MEAN, nullptr, psum + b0 * W, pcnt + b0 * W);
-    e = cudaGetLastError();
-  }
-  if (e == cudaSuccess) {
-    stats_finish_kernel<<<(unsigned)((W + 127) / 128), 128, 0, st>>>(psum, (int)nblocks, W, sums);
-    e = cudaGetLastError();
-  }
+  if (e == cudaSuccess)
+    e = stats_rows_to_sums(Q, W, sums, st, [&](int64_t q0, int64_t nq, double* rows) {
+      a.q0 = q0; a.rows = rows;
+      if (staged) dla_stats_kernel<true><<<(unsigned)nq, STAT_THREADS, smem, st>>>(a);
+      else dla_stats_kernel<false><<<(unsigned)nq, STAT_THREADS, smem, st>>>(a);
+    });
   const cudaError_t ef = cudaFreeAsync(base, st);   // freed on the error path too
   if (e == cudaSuccess) e = ef;
   if (e != cudaSuccess) { g_err = std::string(fn) + ": " + cudaGetErrorString(e); return GPDLA_ERR_CUDA; }
@@ -2022,6 +2048,131 @@ int gpdla_dla_statistics(int64_t Q, int64_t S, const double* sample_log_likeliho
   if (e == cudaSuccess) {
     rc = gpdla_dla_statistics_device(Q, S, d_ll, d_p, d_zlo, d_zhi, d_sel, d_off, d_lnhi, d_nhi, n_z, z_edges, n_nhi,
                                      log_nhi_edges, dla_log_nhi_min, omega_m, d_sums, nullptr);
+    if (rc == GPDLA_OK) e = cudaMemcpy(sums, d_sums, W * 8, cudaMemcpyDeviceToHost);
+  }
+  if (e != cudaSuccess) { g_err = std::string(fn) + ": " + cudaGetErrorString(e); rc = GPDLA_ERR_CUDA; }
+  cudaFree(base);
+  return rc;
+}
+
+// ---- population statistics of the multi-DLA catalogue (Ho et al. 2021) ----
+
+// the checks both multi-DLA statistics entries make before any CUDA call: stats_check, then the level count
+static int mstats_check(const char* fn, int64_t Q, int64_t S, int32_t max_dlas, const double* ll,
+                        const int32_t* base_sample_inds, const double* model_posteriors, const double* min_z_dlas,
+                        const double* max_z_dlas, const double* offset_samples, const double* log_nhi_samples,
+                        const double* nhi_samples, int32_t n_z, const double* z_edges, int32_t n_nhi,
+                        const double* log_nhi_edges, double dla_log_nhi_min, double omega_m, const double* sums) {
+  int rc = stats_check(fn, Q, S, ll, model_posteriors, min_z_dlas, max_z_dlas, offset_samples, log_nhi_samples,
+                       nhi_samples, n_z, z_edges, n_nhi, log_nhi_edges, dla_log_nhi_min, omega_m, sums);
+  if (rc) return rc;
+  auto fail = [&](const std::string& why) { g_err = std::string(fn) + ": " + why; return GPDLA_ERR_INVALID; };
+  if (max_dlas < 1 || max_dlas > MSTAT_MAX_DLAS)
+    return fail("max_dlas = " + std::to_string(max_dlas) + " is outside [1, " + std::to_string(MSTAT_MAX_DLAS) + "]");
+  if (Q > 0 && max_dlas > 1 && !base_sample_inds) return fail("base_sample_inds may be NULL only when max_dlas == 1");
+  return GPDLA_OK;
+}
+
+int gpdla_multi_dla_statistics_device(int64_t Q, int64_t S, int32_t max_dlas, const double* sample_log_likelihoods_dla,
+                                      const int32_t* base_sample_inds, const double* model_posteriors,
+                                      const double* min_z_dlas, const double* max_z_dlas, const uint8_t* select,
+                                      const double* offset_samples, const double* log_nhi_samples,
+                                      const double* nhi_samples, int32_t n_z, const double* z_edges, int32_t n_nhi,
+                                      const double* log_nhi_edges, double dla_log_nhi_min, double omega_m,
+                                      double* sums, void* stream) {
+  const char* fn = "gpdla_multi_dla_statistics_device";
+  int rc = mstats_check(fn, Q, S, max_dlas, sample_log_likelihoods_dla, base_sample_inds, model_posteriors,
+                        min_z_dlas, max_z_dlas, offset_samples, log_nhi_samples, nhi_samples, n_z, z_edges, n_nhi,
+                        log_nhi_edges, dla_log_nhi_min, omega_m, sums);
+  if (rc) return rc;
+  if (Q == 0) return GPDLA_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  const std::vector<double> bound = stats_bounds(log_nhi_edges, n_nhi, dla_log_nhi_min);
+  const int m = (int)bound.size();
+  StatsClassArgs ca;
+  ca.offset = offset_samples; ca.log_nhi = log_nhi_samples; ca.S = S; ca.nbound = m;
+  for (int k = 0; k < m; ++k) ca.bound[k] = bound[k];
+  MultiStatsArgs a;
+  a.ll = sample_log_likelihoods_dla; a.partners = max_dlas > 1 ? base_sample_inds : nullptr;
+  a.model_posteriors = model_posteriors; a.min_z_dlas = min_z_dlas; a.max_z_dlas = max_z_dlas; a.select = select;
+  a.S = S; a.J = max_dlas; a.offset = offset_samples; a.nhi = nhi_samples;
+  a.n_z = n_z; a.n_nhi = n_nhi; a.W = stats_width(n_z, n_nhi);
+  for (int e = 0; e <= n_z; ++e) a.z_edges[e] = z_edges[e];
+  for (int k = 0; k <= m; ++k) a.class_bin[k] = -1;              // class 0: below every boundary, or NaN
+  for (int c = 0; c < n_nhi; ++c)
+    for (int k = stats_class_of(bound, log_nhi_edges[c]); k < stats_class_of(bound, log_nhi_edges[c + 1]); ++k)
+      a.class_bin[k] = (int16_t)c;
+  a.dla_class0 = stats_class_of(bound, dla_log_nhi_min);
+  a.omega_m = omega_m; a.omega_l = 1.0 - omega_m; a.x_coef = 2.0 / (3.0 * omega_m);
+  int dev = 0, optin = 0;
+  CUDA_TRY(cudaGetDevice(&dev), g_err);
+  CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev), g_err);
+  // one accumulator per warp: as many warps (up to 8) as fit; 64 x 128 bins leave one
+  const int nw = (int)std::max<int64_t>(1, std::min<int64_t>(STAT_THREADS / 32, (int64_t)(optin - 64) /
+                                                             (int64_t)mstats_smem_bytes(1, n_z, n_nhi)));
+  const size_t smem = mstats_smem_bytes(nw, n_z, n_nhi);
+  char* base = nullptr;
+  CUDA_TRY(cudaMallocAsync(&base, (size_t)S * (8 + 4) + 32, st), g_err);
+  ca.key = (uint64_t*)base;
+  ca.cls = (int32_t*)(base + (size_t)S * 8);
+  a.cls = ca.cls;
+  stats_class_kernel<<<(unsigned)((S + STAT_THREADS - 1) / STAT_THREADS), STAT_THREADS, 0, st>>>(ca);
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(multi_dla_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e == cudaSuccess)
+    e = stats_rows_to_sums(Q, a.W, sums, st, [&](int64_t q0, int64_t nq, double* rows) {
+      a.q0 = q0; a.rows = rows;
+      multi_dla_stats_kernel<<<(unsigned)nq, nw * 32, smem, st>>>(a);
+    });
+  const cudaError_t ef = cudaFreeAsync(base, st);   // freed on the error path too
+  if (e == cudaSuccess) e = ef;
+  if (e != cudaSuccess) { g_err = std::string(fn) + ": " + cudaGetErrorString(e); return GPDLA_ERR_CUDA; }
+  return GPDLA_OK;
+}
+
+int gpdla_multi_dla_statistics(int64_t Q, int64_t S, int32_t max_dlas, const double* sample_log_likelihoods_dla,
+                               const int32_t* base_sample_inds, const double* model_posteriors,
+                               const double* min_z_dlas, const double* max_z_dlas, const uint8_t* select,
+                               const double* offset_samples, const double* log_nhi_samples, const double* nhi_samples,
+                               int32_t n_z, const double* z_edges, int32_t n_nhi, const double* log_nhi_edges,
+                               double dla_log_nhi_min, double omega_m, double* sums) {
+  const char* fn = "gpdla_multi_dla_statistics";
+  int rc = mstats_check(fn, Q, S, max_dlas, sample_log_likelihoods_dla, base_sample_inds, model_posteriors,
+                        min_z_dlas, max_z_dlas, offset_samples, log_nhi_samples, nhi_samples, n_z, z_edges, n_nhi,
+                        log_nhi_edges, dla_log_nhi_min, omega_m, sums);
+  if (rc) return rc;
+  const size_t J = (size_t)max_dlas, P = max_dlas > 1 ? (size_t)Q * (J - 1) * S : 0;
+  for (size_t n = 0; n < P; ++n)
+    if (base_sample_inds[n] < 0 || base_sample_inds[n] >= S) {
+      g_err = std::string(fn) + ": base_sample_inds[" + std::to_string(n / ((J - 1) * S)) + "][" +
+              std::to_string(n / S % (J - 1)) + "][" + std::to_string(n % S) + "] = " +
+              std::to_string(base_sample_inds[n]) + " is outside [0, S)";
+      return GPDLA_ERR_INVALID;
+    }
+  const size_t QJS = (size_t)Q * J * S, W = (size_t)stats_width(n_z, n_nhi), Sb = (size_t)S * 8;
+  const size_t bytes = QJS * 8 + P * 4 + (size_t)Q * ((J + 2) * 8 + 2 * 8 + 1) + 3 * Sb + W * 8 + 8 * 64;
+  char* base = nullptr;
+  CUDA_TRY(cudaMalloc(&base, bytes), g_err);
+  char* ptr = base;
+  auto take = [&](size_t n) { char* r = ptr; ptr += (n + 15) / 16 * 16; return r; };
+  double* d_ll = (double*)take(QJS * 8); int32_t* d_part = P ? (int32_t*)take(P * 4) : nullptr;
+  double* d_mp = (double*)take((size_t)Q * (J + 2) * 8);
+  double* d_zlo = (double*)take((size_t)Q * 8); double* d_zhi = (double*)take((size_t)Q * 8);
+  double* d_off = (double*)take(Sb); double* d_lnhi = (double*)take(Sb); double* d_nhi = (double*)take(Sb);
+  double* d_sums = (double*)take(W * 8);
+  uint8_t* d_sel = select ? (uint8_t*)take((size_t)Q) : nullptr;
+  cudaError_t e = cudaSuccess;
+  auto up = [&](void* d, const void* h, size_t n) { if (e == cudaSuccess && n) e = cudaMemcpy(d, h, n, cudaMemcpyHostToDevice); };
+  up(d_ll, sample_log_likelihoods_dla, QJS * 8); up(d_part, base_sample_inds, P * 4);
+  up(d_mp, model_posteriors, (size_t)Q * (J + 2) * 8); up(d_zlo, min_z_dlas, (size_t)Q * 8);
+  up(d_zhi, max_z_dlas, (size_t)Q * 8); up(d_off, offset_samples, Sb); up(d_lnhi, log_nhi_samples, Sb);
+  up(d_nhi, nhi_samples, Sb); up(d_sums, sums, W * 8);
+  if (d_sel) up(d_sel, select, (size_t)Q);
+  rc = GPDLA_ERR_CUDA;
+  if (e == cudaSuccess) {
+    rc = gpdla_multi_dla_statistics_device(Q, S, max_dlas, d_ll, d_part, d_mp, d_zlo, d_zhi, d_sel, d_off, d_lnhi, d_nhi,
+                                           n_z, z_edges, n_nhi, log_nhi_edges, dla_log_nhi_min, omega_m, d_sums,
+                                           nullptr);
     if (rc == GPDLA_OK) e = cudaMemcpy(sums, d_sums, W * 8, cudaMemcpyDeviceToHost);
   }
   if (e != cudaSuccess) { g_err = std::string(fn) + ": " + cudaGetErrorString(e); rc = GPDLA_ERR_CUDA; }

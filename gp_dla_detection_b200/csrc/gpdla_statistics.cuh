@@ -272,4 +272,236 @@ __global__ void stats_finish_kernel(const double* __restrict__ psum, int nblocks
   sums[c] = s;
 }
 
+// ---- the multi-DLA model (Ho et al. 2021): sample i of level j (1-based) places j absorbers, slot 0 at sample i and
+// slot t at partners[t - 1][i].  A quasar's count X of a cell is then 0..J, and the row holds its exact mixture mean
+// and variance.  With v_j(i) = p_j w_ji and g_t(i) = sum_{j > t} v_j(i), E[X] = sum_i sum_t g_t a_t and
+// E[X^2] = E[X] + 2 sum_i sum_{t < t'} g_t' a_t a_t' (a_t: slot t lies in the cell; slot t' exists wherever t' does).
+//   multi_dla_stats_kernel    one CTA per quasar: per-level log-sum-exp and the partner bounds check in one pass over
+//                             the rows, then every warp takes 32 samples at a time, merges each sample's slots by
+//                             cell in registers, and adds them into a warp-private accumulator: lanes sharing a cell
+//                             (__match_any_sync) are summed in lane order by the lowest one.  The warps' accumulators
+//                             are added in warp order.  No atomics; the order depends only on the launch shape.
+constexpr int MSTAT_MAX_DLAS = 4;
+
+struct MultiStatsArgs {
+  const double* ll;                          // [Q x J x S] sample_log_likelihoods_dla
+  const int32_t* partners;                   // [Q x (J-1) x S] base_sample_inds, 0-based; nullptr when J == 1
+  const double* model_posteriors;            // [Q x (2 + J)]: no DLA, sub-DLA, 1..J DLAs
+  const double* min_z_dlas;
+  const double* max_z_dlas;
+  const uint8_t* select;                     // nullable
+  int64_t S;
+  int64_t q0;                                // first quasar of this chunk
+  int J;
+  const double* offset;                      // [S] offset_samples
+  const double* nhi;                         // [S] nhi_samples
+  const int32_t* cls;                        // [S] log-N class (stats_class_kernel)
+  int n_z, n_nhi;
+  int64_t W;                                 // stats_width(n_z, n_nhi)
+  double z_edges[STAT_MAX_Z + 1];
+  int16_t class_bin[STAT_MAX_BOUND + 1];     // log-N bin of each class, -1 outside every bin
+  int dla_class0;                            // classes >= dla_class0 are DLAs
+  double omega_m, omega_l, x_coef;
+  double* rows;                              // [chunk x W]
+};
+
+// accumulator doubles per warp: (E[X], E[X^2]) per (z bin, log-N bin) cell, then (d, d2, e, e2) per z bin
+__host__ __device__ inline int mstats_acc_width(int n_z, int n_nhi) { return 2 * n_z * n_nhi + 4 * n_z; }
+__host__ __device__ inline size_t mstats_smem_bytes(int nwarps, int n_z, int n_nhi) {
+  return (size_t)nwarps * (mstats_acc_width(n_z, n_nhi) + 32 * 4 + MSTAT_MAX_DLAS * 2) * sizeof(double);
+}
+
+// running log-sum-exp (m, s = sum exp(v - m)); NaN and -inf carry no weight, s == 0 means nothing seen
+__device__ __forceinline__ void lse_push(double& m, double& s, double v) {
+  if (!(v > -INFINITY)) return;
+  if (v > m) { s = s * exp(m - v) + 1.0; m = v; } else s += exp(v - m);
+}
+__device__ __forceinline__ void lse_merge(double& m, double& s, double m2, double s2) {   // commutative
+  if (s2 == 0.0) return;
+  if (s == 0.0) { m = m2; s = s2; return; }
+  const double mm = fmax(m, m2);
+  s = s * exp(m - mm) + s2 * exp(m2 - mm);
+  m = mm;
+}
+
+__global__ void __launch_bounds__(STAT_THREADS) multi_dla_stats_kernel(const __grid_constant__ MultiStatsArgs a) {
+  extern __shared__ __align__(16) double ms_smem[];
+  __shared__ int s_bad;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = blockDim.x >> 5;
+  const int64_t q = a.q0 + blockIdx.x, S = a.S;
+  const int J = a.J, nzn = a.n_z * a.n_nhi, A = mstats_acc_width(a.n_z, a.n_nhi);
+  double* acc = ms_smem;                                       // [nw][A]
+  double* stage = acc + (size_t)nw * A;                        // [nw][32][4]
+  double* red = stage + nw * 128;                              // [nw][MSTAT_MAX_DLAS][2]
+  double* row = a.rows + (int64_t)blockIdx.x * a.W;
+  const double* ll = a.ll + q * J * S;
+  const int32_t* part = a.partners ? a.partners + q * (J - 1) * S : nullptr;
+  const double* mp = a.model_posteriors + q * (J + 2);
+  const double zlo = a.min_z_dlas[q], zhi = a.max_z_dlas[q];
+  bool ok = (a.select ? a.select[q] != 0 : true) && zhi > zlo;
+  for (int c = 0; c < J + 2; ++c) ok = ok && isfinite(mp[c]);
+  double p[MSTAT_MAX_DLAS];
+  int jmax = 0;                                                // levels 1..jmax can contribute; partner rows < jmax - 1
+#pragma unroll
+  for (int j = 0; j < MSTAT_MAX_DLAS; ++j) {
+    p[j] = (ok && j < J) ? mp[2 + j] : 0.0;
+    if (p[j] > 0.0) jmax = j + 1;
+  }
+  if (tid == 0) s_bad = 0;
+  __syncthreads();
+  double m[MSTAT_MAX_DLAS], s[MSTAT_MAX_DLAS];
+#pragma unroll
+  for (int j = 0; j < MSTAT_MAX_DLAS; ++j) { m[j] = -INFINITY; s[j] = 0.0; }
+  if (ok) {                                                    // pass 1: per-level LSE, partner bounds
+    int bad = 0;
+    for (int64_t i = tid; i < S; i += blockDim.x) {
+      double v[MSTAT_MAX_DLAS];
+      int32_t k[MSTAT_MAX_DLAS - 1];
+#pragma unroll
+      for (int j = 0; j < MSTAT_MAX_DLAS; ++j) v[j] = p[j] > 0.0 ? ll[j * S + i] : NAN;
+#pragma unroll
+      for (int t = 0; t < MSTAT_MAX_DLAS - 1; ++t) k[t] = t + 1 < jmax ? part[t * S + i] : 0;
+#pragma unroll
+      for (int j = 0; j < MSTAT_MAX_DLAS; ++j) lse_push(m[j], s[j], v[j]);
+#pragma unroll
+      for (int t = 0; t < MSTAT_MAX_DLAS - 1; ++t) bad |= (k[t] < 0) | (k[t] >= S);
+    }
+#pragma unroll
+    for (int j = 0; j < MSTAT_MAX_DLAS; ++j)
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1)
+        lse_merge(m[j], s[j], __shfl_xor_sync(0xffffffffu, m[j], o), __shfl_xor_sync(0xffffffffu, s[j], o));
+    bad = __any_sync(0xffffffffu, bad);
+    if (lane == 0) {
+      if (bad) s_bad = 1;                                      // benign: every writer stores 1
+#pragma unroll
+      for (int j = 0; j < MSTAT_MAX_DLAS; ++j) { red[(warp * MSTAT_MAX_DLAS + j) * 2] = m[j]; red[(warp * MSTAT_MAX_DLAS + j) * 2 + 1] = s[j]; }
+    }
+  }
+  __syncthreads();
+  if (ok) {
+#pragma unroll
+    for (int j = 0; j < MSTAT_MAX_DLAS; ++j) {                 // every thread adds the warps in the same order
+      m[j] = red[j * 2]; s[j] = red[j * 2 + 1];
+      for (int w = 1; w < nw; ++w) lse_merge(m[j], s[j], red[(w * MSTAT_MAX_DLAS + j) * 2], red[(w * MSTAT_MAX_DLAS + j) * 2 + 1]);
+      if (p[j] > 0.0 && !isfinite(m[j])) ok = false;           // then s lies in [1, S]
+    }
+    ok = ok && !s_bad;
+  }
+  if (!ok) {                                                   // contributes nothing, not even path or a count
+    for (int64_t c = tid; c < a.W; c += blockDim.x) row[c] = 0.0;
+    return;
+  }
+  double sc[MSTAT_MAX_DLAS];
+#pragma unroll
+  for (int j = 0; j < MSTAT_MAX_DLAS; ++j) sc[j] = p[j] > 0.0 ? p[j] / s[j] : 0.0;
+  double* accw = acc + (size_t)warp * A;
+  double* st = stage + warp * 128;
+  for (int e = lane; e < A; e += 32) accw[e] = 0.0;
+  __syncwarp();
+  const double span = __dsub_rn(zhi, zlo);
+  for (int64_t i0 = (int64_t)warp * 32; i0 < S; i0 += (int64_t)nw * 32) {   // pass 2: 32 samples per warp step
+    const int64_t i = i0 + lane;
+    double g[MSTAT_MAX_DLAS];                                  // g[t] = sum over levels j >= t (0-based) of p_j w_ji
+#pragma unroll
+    for (int j = 0; j < MSTAT_MAX_DLAS; ++j) {
+      const double x = (i < S && sc[j] > 0.0) ? ll[j * S + i] : NAN;
+      g[j] = x == x ? exp(x - m[j]) * sc[j] : 0.0;
+    }
+#pragma unroll
+    for (int t = MSTAT_MAX_DLAS - 2; t >= 0; --t) g[t] += g[t + 1];
+    // this sample's slots merged by cell: item u is keyed by the first slot that lands in its cell
+    int xk[MSTAT_MAX_DLAS], xn[MSTAT_MAX_DLAS], dk[MSTAT_MAX_DLAS], dn[MSTAT_MAX_DLAS];
+    double xm[MSTAT_MAX_DLAS], xs[MSTAT_MAX_DLAS], dm[MSTAT_MAX_DLAS], ds[MSTAT_MAX_DLAS], de[MSTAT_MAX_DLAS],
+        de2[MSTAT_MAX_DLAS], dN[MSTAT_MAX_DLAS];
+#pragma unroll
+    for (int t = 0; t < MSTAT_MAX_DLAS; ++t) {
+      xk[t] = dk[t] = -1; xn[t] = dn[t] = 0;
+      xm[t] = xs[t] = dm[t] = ds[t] = de[t] = de2[t] = dN[t] = 0.0;
+      if (!(g[t] > 0.0)) continue;                             // g is non-increasing in t: no pair needs this slot
+      const int64_t k = t == 0 ? i : (int64_t)part[(t - 1) * S + i];   // in [0, S): checked in pass 1
+      const double z = __dadd_rn(zlo, __dmul_rn(span, a.offset[k]));
+      int lo = 0, hi = a.n_z + 1;                              // number of edges <= z
+      while (lo < hi) { const int mid = (lo + hi) >> 1; if (a.z_edges[mid] <= z) lo = mid + 1; else hi = mid; }
+      const int b = lo - 1;
+      if (b < 0 || b >= a.n_z) continue;
+      const int cl = a.cls[k], c = a.class_bin[cl];
+      const double gt = g[t];
+      if (c >= 0) {
+        const int key = b * a.n_nhi + c;
+        bool merged = false;
+#pragma unroll
+        for (int u = 0; u < t; ++u)
+          if (!merged && xk[u] == key) {                       // pairs with the xn[u] earlier slots: 2 g_t each
+            xm[u] += gt; xs[u] += gt * (double)(1 + 2 * xn[u]); xn[u] += 1; merged = true;
+          }
+        if (!merged) { xk[t] = key; xm[t] = gt; xs[t] = gt; xn[t] = 1; }
+      }
+      if (cl >= a.dla_class0) {
+        const double N = a.nhi[k], gN = gt * N;
+        bool merged = false;
+#pragma unroll
+        for (int u = 0; u < t; ++u)
+          if (!merged && dk[u] == b) {
+            dm[u] += gt; ds[u] += gt * (double)(1 + 2 * dn[u]);
+            de[u] += gN; de2[u] += gN * N + 2.0 * gN * dN[u];
+            dN[u] += N; dn[u] += 1; merged = true;
+          }
+        if (!merged) { dk[t] = b; dm[t] = gt; ds[t] = gt; de[t] = gN; de2[t] = gN * N; dN[t] = N; dn[t] = 1; }
+      }
+    }
+    // into the warp's accumulator: the lowest lane of each cell adds its lanes in lane order
+#pragma unroll
+    for (int u = 0; u < MSTAT_MAX_DLAS; ++u) {
+      if (u >= J) break;
+      unsigned grp = __match_any_sync(0xffffffffu, xk[u]);
+      st[lane * 4] = xm[u]; st[lane * 4 + 1] = xs[u];
+      __syncwarp();
+      if (xk[u] >= 0 && lane == __ffs(grp) - 1) {
+        double s0 = 0.0, s1 = 0.0;
+        for (unsigned r = grp; r; r &= r - 1) { const int l = __ffs(r) - 1; s0 += st[l * 4]; s1 += st[l * 4 + 1]; }
+        accw[2 * xk[u]] += s0; accw[2 * xk[u] + 1] += s1;
+      }
+      __syncwarp();
+      grp = __match_any_sync(0xffffffffu, dk[u]);
+      st[lane * 4] = dm[u]; st[lane * 4 + 1] = ds[u]; st[lane * 4 + 2] = de[u]; st[lane * 4 + 3] = de2[u];
+      __syncwarp();
+      if (dk[u] >= 0 && lane == __ffs(grp) - 1) {
+        double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
+        for (unsigned r = grp; r; r &= r - 1) {
+          const int l = __ffs(r) - 1;
+          s0 += st[l * 4]; s1 += st[l * 4 + 1]; s2 += st[l * 4 + 2]; s3 += st[l * 4 + 3];
+        }
+        double* d = accw + 2 * nzn + 4 * dk[u];
+        d[0] += s0; d[1] += s1; d[2] += s2; d[3] += s3;
+      }
+      __syncwarp();
+    }
+  }
+  __syncthreads();
+  for (int e = tid; e < A; e += blockDim.x) {                  // the warps in warp order, into warp 0's copy
+    double t = acc[e];
+    for (int w = 1; w < nw; ++w) t += acc[(size_t)w * A + e];
+    acc[e] = t;
+  }
+  __syncthreads();
+  for (int c = tid; c < nzn; c += blockDim.x) {
+    const double mean = acc[2 * c];
+    row[c] = mean;
+    row[nzn + c] = acc[2 * c + 1] - mean * mean;
+  }
+  double* tail = row + 2 * nzn;
+  for (int b = tid; b < a.n_z; b += blockDim.x) {
+    const double* d = acc + 2 * nzn + 4 * b;
+    tail[b] = d[0];
+    tail[a.n_z + b] = d[1] - d[0] * d[0];
+    tail[2 * a.n_z + b] = d[2];
+    tail[3 * a.n_z + b] = d[3] - d[2] * d[2];
+    const double xa = absorption_distance(fmax(a.z_edges[b], zlo), a.omega_m, a.omega_l, a.x_coef);
+    const double xb = absorption_distance(fmin(a.z_edges[b + 1], zhi), a.omega_m, a.omega_l, a.x_coef);
+    tail[4 * a.n_z + b] = fmax(0.0, xb - xa);
+  }
+  if (tid == 0) row[a.W - 1] = 1.0;
+}
+
 }  // namespace gpdla

@@ -6,8 +6,8 @@ is a contiguous partition of the catalogue balanced by per-quasar cost (number o
 modelled window x samples); every rank (one process per GPU) runs the hot path on its block with
 no data-path collective, and ONE ``all_gather`` of fixed-width per-quasar records (NCCL over
 NVLink on GPUs, gloo in CPU tests) reassembles the catalogue.  ``sample_log_likelihoods_dla``
-(80 KB/quasar) stays sharded; ``dla_statistics_sharded`` reduces it to the population-statistics sums on the rank
-that produced it and gathers only those (a few KB).
+(80 KB/quasar) stays sharded; ``dla_statistics_sharded`` (and ``multi_dla_statistics_sharded`` for the multi-DLA
+model) reduces it to the population-statistics sums on the rank that produced it and gathers only those (a few KB).
 """
 from __future__ import annotations
 
@@ -144,21 +144,43 @@ def dla_statistics_sharded(model: Dict, samples: Dict, spectra: Dict, prior: Dic
     select, sums) -> sums`` replaces the CUDA path of one rank (tests inject a CPU stand-in); the CUDA path keeps the
     sums on the GPU between batches.  Returns the finished
     dict plus ``sums`` and ``blocks``."""
+    from . import params as P
+    dla_log_nhi_min = P.dla_log_nhi_min if dla_log_nhi_min is None else dla_log_nhi_min
+    omega_m = P.omega_m if omega_m is None else omega_m
+    if compute is None:
+        compute = _device_statistics(model, samples, prior, params, z_edges, log_nhi_edges, dla_log_nhi_min, omega_m)
+    return _statistics_sharded(spectra, z_edges, log_nhi_edges, select, batch_quasars, hubble_h, compute, device)
+
+
+def multi_dla_statistics_sharded(model: Dict, samples: Dict, spectra: Dict, prior: Dict, z_edges, log_nhi_edges,
+                                 select=None, params=None, max_dlas: int = 4, batch_quasars: int = 4096,
+                                 dla_log_nhi_min: float = None, omega_m: float = None, hubble_h: float = None,
+                                 compute: Callable[[Dict, np.ndarray, np.ndarray], np.ndarray] = None,
+                                 device=None) -> Dict:
+    """``dla_statistics_sharded`` for the multi-DLA model: rank r runs its block through ``process_multi_device`` (up
+    to ``max_dlas`` DLAs, sub-DLA model, mean flux; ``samples`` holds the sub-DLA samples) in batches and accumulates
+    ``multi_statistics_device`` sums on its GPU; one ``all_gather``, added in rank order.  ``compute`` as there."""
+    from . import params as P
+    dla_log_nhi_min = P.dla_log_nhi_min if dla_log_nhi_min is None else dla_log_nhi_min
+    omega_m = P.omega_m if omega_m is None else omega_m
+    if compute is None:
+        compute = _device_statistics(model, samples, prior, params, z_edges, log_nhi_edges, dla_log_nhi_min, omega_m,
+                                     max_dlas=max_dlas)
+    return _statistics_sharded(spectra, z_edges, log_nhi_edges, select, batch_quasars, hubble_h, compute, device)
+
+
+def _statistics_sharded(spectra, z_edges, log_nhi_edges, select, batch_quasars, hubble_h, compute, device) -> Dict:
+    """The cost-balanced block of this rank in batches through ``compute``, one gather of the sums, the finish."""
     import torch.distributed as dist
     from . import params as P
     from .api import dla_statistics_width, finish_dla_statistics
-    dla_log_nhi_min = P.dla_log_nhi_min if dla_log_nhi_min is None else dla_log_nhi_min
-    omega_m = P.omega_m if omega_m is None else omega_m
     hubble_h = P.hubble_h if hubble_h is None else hubble_h
     rank, world = dist.get_rank(), dist.get_world_size()
     blocks = partition_by_cost(quasar_costs(spectra), world)
     s, e = blocks[rank]
     Q = len(spectra["z_qsos"])
     sel = np.ones(Q, dtype=bool) if select is None else np.asarray(select, dtype=bool).ravel()
-    width = dla_statistics_width(len(z_edges) - 1, len(log_nhi_edges) - 1)
-    if compute is None:
-        compute = _device_statistics(model, samples, prior, params, z_edges, log_nhi_edges, dla_log_nhi_min, omega_m)
-    local = np.zeros(width)
+    local = np.zeros(dla_statistics_width(len(z_edges) - 1, len(log_nhi_edges) - 1))
     for b0 in range(s, e, max(int(batch_quasars), 1)):
         b1 = min(e, b0 + max(int(batch_quasars), 1))
         local = compute(slice_spectra(spectra, b0, b1), sel[b0:b1], local)
@@ -171,8 +193,9 @@ def dla_statistics_sharded(model: Dict, samples: Dict, spectra: Dict, prior: Dic
     return out
 
 
-def _device_statistics(model, samples, prior, params, z_edges, log_nhi_edges, dla_log_nhi_min, omega_m):
-    """The CUDA path of one rank: spectra -> process_device -> statistics_device into one device sums tensor."""
+def _device_statistics(model, samples, prior, params, z_edges, log_nhi_edges, dla_log_nhi_min, omega_m, max_dlas=0):
+    """The CUDA path of one rank: spectra -> process_device -> statistics_device (``max_dlas`` 0), or
+    process_multi_device -> multi_statistics_device, into one device sums tensor."""
     import os
     import torch
     from .api import DLAProcessor, pad_spectra
@@ -187,11 +210,16 @@ def _device_statistics(model, samples, prior, params, z_edges, log_nhi_edges, dl
         up = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dtype=dt)).to(d)
         if "sums" not in state:
             state["sums"] = up(sums, np.float64)
-        out = proc.process_device(up(pad["wavelengths"], np.float64), up(pad["flux"], np.float64),
-                                  up(pad["noise_variance"], np.float64), up(pad["pixel_mask"], np.uint8),
-                                  up(pad["lengths"], np.int32), up(pad["z_qsos"], np.float64),
-                                  return_sample_log_likelihoods=True)
-        proc.statistics_device(out, z_edges, log_nhi_edges, select=up(sel, np.uint8), sums=state["sums"],
-                               dla_log_nhi_min=dla_log_nhi_min, omega_m=omega_m)
+        planes = (up(pad["wavelengths"], np.float64), up(pad["flux"], np.float64),
+                  up(pad["noise_variance"], np.float64), up(pad["pixel_mask"], np.uint8),
+                  up(pad["lengths"], np.int32), up(pad["z_qsos"], np.float64))
+        if max_dlas:
+            out = proc.process_multi_device(*planes, max_dlas=max_dlas, return_samples=True)
+            proc.multi_statistics_device(out, z_edges, log_nhi_edges, select=up(sel, np.uint8), sums=state["sums"],
+                                         dla_log_nhi_min=dla_log_nhi_min, omega_m=omega_m)
+        else:
+            out = proc.process_device(*planes, return_sample_log_likelihoods=True)
+            proc.statistics_device(out, z_edges, log_nhi_edges, select=up(sel, np.uint8), sums=state["sums"],
+                                   dla_log_nhi_min=dla_log_nhi_min, omega_m=omega_m)
         return state["sums"]
     return compute

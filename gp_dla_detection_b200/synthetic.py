@@ -116,17 +116,25 @@ def forest_suppression(lam: np.ndarray, z_qso: float, tau_0: float, beta: float)
 
 def make_spectra(model: dict, num_quasars: int, seed: int = SPECTRA_SEED, shard: int = 0,
                  fixed_shape: bool = False, dla_fraction: float = 0.1, meanflux: bool = False,
-                 max_injected: int = 1) -> dict:
+                 max_injected: int = 1, second_dla_fraction: float = 0.0) -> dict:
     """BOSS-grid spectra shaped like preload_qsos.m:56-67 output (ragged lists).
 
     ``fixed_shape`` gives the 1217-pixel micro-benchmark variant of BASELINE.json: exactly
-    n = n_u = 1217 consecutive unmasked pixels inside the modelled window."""
+    n = n_u = 1217 consecutive unmasked pixels inside the modelled window.
+    ``second_dla_fraction``: the fraction of spectra with an injected DLA that get a second one, at least
+    kms_to_z(3000) from the first in z (the multi-DLA model's separation); its truth is in ``truth_z_dla2`` /
+    ``truth_log_nhi2`` (NaN where there is none), keys present only when the fraction is positive.  At 0 the
+    generator draws exactly the random numbers it draws without the option."""
     rng = np.random.default_rng(seed + shard)
     lam_rest, mu, M, log_omega = model["rest_wavelengths"], model["mu"], model["M"], model["log_omega"]
     c_0, tau_0, beta = math.exp(model["log_c_0"]), math.exp(model["log_tau_0"]), math.exp(model["log_beta"])
     k = M.shape[1]
     out = dict(all_wavelengths=[], all_flux=[], all_noise_variance=[], all_pixel_mask=[], z_qsos=[],
                truth_z_dla=[], truth_log_nhi=[])
+    truth2 = ("truth_z_dla2", "truth_log_nhi2") if second_dla_fraction > 0 else ()
+    for nm in truth2:
+        out[nm] = []
+    sep = P.kms_to_z(3000.0)
     while len(out["z_qsos"]) < num_quasars:
         z_qso = min(2.15 + rng.gamma(2.0, 0.3), 5.5)
         j0 = math.ceil((math.log10(P.DEFAULT.loading_min_lambda * (1 + z_qso)) - 3.5563) / 1e-4) - 1
@@ -158,6 +166,16 @@ def make_spectra(model: dict, num_quasars: int, seed: int = SPECTRA_SEED, shard:
             for _ in range(int(rng.integers(1, max_injected + 1))):   # truth_* keep the last injected system
                 tz, tn = rng.uniform(zmin, zmax), rng.uniform(20.0, 22.0)
                 flux = flux * _voigt_raw(lam, tz, 10.0 ** tn)
+        tz2, tn2 = np.nan, np.nan
+        if truth2 and np.isfinite(tz) and rng.random() < second_dla_fraction:
+            below, above = max(tz - sep - zmin, 0.0), max(zmax - tz - sep, 0.0)   # [zmin, tz - sep] + [tz + sep, zmax]
+            x = rng.uniform(0.0, below + above)
+            tz2 = zmin + x if x < below else tz + sep + (x - below)
+            tn2 = rng.uniform(20.0, 22.0)
+            if below + above > 0:
+                flux = flux * _voigt_raw(lam, tz2, 10.0 ** tn2)
+            else:
+                tz2, tn2 = np.nan, np.nan
         flux = flux + np.sqrt(noise_variance) * rng.standard_normal(L)
         mask = np.zeros(L, dtype=bool) if fixed_shape else (rng.random(L) < 0.02)
         inside = (rest >= P.DEFAULT.min_lambda) & (rest <= P.DEFAULT.max_lambda)
@@ -166,6 +184,8 @@ def make_spectra(model: dict, num_quasars: int, seed: int = SPECTRA_SEED, shard:
         out["all_wavelengths"].append(lam); out["all_flux"].append(flux)
         out["all_noise_variance"].append(noise_variance); out["all_pixel_mask"].append(mask)
         out["z_qsos"].append(z_qso); out["truth_z_dla"].append(tz); out["truth_log_nhi"].append(tn)
-    for nm in ("z_qsos", "truth_z_dla", "truth_log_nhi"):
+        if truth2:
+            out["truth_z_dla2"].append(tz2); out["truth_log_nhi2"].append(tn2)
+    for nm in ("z_qsos", "truth_z_dla", "truth_log_nhi") + truth2:
         out[nm] = np.asarray(out[nm])
     return out

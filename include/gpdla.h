@@ -319,6 +319,39 @@ int gpdla_dla_statistics_device(int64_t Q, int64_t S, const double* sample_log_l
                                 int32_t n_z, const double* z_edges, int32_t n_nhi, const double* log_nhi_edges,
                                 double dla_log_nhi_min, double omega_m, double* sums, void* stream);
 
+/* Population statistics of the multi-DLA catalogue (Ho et al. 2021) from one gpdla_process_qsos_multi(_device) call's
+ * outputs with the same samples: sample_log_likelihoods_dla [Q x max_dlas x S], base_sample_inds
+ * [Q x (max_dlas-1) x S] (0-based; NULL only when max_dlas == 1), model_posteriors [Q x (2 + max_dlas)] (no DLA,
+ * sub-DLA, 1..max_dlas DLAs), min_z_dlas, max_z_dlas [Q], the nullable uint8 mask `select` [Q], and offset_samples,
+ * log_nhi_samples, nhi_samples [S].  Per quasar the model is a mixture: model M with probability p_M; under j DLAs,
+ * sample i with its normalised weight w_ji (NaN entries, the z-separation filter's, weigh 0), which places j absorbers
+ * at samples i, base_sample_inds[0][i], ..., base_sample_inds[j-2][i].  The no-DLA and sub-DLA models place none.
+ * Quasar q contributes iff select[q] (default 1), every entry of its model_posteriors row is finite, max_z > min_z,
+ * and every level with p_j > 0 has a finite maximum log-likelihood and partner indices in [0, S); levels with p_j == 0
+ * are skipped.  `sums` (in/out, float64, the layout of gpdla_dla_statistics) is ADDED to, with the exact mixture mean
+ * and variance of each per-quasar count:
+ *   counts / counts_var[n_z][n_nhi]   E[X], E[X^2] - E[X]^2 of X = the number of absorbers in the (z, log N) cell
+ *   dla / dla_var[n_z]                the same of D = the number of absorbers in the z bin with log N >= dla_log_nhi_min
+ *   nhi / nhi_var[n_z]                the same of E = the sum of N_HI over those absorbers
+ *   path[n_z], num_quasars            as gpdla_dla_statistics.
+ * With max_dlas == 1 this is the single-DLA statistic.  Every argument check of gpdla_dla_statistics applies, and
+ * 1 <= max_dlas <= 4; else GPDLA_ERR_INVALID before any CUDA call.  The host entry also rejects a base_sample_inds
+ * entry outside [0, S).  No atomics: repeated calls give the same bits, and the host entry those of the _device entry.
+ * Context-free, on the current device; the _device entry takes device arrays and is asynchronous on `stream`. */
+int gpdla_multi_dla_statistics(int64_t Q, int64_t S, int32_t max_dlas, const double* sample_log_likelihoods_dla,
+                               const int32_t* base_sample_inds, const double* model_posteriors,
+                               const double* min_z_dlas, const double* max_z_dlas, const uint8_t* select,
+                               const double* offset_samples, const double* log_nhi_samples, const double* nhi_samples,
+                               int32_t n_z, const double* z_edges, int32_t n_nhi, const double* log_nhi_edges,
+                               double dla_log_nhi_min, double omega_m, double* sums);
+int gpdla_multi_dla_statistics_device(int64_t Q, int64_t S, int32_t max_dlas, const double* sample_log_likelihoods_dla,
+                                      const int32_t* base_sample_inds, const double* model_posteriors,
+                                      const double* min_z_dlas, const double* max_z_dlas, const uint8_t* select,
+                                      const double* offset_samples, const double* log_nhi_samples,
+                                      const double* nhi_samples, int32_t n_z, const double* z_edges, int32_t n_nhi,
+                                      const double* log_nhi_edges, double dla_log_nhi_min, double omega_m,
+                                      double* sums, void* stream);
+
 /* voigt.c:253-304: profile has num_points - 6 entries.  Host buffers; runs on the current device. */
 int gpdla_voigt(const double* lambdas, int64_t num_points, double z, double N, int32_t num_lines, double* profile);
 /* Batched, device buffers: profile[s, :] = voigt(lambdas, z[s], N[s], num_lines), [S x (num_points-6)] */
