@@ -53,6 +53,14 @@ class GpdlaMultiResults(ctypes.Structure):
     _fields_ = [(n, ctypes.c_void_p) for n in MULTI_RESULT_FIELDS]
 
 
+RECONSTRUCTION_FIELDS = ["absorption", "prior_mean", "prior_sd", "fit_mean", "continuum", "continuum_sd", "latent", "chi2",
+                         "log_likelihood", "num_pixels"]
+
+
+class GpdlaReconstruction(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_void_p) for n in RECONSTRUCTION_FIELDS]
+
+
 # every symbol include/gpdla.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "gpdla_default_parameters": (None, [ctypes.POINTER(GpdlaParams)]),
@@ -130,6 +138,12 @@ SYMBOLS = {
                                           + [ctypes.c_void_p] * 9
                                           + [ctypes.c_int32, c_double_p, ctypes.c_int32, c_double_p, ctypes.c_double,
                                              ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]),
+    "gpdla_reconstruct": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64] + [ctypes.c_void_p] * 6
+                          + [ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p,
+                             ctypes.POINTER(GpdlaReconstruction)]),
+    "gpdla_reconstruct_device": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64] + [ctypes.c_void_p] * 6
+                                 + [ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p,
+                                    ctypes.POINTER(GpdlaReconstruction), ctypes.c_void_p]),
 }
 
 _lib = None

@@ -382,6 +382,76 @@ class DLAProcessor:
                 float(omega_m), ptr(sums), stream))
         return sums
 
+    # ---------------------------------------------------------------- fitted model under chosen absorbers
+    def _recon_operands(self, Q: int, absorber_z, absorber_nhi, to):
+        """(num_absorbers, z, N) as [Q x num_absorbers] arrays made by ``to`` (NaN z = no absorber)."""
+        if (absorber_z is None) != (absorber_nhi is None):
+            raise ValueError("absorber_z and absorber_nhi go together")
+        if absorber_z is None:
+            return 0, None, None
+        z, n = to(absorber_z), to(absorber_nhi)
+        if z.ndim == 1:
+            z, n = z.reshape(-1, 1), n.reshape(-1, 1)
+        if tuple(z.shape) != tuple(n.shape) or z.ndim != 2 or z.shape[0] != Q or not 0 <= z.shape[1] <= 4:
+            raise ValueError("absorber_z and absorber_nhi must be [Q, num_absorbers] with 0 <= num_absorbers <= 4")
+        return int(z.shape[1]), z, n
+
+    def reconstruct(self, spectra: Dict, absorber_z=None, absorber_nhi=None, meanflux: bool = False) -> Dict[str, np.ndarray]:
+        """The model fitted to each spectrum under the given absorbers (``gpdla_reconstruct``; what
+        CDDF_analysis/qso_loader.py:1654-1774 draws).  ``spectra``: ragged or padded, as ``process`` takes them;
+        ``absorber_z`` / ``absorber_nhi``: [Q, num_absorbers] (0..4; N in cm^-2; NaN z = none) or None for the null
+        model; ``meanflux``: the multi-DLA path's null model.  Returns NumPy arrays: the planes ``absorption``,
+        ``prior_mean``, ``prior_sd``, ``fit_mean``, ``continuum``, ``continuum_sd`` [Q, L_max] on each quasar's own
+        pixels (``wavelengths[q, :lengths[q]]``; NaN outside the modelled window), ``latent`` [Q, k], ``chi2``,
+        ``log_likelihood`` and ``num_pixels`` [Q]."""
+        sp = pad_spectra(spectra)
+        W, F, V = _f64(sp["wavelengths"]), _f64(sp["flux"]), _f64(sp["noise_variance"])
+        Mk = np.ascontiguousarray(sp["pixel_mask"], dtype=np.uint8)
+        lengths = np.ascontiguousarray(sp["lengths"], dtype=np.int32).ravel()
+        z = _f64(sp["z_qsos"]).ravel()
+        _check_planes(W, F, V, Mk, lengths, z)
+        Q, L_max = W.shape
+        A, az, an = self._recon_operands(Q, absorber_z, absorber_nhi, _f64)
+        out = {n: np.empty((Q, L_max)) for n in _lib.RECONSTRUCTION_FIELDS[:6]}
+        out.update(latent=np.empty((Q, self.k)), chi2=np.empty(Q), log_likelihood=np.empty(Q),
+                   num_pixels=np.empty(Q, dtype=np.int32))
+        res = _lib.GpdlaReconstruction()
+        for n in _lib.RECONSTRUCTION_FIELDS:
+            setattr(res, n, out[n].ctypes.data if out[n].size else None)
+        vp = lambda a: None if a is None else ctypes.c_void_p(a.ctypes.data)
+        _lib.check(self._lib.gpdla_reconstruct(self._ctx, Q, L_max, vp(W), vp(F), vp(V), vp(Mk), vp(lengths), vp(z),
+                                               int(bool(meanflux)), A, vp(az), vp(an), ctypes.byref(res)), self._ctx)
+        return out
+
+    def reconstruct_device(self, wavelengths, flux, noise_variance, pixel_mask, lengths, z_qsos, absorber_z=None,
+                           absorber_nhi=None, meanflux: bool = False) -> Dict:
+        """Device-resident ``reconstruct``: the planes as ``process_device`` (and ``preload_qsos_device``) hold them,
+        absorbers as CUDA tensors or host arrays; returns CUDA tensors with the names of ``reconstruct``.  Asynchronous
+        on torch's current stream."""
+        import torch
+        Q, L_max = wavelengths.shape
+        dev = wavelengths.device
+        assert dev.type == "cuda" and dev.index == self.device
+        for t, dt in ((wavelengths, torch.float64), (flux, torch.float64), (noise_variance, torch.float64),
+                      (pixel_mask, torch.uint8), (lengths, torch.int32), (z_qsos, torch.float64)):
+            assert t.is_cuda and t.dtype == dt and t.is_contiguous()
+        to = lambda a: torch.as_tensor(a, dtype=torch.float64, device=dev).contiguous()
+        A, az, an = self._recon_operands(Q, absorber_z, absorber_nhi, to)
+        f64 = dict(dtype=torch.float64, device=dev)
+        out = {n: torch.empty((Q, L_max), **f64) for n in _lib.RECONSTRUCTION_FIELDS[:6]}
+        out.update(latent=torch.empty((Q, self.k), **f64), chi2=torch.empty(Q, **f64),
+                   log_likelihood=torch.empty(Q, **f64), num_pixels=torch.empty(Q, dtype=torch.int32, device=dev))
+        res = _lib.GpdlaReconstruction()
+        for n in _lib.RECONSTRUCTION_FIELDS:
+            setattr(res, n, out[n].data_ptr() if out[n].numel() else None)
+        ptr = lambda t: None if t is None else ctypes.c_void_p(t.data_ptr())
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(self._lib.gpdla_reconstruct_device(
+            self._ctx, Q, L_max, ptr(wavelengths), ptr(flux), ptr(noise_variance), ptr(pixel_mask), ptr(lengths),
+            ptr(z_qsos), int(bool(meanflux)), A, ptr(az if A else None), ptr(an if A else None), ctypes.byref(res),
+            ctypes.c_void_p(stream)), self._ctx)
+        return out
+
 
 def process_qsos(model: Dict, samples: Dict, spectra: Dict, prior: Dict, params: Parameters = DEFAULT,
                  device: int = 0, return_sample_log_likelihoods: bool = True, gram_digits: int = 0,
@@ -407,6 +477,94 @@ def process_qsos_multiple_dlas_meanflux(model: Dict, samples: Dict, spectra: Dic
         return proc.process_multi(spectra, max_dlas, base_sample_inds, return_samples)
     finally:
         proc.close()
+
+
+def _host(a) -> np.ndarray:
+    """A result array on the host (NumPy as it is; CUDA tensors copied)."""
+    if hasattr(a, "detach"):
+        a = a.detach().cpu().numpy()
+    return np.asarray(a)
+
+
+def map_absorbers(results: Dict, samples: Dict, model="map"):
+    """The absorbers of one model of a processed batch, as ``DLAProcessor.reconstruct`` takes them:
+    ``(absorber_z, absorber_nhi)``, [Q, num_absorbers] NumPy arrays (NaN z = none).  ``results``: what ``process``,
+    ``process_device``, ``process_multi(_device)`` or ``process_qsos_multiple_dlas_meanflux`` returned; ``samples``:
+    the samples they ran with.  ``model``:
+
+    * ``"map"``: each quasar's most probable model by ``model_posteriors`` (single-DLA: ``p_dlas > p_no_dlas``);
+    * ``"null"``: no absorbers;
+    * an integer j: level j's MAP absorbers, z from ``MAP_z_dlas`` (``map_z_dlas``) and N = ``nhi_samples[MAP_inds]``
+      (the sample's own N, not ``10**MAP_log_nhis``), so the reconstruction's log-likelihood is the stored sample's;
+    * ``"sub_dla"``: the arg-max of ``sample_log_likelihoods_lls`` at its (z_i, ``lls_nhi_samples[i]``)."""
+    nhi = _f64(samples["nhi_samples"]).ravel()
+    multi = "MAP_z_dlas" in results
+    Q = _host(results["min_z_dlas"]).shape[0]
+    none = lambda A: (np.full((Q, A), np.nan), np.full((Q, A), np.nan))
+
+    def level(j):
+        if multi:
+            MD = _host(results["MAP_z_dlas"]).shape[1]
+            if not 1 <= j <= MD:
+                raise ValueError("level must lie in [1, %d]" % MD)
+            zz = _host(results["MAP_z_dlas"])[:, j - 1, :j].astype(np.float64)
+            ind = _host(results["MAP_inds"])[:, j - 1, :j].astype(np.int64)
+        else:
+            if j != 1:
+                raise ValueError("single-DLA results hold level 1 only")
+            zz = _host(results["map_z_dlas"]).astype(np.float64).reshape(Q, 1)
+            ind = _host(results["map_inds"]).astype(np.int64).reshape(Q, 1)
+        ok = ind >= 0
+        n = np.where(ok, nhi[np.where(ok, ind, 0)], np.nan)
+        return np.where(ok, zz, np.nan), n
+
+    def sub_dla():
+        if "sample_log_likelihoods_lls" not in results or "lls_nhi_samples" not in samples:
+            raise ValueError('model="sub_dla" needs results["sample_log_likelihoods_lls"] (process_multi with '
+                             'return_samples) and samples["lls_nhi_samples"]')
+        ll = _host(results["sample_log_likelihoods_lls"])
+        lls = _f64(samples["lls_nhi_samples"]).ravel()
+        off = _f64(samples["offset_samples"]).ravel()
+        zlo, zhi = _host(results["min_z_dlas"]), _host(results["max_z_dlas"])
+        zz, n = none(1)
+        for q in range(Q):
+            if np.all(np.isnan(ll[q])):
+                continue
+            i = int(np.nanargmax(ll[q]))
+            zz[q, 0] = zlo[q] + (zhi[q] - zlo[q]) * off[i]
+            n[q, 0] = lls[i]
+        return zz, n
+
+    if isinstance(model, str) and model == "null":
+        return none(0)
+    if isinstance(model, str) and model == "sub_dla":
+        if not multi:
+            raise ValueError('model="sub_dla" needs multi-DLA results')
+        return sub_dla()
+    if isinstance(model, (int, np.integer)) and not isinstance(model, bool):
+        return level(int(model))
+    if not (isinstance(model, str) and model == "map"):
+        raise ValueError('model must be "map", "null", "sub_dla" or a level number')
+    if not multi:
+        p_dla, p_no = _host(results["p_dlas"]), _host(results["p_no_dlas"])
+        zz, n = level(1)
+        dla = p_dla > p_no
+        return np.where(dla[:, None], zz, np.nan), np.where(dla[:, None], n, np.nan)
+    mp = _host(results["model_posteriors"])
+    MD = mp.shape[1] - 2
+    zz, n = none(MD)
+    # NaN-ignoring arg-max (levels past an early exit are NaN); a row without a finite entry gets no absorber
+    finite = np.any(np.isfinite(mp), axis=1)
+    best = np.where(finite, np.argmax(np.where(np.isfinite(mp), mp, -np.inf), axis=1), 0)
+    if np.any(best == 1):
+        zs, ns = sub_dla()
+        zz[best == 1, :1], n[best == 1, :1] = zs[best == 1], ns[best == 1]
+    for j in range(1, MD + 1):
+        sel = best == j + 1
+        if np.any(sel):
+            zj, nj = level(j)
+            zz[sel, :j], n[sel, :j] = zj[sel], nj[sel]
+    return zz, n
 
 
 def _pad_raw(raw: Dict) -> Dict[str, np.ndarray]:

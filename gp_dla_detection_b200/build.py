@@ -8,7 +8,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libgpdla.so")
 SOURCES = ["gpdla_capi.cu"]
-HEADERS = ["gpdla_kernels.cuh", "gpdla_i8_kernels.cuh", "gpdla_preload.cuh", "gpdla_objective.cuh", "gpdla_training.cuh", "gpdla_statistics.cuh", "gpdla_math.cuh", "voigt_tables.h", "gpdla_rest_table.h", os.path.join("..", "..", "include", "gpdla.h")]
+HEADERS = ["gpdla_kernels.cuh", "gpdla_i8_kernels.cuh", "gpdla_preload.cuh", "gpdla_objective.cuh", "gpdla_training.cuh", "gpdla_statistics.cuh", "gpdla_reconstruct.cuh", "gpdla_math.cuh", "voigt_tables.h", "gpdla_rest_table.h", os.path.join("..", "..", "include", "gpdla.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC"]
 

@@ -22,6 +22,7 @@
 #include "gpdla_objective.cuh"
 #include "gpdla_training.cuh"
 #include "gpdla_statistics.cuh"
+#include "gpdla_reconstruct.cuh"
 #include "gpdla_rest_table.h"
 
 using namespace gpdla;
@@ -2178,6 +2179,150 @@ int gpdla_multi_dla_statistics(int64_t Q, int64_t S, int32_t max_dlas, const dou
   if (e != cudaSuccess) { g_err = std::string(fn) + ": " + cudaGetErrorString(e); rc = GPDLA_ERR_CUDA; }
   cudaFree(base);
   return rc;
+}
+
+// ---- the fitted model of each quasar under chosen absorbers (CDDF_analysis/qso_loader.py:1654-1774) ----
+
+// the checks both reconstruction entries make before any CUDA call
+static int recon_check(gpdla_ctx* c, const char* fn, int64_t Q, int64_t L_max, const double* wavelengths,
+                       const double* flux, const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                       const double* z_qsos, int32_t meanflux, int32_t num_absorbers, const double* absorber_z,
+                       const double* absorber_nhi, const gpdla_reconstruction* out) {
+  if (Q < 0 || Q > 2147483647LL || L_max < 1 || !out || num_absorbers < 0 || num_absorbers > RC_MAX_ABSORBERS ||
+      !(meanflux == 0 || meanflux == 1) ||
+      (Q > 0 && (!wavelengths || !flux || !noise_variance || !pixel_mask || !lengths || !z_qsos)) ||
+      (Q > 0 && num_absorbers > 0 && (!absorber_z || !absorber_nhi))) {
+    c->err = std::string(fn) + ": invalid arguments (0 <= num_absorbers <= 4, meanflux 0 or 1, non-NULL inputs)";
+    return GPDLA_ERR_INVALID;
+  }
+  if (!c->d_M) {
+    c->err = std::string(fn) + ": set_model must be called first";
+    return GPDLA_ERR_STATE;
+  }
+  if (!rank_supported(c->k)) {
+    c->err = std::string(fn) + ": rank k=" + std::to_string(c->k) + " not compiled in (available: 10, 20, 40)";
+    return GPDLA_ERR_UNSUPPORTED;
+  }
+  return GPDLA_OK;
+}
+
+// one CTA per quasar; the row of L_max pixels' absorption is staged in shared memory, which bounds L_max
+extern "C++" {
+template <int K>
+static int launch_reconstruct(gpdla_ctx* c, const ReconArgs& ra, int64_t Q, cudaStream_t st) {
+  const size_t smem = reconstruct_smem_doubles<K>(ra.L_max) * sizeof(double);
+  int optin = 0;
+  cudaFuncAttributes fa;
+  CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device), c->err);
+  CUDA_TRY(cudaFuncGetAttributes(&fa, reconstruct_kernel<K>), c->err);
+  if (smem + fa.sharedSizeBytes > (size_t)optin) {
+    c->err = "gpdla_reconstruct: L_max=" + std::to_string(ra.L_max) + " does not fit one CTA's shared memory";
+    return GPDLA_ERR_UNSUPPORTED;
+  }
+  int rc = configure_smem(c->device, reconstruct_kernel<K>, smem, c->err);
+  if (rc) return rc;
+  reconstruct_kernel<K><<<(unsigned)Q, NTHREADS, smem, st>>>(ra);
+  return GPDLA_OK;
+}
+}  // extern "C++"
+
+int gpdla_reconstruct_device(gpdla_ctx* c, int64_t Q, int64_t L_max, const double* wavelengths, const double* flux,
+                             const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                             const double* z_qsos, int32_t meanflux, int32_t num_absorbers, const double* absorber_z,
+                             const double* absorber_nhi, const gpdla_reconstruction* out, void* stream) {
+  if (!c) return GPDLA_ERR_INVALID;
+  int rc = recon_check(c, "gpdla_reconstruct_device", Q, L_max, wavelengths, flux, noise_variance, pixel_mask, lengths,
+                       z_qsos, meanflux, num_absorbers, absorber_z, absorber_nhi, out);
+  if (rc || Q == 0) return rc;
+  DeviceGuard guard(c->device);
+  ReconArgs ra;
+  memset(&ra, 0, sizeof ra);
+  ra.wavelengths = wavelengths; ra.flux = flux; ra.noise_variance = noise_variance; ra.pixel_mask = pixel_mask;
+  ra.lengths = lengths; ra.z_qsos = z_qsos; ra.L_max = L_max;
+  ra.rest_wavelengths = c->d_rest; ra.mu = c->d_mu; ra.M = c->d_M; ra.log_omega = c->d_log_omega; ra.n_rest = c->n_rest;
+  ra.c_0 = c->c_0; ra.tau_0 = c->tau_0; ra.beta = c->beta;
+  ra.min_lambda = c->params.min_lambda; ra.max_lambda = c->params.max_lambda;
+  ra.lya_wavelength = c->params.lya_wavelength; ra.pixel_spacing = c->params.pixel_spacing;
+  ra.num_lines = c->params.num_lines; ra.meanflux = meanflux;
+  ra.num_absorbers = num_absorbers; ra.absorber_z = absorber_z; ra.absorber_nhi = absorber_nhi;
+  ra.absorption = out->absorption; ra.prior_mean = out->prior_mean; ra.prior_sd = out->prior_sd;
+  ra.fit_mean = out->fit_mean; ra.continuum = out->continuum; ra.continuum_sd = out->continuum_sd;
+  ra.latent = out->latent; ra.chi2 = out->chi2; ra.log_likelihood = out->log_likelihood; ra.num_pixels = out->num_pixels;
+  switch (c->k) {
+    case 10: rc = launch_reconstruct<10>(c, ra, Q, (cudaStream_t)stream); break;
+    case 20: rc = launch_reconstruct<20>(c, ra, Q, (cudaStream_t)stream); break;
+    case 40: rc = launch_reconstruct<40>(c, ra, Q, (cudaStream_t)stream); break;
+    default: c->err = "gpdla_reconstruct: rank not compiled in"; rc = GPDLA_ERR_UNSUPPORTED;
+  }
+  if (rc) return rc;
+  c->launches++;
+  CUDA_TRY(cudaGetLastError(), c->err);
+  return GPDLA_OK;
+}
+
+int gpdla_reconstruct(gpdla_ctx* c, int64_t Q, int64_t L_max, const double* wavelengths, const double* flux,
+                      const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                      const double* z_qsos, int32_t meanflux, int32_t num_absorbers, const double* absorber_z,
+                      const double* absorber_nhi, const gpdla_reconstruction* out) {
+  if (!c) return GPDLA_ERR_INVALID;
+  int rc = recon_check(c, "gpdla_reconstruct", Q, L_max, wavelengths, flux, noise_variance, pixel_mask, lengths, z_qsos,
+                       meanflux, num_absorbers, absorber_z, absorber_nhi, out);
+  if (rc || Q == 0) return rc;
+  const size_t QA = (size_t)Q * num_absorbers;
+  for (size_t i = 0; i < QA; ++i) {
+    const double z = absorber_z[i], N = absorber_nhi[i];
+    if (std::isnan(z)) continue;
+    if (!(std::isfinite(z) && z > -1.0 && std::isfinite(N) && N >= 0.0)) {
+      c->err = "gpdla_reconstruct: absorber " + std::to_string(i) + " needs z > -1 and a finite N >= 0 (NaN z = none)";
+      return GPDLA_ERR_INVALID;
+    }
+  }
+  DeviceGuard guard(c->device);
+  const size_t QL = (size_t)Q * L_max;
+  struct Item { void** dev; const void* host_in; void* host_out; size_t bytes; };
+  double *d_w, *d_f, *d_v, *d_z, *d_az = nullptr, *d_an = nullptr;
+  uint8_t* d_m;
+  int32_t* d_len;
+  gpdla_reconstruction dr;
+  memset(&dr, 0, sizeof dr);
+  std::vector<Item> items = {
+      {(void**)&d_w, wavelengths, nullptr, QL * 8}, {(void**)&d_f, flux, nullptr, QL * 8},
+      {(void**)&d_v, noise_variance, nullptr, QL * 8}, {(void**)&d_z, z_qsos, nullptr, (size_t)Q * 8},
+      {(void**)&d_len, lengths, nullptr, (size_t)Q * 4}, {(void**)&d_m, pixel_mask, nullptr, QL}};
+  if (QA) {
+    items.push_back({(void**)&d_az, absorber_z, nullptr, QA * 8});
+    items.push_back({(void**)&d_an, absorber_nhi, nullptr, QA * 8});
+  }
+  auto want = [&](void** dev, void* host, size_t bytes) { if (host) items.push_back({dev, nullptr, host, bytes}); };
+  want((void**)&dr.absorption, out->absorption, QL * 8);
+  want((void**)&dr.prior_mean, out->prior_mean, QL * 8);
+  want((void**)&dr.prior_sd, out->prior_sd, QL * 8);
+  want((void**)&dr.fit_mean, out->fit_mean, QL * 8);
+  want((void**)&dr.continuum, out->continuum, QL * 8);
+  want((void**)&dr.continuum_sd, out->continuum_sd, QL * 8);
+  want((void**)&dr.latent, out->latent, (size_t)Q * c->k * 8);
+  want((void**)&dr.chi2, out->chi2, (size_t)Q * 8);
+  want((void**)&dr.log_likelihood, out->log_likelihood, (size_t)Q * 8);
+  want((void**)&dr.num_pixels, out->num_pixels, (size_t)Q * 4);
+  size_t bytes = 256;
+  for (auto& it : items) bytes += (it.bytes + 255) / 256 * 256;
+  if (c->st_bytes < bytes) {
+    cudaFree(c->d_stage); c->d_stage = nullptr; c->st_bytes = 0;
+    CUDA_TRY(cudaMalloc(&c->d_stage, bytes), c->err);
+    c->st_bytes = bytes;
+  }
+  char* p = (char*)c->d_stage;
+  cudaStream_t st = c->stream;
+  for (auto& it : items) {
+    *it.dev = p; p += (it.bytes + 255) / 256 * 256;
+    if (it.host_in) CUDA_TRY(cudaMemcpyAsync(*it.dev, it.host_in, it.bytes, cudaMemcpyHostToDevice, st), c->err);
+  }
+  rc = gpdla_reconstruct_device(c, Q, L_max, d_w, d_f, d_v, d_m, d_len, d_z, meanflux, num_absorbers, d_az, d_an, &dr, st);
+  if (rc) return rc;
+  for (auto& it : items)
+    if (it.host_out) CUDA_TRY(cudaMemcpyAsync(it.host_out, *it.dev, it.bytes, cudaMemcpyDeviceToHost, st), c->err);
+  CUDA_TRY(cudaStreamSynchronize(st), c->err);
+  return GPDLA_OK;
 }
 
 }  // extern "C"

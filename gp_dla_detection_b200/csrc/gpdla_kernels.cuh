@@ -168,6 +168,75 @@ __device__ __forceinline__ double interp_linear(const double* xp, const double* 
   return slope * (x - xp[j]) + fp[j * stride];
 }
 
+// The null model at one window pixel (observed wavelength w, emitted wavelength rest): process_qsos.m:138-146, and in
+// mean-flux mode ...meanflux.m:245-293.  Returns the bracketing rest interval j and
+//   mu     interpolated mu, NOT suppressed (mu~ = mu * absorb)
+//   om2    omega~^2: interpolated omega^2 times the forest noise scaling and, in mean-flux mode, absorb^2
+//   absorb the mean-flux suppression factor s (1 outside mean-flux mode); row c of M~ is interp(M_c) * absorb
+// prepare_quasars_kernel and reconstruct_kernel both evaluate the model through this function.
+struct PixelModel {
+  int j;
+  double mu, om2, absorb;
+};
+__device__ __forceinline__ PixelModel null_model_pixel(const double* __restrict__ rest_wavelengths,
+                                                       const double* __restrict__ mu, const double* __restrict__ log_omega,
+                                                       int n_rest, double c_0, double tau_0, double beta,
+                                                       double lya_wavelength, int meanflux, double w, double rest,
+                                                       double z_qso) {
+  PixelModel pm;
+  const double x0 = rest_wavelengths[0];
+  const double inv_dx = (n_rest - 1) / (rest_wavelengths[n_rest - 1] - x0);
+  int j = (int)((rest - x0) * inv_dx);
+  j = max(0, min(j, n_rest - 2));
+  while (j > 0 && rest_wavelengths[j] > rest) --j;
+  while (j < n_rest - 2 && rest_wavelengths[j + 1] <= rest) ++j;
+  pm.j = j;
+  pm.mu = interp_linear(rest_wavelengths, mu, 1, j, rest);
+  pm.absorb = 1.0;
+  double lw = interp_linear(rest_wavelengths, log_omega, 1, j, rest);
+  double lya_z = (w - lya_wavelength) / lya_wavelength;                           // :117-119
+  if (!meanflux) {
+    double scaling = 1.0 - exp(-tau_0 * pow(1.0 + lya_z, beta)) + c_0;           // :144
+    pm.om2 = exp(2.0 * lw) * (scaling * scaling);                                 // :142,146
+  } else {
+    // multi_dlas/process_qsos_multiple_dlas_meanflux.m:245-293
+    double depth = tau_0 * pow(1.0 + lya_z, beta);                                // :245
+    for (int l = 1; l < c_forest.num_forest_lines; ++l) {                         // :247-259
+      double lyman_1pz = c_forest.wavelength[0] * (1.0 + lya_z) / c_forest.wavelength[l];
+      if (lyman_1pz <= 1.0 + z_qso) depth = depth + (tau_0 * c_forest.tau_ratio[l]) * pow(lyman_1pz, beta);
+    }
+    double scaling = 1.0 - exp(-depth) + c_0;                                     // :261
+    double om2 = exp(2.0 * lw) * (scaling * scaling);                             // :263
+    double total = 0.0;
+    for (int l = 0; l < c_forest.num_forest_lines; ++l) {                         // :269-283
+      double zl = (w - c_forest.wavelength[l]) / c_forest.wavelength[l];          // :183-187
+      if (l == 0 || !(zl > z_qso)) total = total + c_forest.kim_tau[l] * pow(1.0 + zl, c_forest.prev_beta);
+    }
+    pm.absorb = exp(-total);                                                      // :285
+    pm.om2 = om2 * (pm.absorb * pm.absorb);                                       // :293
+  }
+  return pm;
+}
+
+// Entry p of the padded wavelength grid of process_qsos.m:168-176 for a window of n_u pixels starting at `wl_first`
+// whose smallest / largest wavelengths have log10 lo / hi; entries past the reference's trailing pad continue the log
+// grid.
+__device__ __forceinline__ double padded_wavelength(int p, int n_u, const double* wl_first, double lo, double hi,
+                                                    double pixel_spacing) {
+  const int W3 = 3;
+  if (p < W3) {
+    // logspace(lo - 3 ps, lo - ps, 3) = 10.^linspace(a, b, 3)
+    double a0 = lo - W3 * pixel_spacing, b0 = lo - pixel_spacing;
+    double ex = (p == W3 - 1) ? b0 : a0 + p * ((b0 - a0) / (W3 - 1));
+    return exp10(ex);
+  }
+  if (p < W3 + n_u) return wl_first[p - W3];
+  int t = p - (W3 + n_u);   // 0,1,2 are the reference's trailing pad; beyond that: filler
+  double a0 = hi + pixel_spacing, b0 = hi + W3 * pixel_spacing;
+  double ex = (t == W3 - 1) ? b0 : a0 + t * ((b0 - a0) / (W3 - 1));
+  return exp10(ex);
+}
+
 __global__ void __launch_bounds__(NTHREADS) prepare_quasars_kernel(PrepArgs a) {
   const int q = blockIdx.x, tid = threadIdx.x;
   const int64_t L = min(max((int64_t)a.lengths[q], (int64_t)0), a.L_max);   // a length beyond the padded row is clamped
@@ -252,29 +321,13 @@ __global__ void __launch_bounds__(NTHREADS) prepare_quasars_kernel(PrepArgs a) {
 
   // padded wavelength grid (process_qsos.m:168-176); pixels past the end continue the log grid
   const double lo = log10(s_minu), hi = log10(s_maxu);
-  const int W3 = 3;
   for (int p = tid; p < NPIX + 8; p += NTHREADS) {
-    double v;
-    if (p < W3) {
-      // logspace(lo - 3 ps, lo - ps, 3) = 10.^linspace(a, b, 3)
-      double a0 = lo - W3 * a.pixel_spacing, b0 = lo - a.pixel_spacing;
-      double ex = (p == W3 - 1) ? b0 : a0 + p * ((b0 - a0) / (W3 - 1));
-      v = exp10(ex);
-    } else if (p < W3 + n_u) {
-      v = wl[s_first + (p - W3)];
-    } else {
-      int t = p - (W3 + n_u);   // 0,1,2 are the reference's trailing pad; beyond that: filler
-      double a0 = hi + a.pixel_spacing, b0 = hi + W3 * a.pixel_spacing;
-      double ex = (t == W3 - 1) ? b0 : a0 + t * ((b0 - a0) / (W3 - 1));
-      v = exp10(ex);
-    }
+    const double v = padded_wavelength(p, n_u, wl + s_first, lo, hi, a.pixel_spacing);
     lam[p] = v;
     lamh[p] = log1p((v - lam_ref) / lam_ref) * a.inv_h;
   }
 
   // per-pixel model interpolation (process_qsos.m:138-146)
-  const double x0 = a.rest_wavelengths[0];
-  const double inv_dx = (a.n_rest - 1) / (a.rest_wavelengths[a.n_rest - 1] - x0);
   for (int i = tid; i < NPIX; i += NTHREADS) {
     double y = 0.0, v = 1.0, mu = 0.0, om2 = 0.0, absorb = 1.0;
     bool used = false;
@@ -286,35 +339,11 @@ __global__ void __launch_bounds__(NTHREADS) prepare_quasars_kernel(PrepArgs a) {
       rest = w / (1.0 + z_qso);
       used = !pm[src] && (rest >= a.min_lambda) && (rest <= a.max_lambda);
       if (used) {
-        j = (int)((rest - x0) * inv_dx);
-        j = max(0, min(j, a.n_rest - 2));
-        while (j > 0 && a.rest_wavelengths[j] > rest) --j;
-        while (j < a.n_rest - 2 && a.rest_wavelengths[j + 1] <= rest) ++j;
         y = fl[src]; v = nv[src];
-        mu = interp_linear(a.rest_wavelengths, a.mu, 1, j, rest);
-        double lw = interp_linear(a.rest_wavelengths, a.log_omega, 1, j, rest);
-        double lya_z = (w - a.lya_wavelength) / a.lya_wavelength;                 // :117-119
-        if (!a.meanflux) {
-          double scaling = 1.0 - exp(-a.tau_0 * pow(1.0 + lya_z, a.beta)) + a.c_0;   // :144
-          om2 = exp(2.0 * lw) * (scaling * scaling);                                 // :142,146
-        } else {
-          // multi_dlas/process_qsos_multiple_dlas_meanflux.m:245-293
-          double depth = a.tau_0 * pow(1.0 + lya_z, a.beta);                         // :245
-          for (int l = 1; l < c_forest.num_forest_lines; ++l) {                      // :247-259
-            double lyman_1pz = c_forest.wavelength[0] * (1.0 + lya_z) / c_forest.wavelength[l];
-            if (lyman_1pz <= 1.0 + z_qso) depth = depth + (a.tau_0 * c_forest.tau_ratio[l]) * pow(lyman_1pz, a.beta);
-          }
-          double scaling = 1.0 - exp(-depth) + a.c_0;                                // :261
-          om2 = exp(2.0 * lw) * (scaling * scaling);                                 // :263
-          double total = 0.0;
-          for (int l = 0; l < c_forest.num_forest_lines; ++l) {                      // :269-283
-            double zl = (w - c_forest.wavelength[l]) / c_forest.wavelength[l];       // :183-187
-            if (l == 0 || !(zl > z_qso)) total = total + c_forest.kim_tau[l] * pow(1.0 + zl, c_forest.prev_beta);
-          }
-          absorb = exp(-total);                                                      // :285
-          mu = mu * absorb;                                                          // :287
-          om2 = om2 * (absorb * absorb);                                             // :293
-        }
+        const PixelModel m = null_model_pixel(a.rest_wavelengths, a.mu, a.log_omega, a.n_rest, a.c_0, a.tau_0, a.beta,
+                                              a.lya_wavelength, a.meanflux, w, rest, z_qso);
+        j = m.j; om2 = m.om2; absorb = m.absorb;
+        mu = m.mu * absorb;                                                          // :287 (exact when absorb = 1)
       }
     }
     pix[i * 4 + 0] = y; pix[i * 4 + 1] = v; pix[i * 4 + 2] = mu; pix[i * 4 + 3] = om2;

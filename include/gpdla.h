@@ -352,6 +352,55 @@ int gpdla_multi_dla_statistics_device(int64_t Q, int64_t S, int32_t max_dlas, co
                                       const double* log_nhi_edges, double dla_log_nhi_min, double omega_m,
                                       double* sums, void* stream);
 
+/* ---- The fitted model of each quasar under chosen absorbers: what CDDF_analysis/qso_loader.py:1654-1774
+ * (plot_this_mu) draws, on the device, with the hot path's own model evaluation ----
+ * Spectra as gpdla_process_qsos takes them.  absorber_z, absorber_nhi: [Q x num_absorbers] (N in cm^-2, as voigt and
+ * nhi_samples take it); an entry with NaN z is no absorber, so rows may hold fewer; 0 <= num_absorbers <= 4, and the two
+ * arrays may be NULL only when it is 0.  meanflux = 1 evaluates the null model of the multi-DLA path (Lyman-series
+ * mean-flux suppression s and noise scaling), 0 that of process_qsos.m (s = 1).  For quasar q, over the pixels of the
+ * modelled window (min_lambda <= lambda / (1 + z_qso) <= max_lambda, masked ones included):
+ *   mu~, M~, om2~   the interpolated model exactly as the hot path evaluates it, suppressed by s
+ *   a               the product of the absorbers' instrument-convolved profiles on the padded window grid (voigt.c,
+ *                   params.num_lines lines, optical depth always evaluated directly)
+ * and over the used pixels (window, not masked), d = a^2 om2~ + v, r = y - a mu~, B = I + (a M~)' D^-1 (a M~),
+ * g = (a M~)' D^-1 r.  Outputs, each nullable (skipped when NULL); planes are [Q x L_max], NaN outside the window and
+ * past lengths[q]:
+ *   absorption      a
+ *   prior_mean      a mu~
+ *   prior_sd        sqrt(a^2 (sum_c M~_c^2 + om2~) + v); NaN on masked pixels
+ *   fit_mean        a (mu~ + M~ x^), the conditional mean of the smooth part
+ *   continuum       mu + M x^: the emitted continuum, without the forest's mean absorption and the absorbers
+ *   continuum_sd    sqrt(m' B^-1 m), m the unsuppressed interpolated row of M
+ *   latent [Q x k]  x^ = B^-1 g
+ *   chi2 [Q]        sum r^2/d - g' B^-1 g
+ *   log_likelihood  -1/2 (chi2 + sum log d + 2 sum log L_ii + n log 2pi), B = L L': the hot path's Gaussian log-density
+ *   num_pixels      n (int32)
+ * A quasar without a used pixel gets NaN everywhere and num_pixels = 0.  Needs a model (GPDLA_ERR_STATE without one);
+ * samples and prior are not read.  k = 10, 20, 40 (else GPDLA_ERR_UNSUPPORTED); L_max is bounded by one CTA's shared
+ * memory (about 20 000 pixels).  The argument checks (and, in the host entry, that every finite z is > -1 with a finite
+ * N >= 0) come before any CUDA call.  No atomics: repeated calls give the same bits, and the host entry those of the
+ * _device entry, which takes device arrays and is asynchronous on `stream`. */
+typedef struct {
+  double* absorption;
+  double* prior_mean;
+  double* prior_sd;
+  double* fit_mean;
+  double* continuum;
+  double* continuum_sd;
+  double* latent;
+  double* chi2;
+  double* log_likelihood;
+  int32_t* num_pixels;
+} gpdla_reconstruction;
+int gpdla_reconstruct(gpdla_ctx* ctx, int64_t Q, int64_t L_max, const double* wavelengths, const double* flux,
+                      const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                      const double* z_qsos, int32_t meanflux, int32_t num_absorbers, const double* absorber_z,
+                      const double* absorber_nhi, const gpdla_reconstruction* out);
+int gpdla_reconstruct_device(gpdla_ctx* ctx, int64_t Q, int64_t L_max, const double* wavelengths, const double* flux,
+                             const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                             const double* z_qsos, int32_t meanflux, int32_t num_absorbers, const double* absorber_z,
+                             const double* absorber_nhi, const gpdla_reconstruction* out, void* stream);
+
 /* voigt.c:253-304: profile has num_points - 6 entries.  Host buffers; runs on the current device. */
 int gpdla_voigt(const double* lambdas, int64_t num_points, double z, double N, int32_t num_lines, double* profile);
 /* Batched, device buffers: profile[s, :] = voigt(lambdas, z[s], N[s], num_lines), [S x (num_points-6)] */
