@@ -26,22 +26,26 @@ def load_golden_multi(golden_dir):
     return model, samples, spectra, prior, expect
 
 
-def assert_multi_parity(res, ref, check_base=True):
+def assert_multi_parity(res, ref, check_base=True, ll_rtol=LL_RTOL, check_map=True):
+    """``ll_rtol``: the log-likelihood bar (1e-9 for the 5-digit INT8 Gram and for extreme inputs, as on the
+    single-DLA path); ``check_map=False`` leaves the MAP to a caller that checks it only where it is tie-free."""
     if check_base:
         assert np.array_equal(res["base_sample_inds"], ref["base_sample_inds"])
     a, b = res["sample_log_likelihoods_dla"], ref["sample_log_likelihoods_dla"]
     assert np.array_equal(np.isnan(a), np.isnan(b))                      # z-separation filter / early exit pattern
-    assert np.allclose(a, b, rtol=LL_RTOL, atol=0, equal_nan=True)
-    assert np.allclose(res["sample_log_likelihoods_lls"], ref["sample_log_likelihoods_lls"], rtol=LL_RTOL, atol=0)
+    assert np.allclose(a, b, rtol=ll_rtol, atol=0, equal_nan=True)
+    assert np.array_equal(np.isnan(res["sample_log_likelihoods_lls"]), np.isnan(ref["sample_log_likelihoods_lls"]))
+    assert np.allclose(res["sample_log_likelihoods_lls"], ref["sample_log_likelihoods_lls"], rtol=ll_rtol, atol=0,
+                       equal_nan=True)
     for k in ("log_likelihoods_no_dla", "log_likelihoods_lls", "log_likelihoods_dla", "log_posteriors_no_dla",
               "log_posteriors_lls", "log_posteriors_dla"):
-        assert np.allclose(res[k], ref[k], rtol=LL_RTOL, atol=0, equal_nan=True), k
+        assert np.allclose(res[k], ref[k], rtol=ll_rtol, atol=0, equal_nan=True), k
     for k in ("log_priors_no_dla", "log_priors_lls", "log_priors_dla", "min_z_dlas", "max_z_dlas"):
         assert np.allclose(res[k], ref[k], rtol=1e-13, atol=0, equal_nan=True), k
     # MAP: same arg-max sample, except for exact ties -- at levels >= 2 resampling with replacement produces
     # samples that describe the same set of DLAs in a different order, whose likelihoods agree to rounding
     Q, MD = res["MAP_inds"].shape[:2]
-    for q in range(Q):
+    for q in range(Q if check_map else 0):
         for l in range(MD):
             i, j = res["MAP_inds"][q, l, 0], ref["MAP_inds"][q, l, 0]
             if i == j:
