@@ -24,6 +24,7 @@ from .params import DEFAULT, MULTI, Parameters, lya_wavelength
 RESULT_NAMES = ["min_z_dlas", "max_z_dlas", "log_priors_no_dla", "log_priors_dla", "log_likelihoods_no_dla",
                 "log_likelihoods_dla", "log_posteriors_no_dla", "log_posteriors_dla", "model_posteriors",
                 "p_no_dlas", "p_dlas", "map_z_dlas", "map_log_nhis"]
+DEFAULT_QUANTILES = (0.025, 0.16, 0.5, 0.84, 0.975)      # the 95 % and 68 % central intervals and the median
 
 
 def _f64(a) -> np.ndarray:
@@ -304,13 +305,19 @@ class DLAProcessor:
             None if bin_ is None else bin_.data_ptr(), ctypes.byref(res), ctypes.c_void_p(stream)), self._ctx)
         return out
 
-    def _stats_operands(self, dev, Q: int, S: int, width: int, select, sums):
-        """Device samples (copied once), the sums tensor to add into and the uint8 select mask of a statistics call."""
+    def _device_samples(self, dev, S: int):
+        """CUDA copies of (offset, log N, N) of the samples, made on the first call."""
         import torch
         if S != self.num_dla_samples:
             raise ValueError("sample_log_likelihoods_dla has %d samples, this processor %d" % (S, self.num_dla_samples))
         if self._samples_device is None:
             self._samples_device = tuple(torch.from_numpy(a).to(dev) for a in self._samples_host)
+        return self._samples_device
+
+    def _stats_operands(self, dev, Q: int, S: int, width: int, select, sums):
+        """Device samples (copied once), the sums tensor to add into and the uint8 select mask of a statistics call."""
+        import torch
+        self._device_samples(dev, S)
         if sums is None:
             sums = torch.zeros(width, dtype=torch.float64, device=dev)
         if not (sums.is_cuda and sums.device == dev and sums.dtype == torch.float64 and sums.is_contiguous()
@@ -381,6 +388,56 @@ class DLAProcessor:
                 ptr(off), ptr(lnhi), ptr(nhi), ze.size - 1, _dp(ze), ne.size - 1, _dp(ne), float(dla_log_nhi_min),
                 float(omega_m), ptr(sums), stream))
         return sums
+
+    def posteriors_device(self, out: Dict, quantiles=DEFAULT_QUANTILES,
+                          log_nhi_threshold: float = _params.dla_log_nhi_min):
+        """Per-quasar summary of the absorber posterior (``dla_posteriors``) of what ``process_device(...,
+        return_sample_log_likelihoods=True)`` returned, without the sample log-likelihoods leaving the GPU: a float64
+        CUDA tensor [Q, 7 + 2 P] (``unpack_dla_posteriors``).  Asynchronous on torch's current stream.  Uses device
+        copies of this processor's samples, made once."""
+        import torch
+        ll = out.get("sample_log_likelihoods_dla")
+        if ll is None:
+            raise ValueError("posteriors_device needs process_device(..., return_sample_log_likelihoods=True)")
+        dev = ll.device
+        Q, S = ll.shape
+        qs = _quantiles(quantiles)
+        off, lnhi, _ = self._device_samples(dev, S)
+        ll, zlo, zhi = ll.contiguous(), out["min_z_dlas"].contiguous(), out["max_z_dlas"].contiguous()
+        rec = torch.empty((Q, dla_posteriors_width(qs.size)), dtype=torch.float64, device=dev)
+        with torch.cuda.device(dev):
+            stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+            _lib.check(self._lib.gpdla_dla_posteriors_device(
+                Q, S, ctypes.c_void_p(ll.data_ptr()), ctypes.c_void_p(zlo.data_ptr()),
+                ctypes.c_void_p(zhi.data_ptr()), ctypes.c_void_p(off.data_ptr()), ctypes.c_void_p(lnhi.data_ptr()),
+                qs.size, _dp(qs), float(log_nhi_threshold), ctypes.c_void_p(rec.data_ptr()), stream))
+        return rec
+
+    def multi_posteriors_device(self, out: Dict):
+        """Per-quasar, per-level summary of the multi-DLA absorber posterior (``multi_dla_posteriors``) of what
+        ``process_multi_device(..., return_samples=True)`` returned: a float64 CUDA tensor [Q, J + 2 J (J + 1)]
+        (``unpack_multi_dla_posteriors``).  Asynchronous on torch's current stream."""
+        import torch
+        ll = out.get("sample_log_likelihoods_dla")
+        if ll is None:
+            raise ValueError("multi_posteriors_device needs process_multi_device(..., return_samples=True)")
+        dev = ll.device
+        Q, J, S = ll.shape
+        part = out.get("base_sample_inds")
+        if J > 1 and (part is None or tuple(part.shape) != (Q, J - 1, S) or part.dtype != torch.int32
+                      or not part.is_contiguous()):
+            raise ValueError("base_sample_inds must be a contiguous int32 tensor [Q, max_dlas - 1, S]")
+        if not all(out[n].is_contiguous() for n in ("sample_log_likelihoods_dla", "min_z_dlas", "max_z_dlas")):
+            raise ValueError("the arrays of process_multi_device must be contiguous")
+        off, lnhi, _ = self._device_samples(dev, S)
+        rec = torch.empty((Q, multi_dla_posteriors_width(J)), dtype=torch.float64, device=dev)
+        ptr = lambda t: None if t is None else ctypes.c_void_p(t.data_ptr())
+        with torch.cuda.device(dev):
+            stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+            _lib.check(self._lib.gpdla_multi_dla_posteriors_device(
+                Q, S, J, ptr(ll), ptr(part if J > 1 else None), ptr(out["min_z_dlas"]), ptr(out["max_z_dlas"]),
+                ptr(off), ptr(lnhi), ptr(rec), stream))
+        return rec
 
     # ---------------------------------------------------------------- fitted model under chosen absorbers
     def _recon_operands(self, Q: int, absorber_z, absorber_nhi, to):
@@ -1178,6 +1235,130 @@ def multi_dla_statistics_sums(results: Dict, samples: Dict, z_edges, log_nhi_edg
                                                   vp(lnhi), vp(nhi), ze.size - 1, _dp(ze), ne.size - 1, _dp(ne),
                                                   float(dla_log_nhi_min), float(omega_m), vp(out)))
     return out
+
+
+# ---------------------------------------------------------------- per-quasar absorber posteriors
+POSTERIOR_FIELDS = ["ess", "z_mean", "z_sd", "log_nhi_mean", "log_nhi_sd", "z_log_nhi_cov", "mass_above_threshold"]
+MULTI_POSTERIOR_FIELDS = ["z_mean", "z_sd", "log_nhi_mean", "log_nhi_sd"]
+
+
+def dla_posteriors_width(num_quantiles: int) -> int:
+    """Doubles per quasar of a single-DLA posterior record."""
+    return len(POSTERIOR_FIELDS) + 2 * int(num_quantiles)
+
+
+def multi_dla_posteriors_width(max_dlas: int) -> int:
+    """Doubles per quasar of a multi-DLA posterior record: per level j, ess_j and 4 moments of each of its j ranks."""
+    return int(max_dlas) + 2 * int(max_dlas) * (int(max_dlas) + 1)
+
+
+def _quantiles(quantiles) -> np.ndarray:
+    qs = _f64(quantiles).ravel()
+    if not 1 <= qs.size <= 16 or not np.all((qs > 0) & (qs < 1)):
+        raise ValueError("quantiles must hold 1 to 16 probabilities inside (0, 1)")
+    return qs
+
+
+def dla_posteriors(results: Dict, samples: Dict, quantiles=DEFAULT_QUANTILES,
+                   log_nhi_threshold: float = _params.dla_log_nhi_min, device: int = 0) -> np.ndarray:
+    """Per-quasar summary of the DLA-model posterior over the samples, computed on the GPU, from one ``process`` /
+    ``process_qsos`` result (host arrays, with ``sample_log_likelihoods_dla``) and the samples it was run with.
+    w_i = exp(ll_i - max ll) (NaN and -inf weigh 0); z_i is rounded as ``map_z_dlas``.  Returns [Q, 7 + 2 P]:
+    ess (Kish), z and log N means and standard deviations, their covariance, the posterior mass at log N >=
+    ``log_nhi_threshold`` and the lower inverse-CDF ``quantiles`` of z and of log N; ``unpack_dla_posteriors`` names
+    them.  A quasar with no finite weight or an empty z range gets NaN."""
+    import torch
+    lib = _lib.load()
+    qs = _quantiles(quantiles)
+    ll = _f64(results["sample_log_likelihoods_dla"])
+    if ll.ndim != 2:
+        raise ValueError("sample_log_likelihoods_dla must be (Q, S)")
+    Q, S = ll.shape
+    zlo, zhi = (_f64(results[n]).ravel() for n in ("min_z_dlas", "max_z_dlas"))
+    off, lnhi = (_f64(samples[k]).ravel() for k in ("offset_samples", "log_nhi_samples"))
+    if zlo.size != Q or zhi.size != Q or off.size != S or lnhi.size != S:
+        raise ValueError("results need Q entries per quasar and the samples S entries each (Q, S = %d, %d)" % (Q, S))
+    out = np.empty((Q, dla_posteriors_width(qs.size)))
+    vp = lambda a: ctypes.c_void_p(a.ctypes.data)
+    with torch.cuda.device(device):
+        _lib.check(lib.gpdla_dla_posteriors(Q, S, vp(ll), vp(zlo), vp(zhi), vp(off), vp(lnhi), qs.size, _dp(qs),
+                                            float(log_nhi_threshold), vp(out)))
+    return out
+
+
+def multi_dla_posteriors(results: Dict, samples: Dict, device: int = 0) -> np.ndarray:
+    """``dla_posteriors`` for the multi-DLA model, computed on the GPU, from one ``process_multi`` /
+    ``process_qsos_multiple_dlas_meanflux`` result in the reference layout -- ``sample_log_likelihoods_dla`` (Q, S, J),
+    ``base_sample_inds`` (Q, S, J-1), 0-based.  Per level j, ess_j and the posterior means and standard deviations of
+    z and log N of the absorber of rank r < j in ascending z (``unpack_multi_dla_posteriors``).  A level with no finite
+    weight or a partner index outside [0, S) is NaN.  Quantiles are not computed: the ranks have no quasar-independent
+    sample order."""
+    import torch
+    lib = _lib.load()
+    sll = np.asarray(results["sample_log_likelihoods_dla"], dtype=np.float64)
+    if sll.ndim != 3:
+        raise ValueError("sample_log_likelihoods_dla must be (Q, S, max_dlas)")
+    Q, S, J = sll.shape
+    ll = np.ascontiguousarray(np.transpose(sll, (0, 2, 1)))
+    part = None
+    if J > 1:
+        bsi = np.asarray(results["base_sample_inds"])
+        if bsi.shape != (Q, S, J - 1):
+            raise ValueError("base_sample_inds must be (Q, S, max_dlas - 1)")
+        part = np.ascontiguousarray(np.transpose(bsi, (0, 2, 1)), dtype=np.int32)
+    zlo, zhi = (_f64(results[n]).ravel() for n in ("min_z_dlas", "max_z_dlas"))
+    off, lnhi = (_f64(samples[k]).ravel() for k in ("offset_samples", "log_nhi_samples"))
+    if zlo.size != Q or zhi.size != Q or off.size != S or lnhi.size != S:
+        raise ValueError("results need Q entries per quasar and the samples S entries each (Q, S = %d, %d)" % (Q, S))
+    out = np.empty((Q, multi_dla_posteriors_width(J)))
+    vp = lambda a: None if a is None else ctypes.c_void_p(a.ctypes.data)
+    with torch.cuda.device(device):
+        _lib.check(lib.gpdla_multi_dla_posteriors(Q, S, J, vp(ll), vp(part), vp(zlo), vp(zhi), vp(off), vp(lnhi),
+                                                  vp(out)))
+    return out
+
+
+def unpack_dla_posteriors(rec, num_quantiles: int, num_samples: Optional[int] = None, p_dlas=None) -> Dict[str, np.ndarray]:
+    """A single-DLA posterior record [Q, 7 + 2 P] (host array or tensor) -> named arrays: the ``POSTERIOR_FIELDS``
+    [Q] and ``z_quantiles``, ``log_nhi_quantiles`` [Q, P].  With ``num_samples`` S it adds the Monte Carlo standard
+    deviation of the log evidence estimate, ``log_likelihood_dla_mc_sd = sqrt(max(1/ess - 1/S, 0))``, and with
+    ``p_dlas`` [Q] also ``p_dla_mc_sd = p (1 - p) log_likelihood_dla_mc_sd``.  Both are delta-method figures for iid
+    draws from the prior; for the quasi-Monte Carlo samples they are an upper estimate."""
+    v = np.asarray(rec.cpu().numpy() if hasattr(rec, "cpu") else rec, dtype=np.float64)
+    P = int(num_quantiles)
+    if v.ndim != 2 or v.shape[1] != dla_posteriors_width(P):
+        raise ValueError("records must be [Q, %d] for %d quantiles" % (dla_posteriors_width(P), P))
+    out = {n: v[:, i].copy() for i, n in enumerate(POSTERIOR_FIELDS)}
+    k = len(POSTERIOR_FIELDS)
+    out["z_quantiles"], out["log_nhi_quantiles"] = v[:, k:k + P].copy(), v[:, k + P:k + 2 * P].copy()
+    if num_samples is not None:
+        with np.errstate(invalid="ignore", divide="ignore"):
+            out["log_likelihood_dla_mc_sd"] = np.sqrt(np.maximum(1.0 / out["ess"] - 1.0 / int(num_samples), 0.0))
+        if p_dlas is not None:
+            p = _f64(p_dlas.cpu().numpy() if hasattr(p_dlas, "cpu") else p_dlas).ravel()
+            out["p_dla_mc_sd"] = p * (1.0 - p) * out["log_likelihood_dla_mc_sd"]
+    return out
+
+
+def unpack_multi_dla_posteriors(rec, max_dlas: int) -> Dict[str, np.ndarray]:
+    """A multi-DLA posterior record [Q, J + 2 J (J + 1)] -> ``ess`` [Q, J] and ``z_mean``, ``z_sd``, ``log_nhi_mean``,
+    ``log_nhi_sd`` [Q, J, J], indexed (level - 1, rank); entries with rank >= level are NaN."""
+    v = np.asarray(rec.cpu().numpy() if hasattr(rec, "cpu") else rec, dtype=np.float64)
+    J = int(max_dlas)
+    if v.ndim != 2 or v.shape[1] != multi_dla_posteriors_width(J):
+        raise ValueError("records must be [Q, %d] for max_dlas = %d" % (multi_dla_posteriors_width(J), J))
+    Q = v.shape[0]
+    out = {"ess": np.empty((Q, J))}
+    out.update({n: np.full((Q, J, J), np.nan) for n in MULTI_POSTERIOR_FIELDS})
+    c = 0
+    for j in range(1, J + 1):
+        out["ess"][:, j - 1] = v[:, c]
+        block = v[:, c + 1:c + 1 + 4 * j].reshape(Q, j, 4)
+        for i, n in enumerate(MULTI_POSTERIOR_FIELDS):
+            out[n][:, j - 1, :j] = block[:, :, i]
+        c += 1 + 4 * j
+    return out
+
 
 def omega_dla_coefficient(hubble_h: float = _params.hubble_h) -> float:
     """8 pi G m_H / (3 c H0) in cm^2: Omega_DLA = this x (sum of N_HI) / (absorption path).  HI only, no helium."""

@@ -22,6 +22,7 @@
 #include "gpdla_objective.cuh"
 #include "gpdla_training.cuh"
 #include "gpdla_statistics.cuh"
+#include "gpdla_posteriors.cuh"
 #include "gpdla_reconstruct.cuh"
 #include "gpdla_rest_table.h"
 
@@ -2175,6 +2176,180 @@ int gpdla_multi_dla_statistics(int64_t Q, int64_t S, int32_t max_dlas, const dou
                                            n_z, z_edges, n_nhi, log_nhi_edges, dla_log_nhi_min, omega_m, d_sums,
                                            nullptr);
     if (rc == GPDLA_OK) e = cudaMemcpy(sums, d_sums, W * 8, cudaMemcpyDeviceToHost);
+  }
+  if (e != cudaSuccess) { g_err = std::string(fn) + ": " + cudaGetErrorString(e); rc = GPDLA_ERR_CUDA; }
+  cudaFree(base);
+  return rc;
+}
+
+// ---- per-quasar summaries of the absorber posterior ----
+
+// the checks of every posterior entry before any CUDA call; quantiles only for the single-DLA entries (max_dlas 0)
+static int post_check(const char* fn, int64_t Q, int64_t S, int32_t max_dlas, const double* ll,
+                      const int32_t* base_sample_inds, const double* min_z_dlas, const double* max_z_dlas,
+                      const double* offset_samples, const double* log_nhi_samples, int32_t num_quantiles,
+                      const double* quantiles, double log_nhi_threshold, const double* out) {
+  auto fail = [&](const std::string& why) { g_err = std::string(fn) + ": " + why; return GPDLA_ERR_INVALID; };
+  if (Q < 0 || Q > INT32_MAX || S < 1 || S > INT32_MAX) return fail("Q must lie in [0, 2^31) and S in [1, 2^31)");
+  if (!offset_samples || !log_nhi_samples || (Q > 0 && (!ll || !min_z_dlas || !max_z_dlas || !out)))
+    return fail("a required array is NULL");
+  if (max_dlas == 0) {
+    if (num_quantiles < 1 || num_quantiles > POST_MAX_P)
+      return fail("num_quantiles = " + std::to_string(num_quantiles) + " is outside [1, " + std::to_string(POST_MAX_P) + "]");
+    if (!quantiles) return fail("a required array is NULL");
+    for (int p = 0; p < num_quantiles; ++p)
+      if (!(quantiles[p] > 0.0 && quantiles[p] < 1.0))
+        return fail("quantiles[" + std::to_string(p) + "] is not inside (0, 1)");
+    if (!std::isfinite(log_nhi_threshold)) return fail("log_nhi_threshold is not finite");
+  } else {
+    if (max_dlas < 1 || max_dlas > MSTAT_MAX_DLAS)
+      return fail("max_dlas = " + std::to_string(max_dlas) + " is outside [1, " + std::to_string(MSTAT_MAX_DLAS) + "]");
+    if (Q > 0 && max_dlas > 1 && !base_sample_inds) return fail("base_sample_inds may be NULL only when max_dlas == 1");
+  }
+  return GPDLA_OK;
+}
+
+int gpdla_dla_posteriors_device(int64_t Q, int64_t S, const double* sample_log_likelihoods_dla,
+                                const double* min_z_dlas, const double* max_z_dlas, const double* offset_samples,
+                                const double* log_nhi_samples, int32_t num_quantiles, const double* quantiles,
+                                double log_nhi_threshold, double* out, void* stream) {
+  const char* fn = "gpdla_dla_posteriors_device";
+  int rc = post_check(fn, Q, S, 0, sample_log_likelihoods_dla, nullptr, min_z_dlas, max_z_dlas, offset_samples,
+                      log_nhi_samples, num_quantiles, quantiles, log_nhi_threshold, out);
+  if (rc) return rc;
+  if (Q == 0) return GPDLA_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int64_t C = posterior_chunk(S);
+  PostArgs a;
+  a.ll = sample_log_likelihoods_dla; a.min_z_dlas = min_z_dlas; a.max_z_dlas = max_z_dlas; a.S = S; a.C = C;
+  a.P = num_quantiles;
+  for (int p = 0; p < num_quantiles; ++p) a.prob[p] = quantiles[p];
+  a.threshold = log_nhi_threshold; a.out = out;
+  int dev = 0, optin = 0;
+  CUDA_TRY(cudaGetDevice(&dev), g_err);
+  CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev), g_err);
+  const bool staged = (size_t)S * 8 + 4096 <= (size_t)optin;   // 4 KB: room for the static shared memory
+  const size_t smem = staged ? (size_t)S * 8 : 0;
+  const size_t bytes = (size_t)S * (3 * 8 + 8 + 4 + 4 * 4) + (size_t)C * POST_THREADS * 4 + 8 * 64;
+  char* base = nullptr;
+  CUDA_TRY(cudaMallocAsync(&base, bytes, st), g_err);
+  char* ptr = base;
+  auto take = [&](size_t n) { char* r = ptr; ptr += (n + 15) / 16 * 16; return r; };
+  double* z_offset = (double*)take(S * 8); double* z_lnhi = (double*)take(S * 8); double* n_lnhi = (double*)take(S * 8);
+  uint64_t* key = (uint64_t*)take(S * 8);
+  int32_t* cls = (int32_t*)take(S * 4); int32_t* z_perm = (int32_t*)take(S * 4); int32_t* z_rank = (int32_t*)take(S * 4);
+  int32_t* n_perm = (int32_t*)take(S * 4); int32_t* n_rank = (int32_t*)take(S * 4);
+  int32_t* class_start = (int32_t*)take(2 * 4);
+  int32_t* n_chunk = (int32_t*)take((size_t)C * POST_THREADS * 4);
+  a.z_offset = z_offset; a.z_lnhi = z_lnhi; a.z_perm = z_perm; a.z_rank = z_rank; a.n_lnhi = n_lnhi; a.n_chunk = n_chunk;
+  // the two sample orders, with the statistics' counting rank and one class: by offset, and by log N
+  const unsigned sblocks = (unsigned)((S + STAT_THREADS - 1) / STAT_THREADS);
+  StatsClassArgs ca;
+  ca.S = S; ca.nbound = 0; ca.cls = cls; ca.key = key;
+  ca.offset = offset_samples; ca.log_nhi = log_nhi_samples;
+  stats_class_kernel<<<sblocks, STAT_THREADS, 0, st>>>(ca);
+  stats_rank_kernel<<<sblocks, STAT_THREADS, 0, st>>>(cls, key, S, z_perm);
+  stats_gather_kernel<<<sblocks, STAT_THREADS, 0, st>>>(z_perm, cls, offset_samples, log_nhi_samples, S, 0, z_offset,
+                                                        z_lnhi, z_rank, class_start);
+  ca.offset = log_nhi_samples;                                  // the key of the second order
+  stats_class_kernel<<<sblocks, STAT_THREADS, 0, st>>>(ca);
+  stats_rank_kernel<<<sblocks, STAT_THREADS, 0, st>>>(cls, key, S, n_perm);
+  stats_gather_kernel<<<sblocks, STAT_THREADS, 0, st>>>(n_perm, cls, log_nhi_samples, log_nhi_samples, S, 0, n_lnhi,
+                                                        (double*)key, n_rank, class_start);   // key: ranked, unused
+
+  posterior_chunk_kernel<<<(unsigned)((C * POST_THREADS + 255) / 256), 256, 0, st>>>(n_perm, z_rank, S, C, n_chunk);
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess && staged)
+    e = cudaFuncSetAttribute(dla_posterior_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e == cudaSuccess) {
+    if (staged) dla_posterior_kernel<true><<<(unsigned)Q, POST_THREADS, smem, st>>>(a);
+    else dla_posterior_kernel<false><<<(unsigned)Q, POST_THREADS, 0, st>>>(a);
+    e = cudaGetLastError();
+  }
+  const cudaError_t ef = cudaFreeAsync(base, st);   // freed on the error path too
+  if (e == cudaSuccess) e = ef;
+  if (e != cudaSuccess) { g_err = std::string(fn) + ": " + cudaGetErrorString(e); return GPDLA_ERR_CUDA; }
+  return GPDLA_OK;
+}
+
+int gpdla_dla_posteriors(int64_t Q, int64_t S, const double* sample_log_likelihoods_dla, const double* min_z_dlas,
+                         const double* max_z_dlas, const double* offset_samples, const double* log_nhi_samples,
+                         int32_t num_quantiles, const double* quantiles, double log_nhi_threshold, double* out) {
+  const char* fn = "gpdla_dla_posteriors";
+  int rc = post_check(fn, Q, S, 0, sample_log_likelihoods_dla, nullptr, min_z_dlas, max_z_dlas, offset_samples,
+                      log_nhi_samples, num_quantiles, quantiles, log_nhi_threshold, out);
+  if (rc) return rc;
+  const size_t QS = (size_t)Q * S, W = (size_t)Q * posterior_width(num_quantiles), Sb = (size_t)S * 8;
+  const size_t bytes = QS * 8 + (size_t)Q * 2 * 8 + 2 * Sb + W * 8 + 6 * 64;
+  char* base = nullptr;
+  CUDA_TRY(cudaMalloc(&base, bytes), g_err);
+  char* ptr = base;
+  auto take = [&](size_t n) { char* r = ptr; ptr += (n + 15) / 16 * 16; return r; };
+  double* d_ll = (double*)take(QS * 8);
+  double* d_zlo = (double*)take((size_t)Q * 8); double* d_zhi = (double*)take((size_t)Q * 8);
+  double* d_off = (double*)take(Sb); double* d_lnhi = (double*)take(Sb);
+  double* d_out = (double*)take(W * 8);
+  cudaError_t e = cudaSuccess;
+  auto up = [&](void* d, const void* h, size_t n) { if (e == cudaSuccess && n) e = cudaMemcpy(d, h, n, cudaMemcpyHostToDevice); };
+  up(d_ll, sample_log_likelihoods_dla, QS * 8); up(d_zlo, min_z_dlas, (size_t)Q * 8); up(d_zhi, max_z_dlas, (size_t)Q * 8);
+  up(d_off, offset_samples, Sb); up(d_lnhi, log_nhi_samples, Sb);
+  rc = GPDLA_ERR_CUDA;
+  if (e == cudaSuccess) {
+    rc = gpdla_dla_posteriors_device(Q, S, d_ll, d_zlo, d_zhi, d_off, d_lnhi, num_quantiles, quantiles,
+                                     log_nhi_threshold, d_out, nullptr);
+    if (rc == GPDLA_OK && W) e = cudaMemcpy(out, d_out, W * 8, cudaMemcpyDeviceToHost);
+  }
+  if (e != cudaSuccess) { g_err = std::string(fn) + ": " + cudaGetErrorString(e); rc = GPDLA_ERR_CUDA; }
+  cudaFree(base);
+  return rc;
+}
+
+int gpdla_multi_dla_posteriors_device(int64_t Q, int64_t S, int32_t max_dlas, const double* sample_log_likelihoods_dla,
+                                      const int32_t* base_sample_inds, const double* min_z_dlas,
+                                      const double* max_z_dlas, const double* offset_samples,
+                                      const double* log_nhi_samples, double* out, void* stream) {
+  const char* fn = "gpdla_multi_dla_posteriors_device";
+  int rc = post_check(fn, Q, S, max_dlas, sample_log_likelihoods_dla, base_sample_inds, min_z_dlas, max_z_dlas,
+                      offset_samples, log_nhi_samples, 0, nullptr, 0.0, out);
+  if (rc) return rc;
+  if (Q == 0) return GPDLA_OK;
+  MultiPostArgs a;
+  a.ll = sample_log_likelihoods_dla; a.partners = max_dlas > 1 ? base_sample_inds : nullptr;
+  a.min_z_dlas = min_z_dlas; a.max_z_dlas = max_z_dlas; a.S = S; a.J = max_dlas;
+  a.offset = offset_samples; a.log_nhi = log_nhi_samples; a.out = out;
+  multi_dla_posterior_kernel<<<(unsigned)Q, STAT_THREADS, 0, (cudaStream_t)stream>>>(a);
+  const cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) { g_err = std::string(fn) + ": " + cudaGetErrorString(e); return GPDLA_ERR_CUDA; }
+  return GPDLA_OK;
+}
+
+int gpdla_multi_dla_posteriors(int64_t Q, int64_t S, int32_t max_dlas, const double* sample_log_likelihoods_dla,
+                               const int32_t* base_sample_inds, const double* min_z_dlas, const double* max_z_dlas,
+                               const double* offset_samples, const double* log_nhi_samples, double* out) {
+  const char* fn = "gpdla_multi_dla_posteriors";
+  int rc = post_check(fn, Q, S, max_dlas, sample_log_likelihoods_dla, base_sample_inds, min_z_dlas, max_z_dlas,
+                      offset_samples, log_nhi_samples, 0, nullptr, 0.0, out);
+  if (rc) return rc;
+  const size_t J = (size_t)max_dlas, P = max_dlas > 1 ? (size_t)Q * (J - 1) * S : 0;
+  const size_t QJS = (size_t)Q * J * S, W = (size_t)Q * multi_posterior_width(max_dlas), Sb = (size_t)S * 8;
+  const size_t bytes = QJS * 8 + P * 4 + (size_t)Q * 2 * 8 + 2 * Sb + W * 8 + 7 * 64;
+  char* base = nullptr;
+  CUDA_TRY(cudaMalloc(&base, bytes), g_err);
+  char* ptr = base;
+  auto take = [&](size_t n) { char* r = ptr; ptr += (n + 15) / 16 * 16; return r; };
+  double* d_ll = (double*)take(QJS * 8); int32_t* d_part = P ? (int32_t*)take(P * 4) : nullptr;
+  double* d_zlo = (double*)take((size_t)Q * 8); double* d_zhi = (double*)take((size_t)Q * 8);
+  double* d_off = (double*)take(Sb); double* d_lnhi = (double*)take(Sb);
+  double* d_out = (double*)take(W * 8);
+  cudaError_t e = cudaSuccess;
+  auto up = [&](void* d, const void* h, size_t n) { if (e == cudaSuccess && n) e = cudaMemcpy(d, h, n, cudaMemcpyHostToDevice); };
+  up(d_ll, sample_log_likelihoods_dla, QJS * 8); up(d_part, base_sample_inds, P * 4);
+  up(d_zlo, min_z_dlas, (size_t)Q * 8); up(d_zhi, max_z_dlas, (size_t)Q * 8);
+  up(d_off, offset_samples, Sb); up(d_lnhi, log_nhi_samples, Sb);
+  rc = GPDLA_ERR_CUDA;
+  if (e == cudaSuccess) {
+    rc = gpdla_multi_dla_posteriors_device(Q, S, max_dlas, d_ll, d_part, d_zlo, d_zhi, d_off, d_lnhi, d_out, nullptr);
+    if (rc == GPDLA_OK && W) e = cudaMemcpy(out, d_out, W * 8, cudaMemcpyDeviceToHost);
   }
   if (e != cudaSuccess) { g_err = std::string(fn) + ": " + cudaGetErrorString(e); rc = GPDLA_ERR_CUDA; }
   cudaFree(base);

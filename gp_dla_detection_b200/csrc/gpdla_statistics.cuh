@@ -277,7 +277,7 @@ __global__ void stats_finish_kernel(const double* __restrict__ psum, int nblocks
 // and variance.  With v_j(i) = p_j w_ji and g_t(i) = sum_{j > t} v_j(i), E[X] = sum_i sum_t g_t a_t and
 // E[X^2] = E[X] + 2 sum_i sum_{t < t'} g_t' a_t a_t' (a_t: slot t lies in the cell; slot t' exists wherever t' does).
 //   multi_dla_stats_kernel    one CTA per quasar: per-level log-sum-exp and the partner bounds check in one pass over
-//                             the rows, then every warp takes 32 samples at a time, merges each sample's slots by
+//                             the rows (multi_level_lse, shared with gpdla_posteriors.cuh), then every warp takes 32 samples at a time, merges each sample's slots by
 //                             cell in registers, and adds them into a warp-private accumulator: lanes sharing a cell
 //                             (__match_any_sync) are summed in lane order by the lowest one.  The warps' accumulators
 //                             are added in warp order.  No atomics; the order depends only on the launch shape.
@@ -324,9 +324,54 @@ __device__ __forceinline__ void lse_merge(double& m, double& s, double m2, doubl
   m = mm;
 }
 
+// Pass 1 of both multi-DLA reductions (this file and gpdla_posteriors.cuh), one read of the J rows [J x S] of a quasar:
+// every thread of the CTA gets each level's log-sum-exp (m, s) over the levels in `use` (s == 0: nothing seen), merged
+// in a fixed order, and the returned mask has bit t set when partner row t < nrows holds an index outside [0, S).
+// Shared memory: red [nwarps x MSTAT_MAX_DLAS x 2] doubles, s_bad [nwarps] ints.
+__device__ __forceinline__ int multi_level_lse(const double* __restrict__ ll, const int32_t* __restrict__ part, int64_t S,
+                                               const bool use[MSTAT_MAX_DLAS], int nrows, double* red, int* s_bad,
+                                               double m[MSTAT_MAX_DLAS], double s[MSTAT_MAX_DLAS]) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = blockDim.x >> 5;
+#pragma unroll
+  for (int j = 0; j < MSTAT_MAX_DLAS; ++j) { m[j] = -INFINITY; s[j] = 0.0; }
+  int bad = 0;
+  for (int64_t i = tid; i < S; i += blockDim.x) {
+    double v[MSTAT_MAX_DLAS];
+    int32_t k[MSTAT_MAX_DLAS - 1];
+#pragma unroll
+    for (int j = 0; j < MSTAT_MAX_DLAS; ++j) v[j] = use[j] ? ll[j * S + i] : NAN;
+#pragma unroll
+    for (int t = 0; t < MSTAT_MAX_DLAS - 1; ++t) k[t] = t < nrows ? part[t * S + i] : 0;
+#pragma unroll
+    for (int j = 0; j < MSTAT_MAX_DLAS; ++j) lse_push(m[j], s[j], v[j]);
+#pragma unroll
+    for (int t = 0; t < MSTAT_MAX_DLAS - 1; ++t) bad |= ((k[t] < 0) | (k[t] >= S)) << t;
+  }
+#pragma unroll
+  for (int j = 0; j < MSTAT_MAX_DLAS; ++j)
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1)
+      lse_merge(m[j], s[j], __shfl_xor_sync(0xffffffffu, m[j], o), __shfl_xor_sync(0xffffffffu, s[j], o));
+  bad = __reduce_or_sync(0xffffffffu, bad);
+  if (lane == 0) {
+    s_bad[warp] = bad;
+#pragma unroll
+    for (int j = 0; j < MSTAT_MAX_DLAS; ++j) { red[(warp * MSTAT_MAX_DLAS + j) * 2] = m[j]; red[(warp * MSTAT_MAX_DLAS + j) * 2 + 1] = s[j]; }
+  }
+  __syncthreads();
+  bad = 0;
+#pragma unroll
+  for (int j = 0; j < MSTAT_MAX_DLAS; ++j) {                   // every thread adds the warps in the same order
+    m[j] = red[j * 2]; s[j] = red[j * 2 + 1];
+    for (int w = 1; w < nw; ++w) lse_merge(m[j], s[j], red[(w * MSTAT_MAX_DLAS + j) * 2], red[(w * MSTAT_MAX_DLAS + j) * 2 + 1]);
+  }
+  for (int w = 0; w < nw; ++w) bad |= s_bad[w];
+  return bad;
+}
+
 __global__ void __launch_bounds__(STAT_THREADS) multi_dla_stats_kernel(const __grid_constant__ MultiStatsArgs a) {
   extern __shared__ __align__(16) double ms_smem[];
-  __shared__ int s_bad;
+  __shared__ int s_bad[STAT_THREADS / 32];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = blockDim.x >> 5;
   const int64_t q = a.q0 + blockIdx.x, S = a.S;
   const int J = a.J, nzn = a.n_z * a.n_nhi, A = mstats_acc_width(a.n_z, a.n_nhi);
@@ -341,52 +386,21 @@ __global__ void __launch_bounds__(STAT_THREADS) multi_dla_stats_kernel(const __g
   bool ok = (a.select ? a.select[q] != 0 : true) && zhi > zlo;
   for (int c = 0; c < J + 2; ++c) ok = ok && isfinite(mp[c]);
   double p[MSTAT_MAX_DLAS];
+  bool use[MSTAT_MAX_DLAS];
   int jmax = 0;                                                // levels 1..jmax can contribute; partner rows < jmax - 1
 #pragma unroll
   for (int j = 0; j < MSTAT_MAX_DLAS; ++j) {
     p[j] = (ok && j < J) ? mp[2 + j] : 0.0;
-    if (p[j] > 0.0) jmax = j + 1;
+    use[j] = p[j] > 0.0;
+    if (use[j]) jmax = j + 1;
   }
-  if (tid == 0) s_bad = 0;
-  __syncthreads();
   double m[MSTAT_MAX_DLAS], s[MSTAT_MAX_DLAS];
-#pragma unroll
-  for (int j = 0; j < MSTAT_MAX_DLAS; ++j) { m[j] = -INFINITY; s[j] = 0.0; }
-  if (ok) {                                                    // pass 1: per-level LSE, partner bounds
-    int bad = 0;
-    for (int64_t i = tid; i < S; i += blockDim.x) {
-      double v[MSTAT_MAX_DLAS];
-      int32_t k[MSTAT_MAX_DLAS - 1];
-#pragma unroll
-      for (int j = 0; j < MSTAT_MAX_DLAS; ++j) v[j] = p[j] > 0.0 ? ll[j * S + i] : NAN;
-#pragma unroll
-      for (int t = 0; t < MSTAT_MAX_DLAS - 1; ++t) k[t] = t + 1 < jmax ? part[t * S + i] : 0;
-#pragma unroll
-      for (int j = 0; j < MSTAT_MAX_DLAS; ++j) lse_push(m[j], s[j], v[j]);
-#pragma unroll
-      for (int t = 0; t < MSTAT_MAX_DLAS - 1; ++t) bad |= (k[t] < 0) | (k[t] >= S);
-    }
+  if (ok) {                                                    // ok is the same for the whole CTA
+    const int bad = multi_level_lse(ll, part, S, use, jmax - 1, red, s_bad, m, s);   // pass 1: per-level LSE, partner bounds
 #pragma unroll
     for (int j = 0; j < MSTAT_MAX_DLAS; ++j)
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1)
-        lse_merge(m[j], s[j], __shfl_xor_sync(0xffffffffu, m[j], o), __shfl_xor_sync(0xffffffffu, s[j], o));
-    bad = __any_sync(0xffffffffu, bad);
-    if (lane == 0) {
-      if (bad) s_bad = 1;                                      // benign: every writer stores 1
-#pragma unroll
-      for (int j = 0; j < MSTAT_MAX_DLAS; ++j) { red[(warp * MSTAT_MAX_DLAS + j) * 2] = m[j]; red[(warp * MSTAT_MAX_DLAS + j) * 2 + 1] = s[j]; }
-    }
-  }
-  __syncthreads();
-  if (ok) {
-#pragma unroll
-    for (int j = 0; j < MSTAT_MAX_DLAS; ++j) {                 // every thread adds the warps in the same order
-      m[j] = red[j * 2]; s[j] = red[j * 2 + 1];
-      for (int w = 1; w < nw; ++w) lse_merge(m[j], s[j], red[(w * MSTAT_MAX_DLAS + j) * 2], red[(w * MSTAT_MAX_DLAS + j) * 2 + 1]);
       if (p[j] > 0.0 && !isfinite(m[j])) ok = false;           // then s lies in [1, S]
-    }
-    ok = ok && !s_bad;
+    ok = ok && !bad;
   }
   if (!ok) {                                                   // contributes nothing, not even path or a count
     for (int64_t c = tid; c < a.W; c += blockDim.x) row[c] = 0.0;

@@ -7,7 +7,8 @@ modelled window x samples); every rank (one process per GPU) runs the hot path o
 no data-path collective, and ONE ``all_gather`` of fixed-width per-quasar records (NCCL over
 NVLink on GPUs, gloo in CPU tests) reassembles the catalogue.  ``sample_log_likelihoods_dla``
 (80 KB/quasar) stays sharded; ``dla_statistics_sharded`` (and ``multi_dla_statistics_sharded`` for the multi-DLA
-model) reduces it to the population-statistics sums on the rank that produced it and gathers only those (a few KB).
+model) reduces it to the population-statistics sums on the rank that produced it and gathers only those (a few KB);
+``dla_posteriors_sharded`` reduces it to one fixed-width posterior summary per quasar and gathers those.
 """
 from __future__ import annotations
 
@@ -76,18 +77,18 @@ def unpack_records(rec: np.ndarray) -> Dict[str, np.ndarray]:
     return out
 
 
-def gather_records(local: np.ndarray, blocks: List[Tuple[int, int]], device=None) -> np.ndarray:
-    """One all_gather of the padded record blocks; returns the catalogue-ordered ``[Q x RECORD_WIDTH]``."""
+def gather_records(local: np.ndarray, blocks: List[Tuple[int, int]], device=None, width: int = RECORD_WIDTH) -> np.ndarray:
+    """One all_gather of the padded record blocks; returns the catalogue-ordered ``[Q x width]``."""
     import torch
     import torch.distributed as dist
     world = dist.get_world_size()
     qmax = max(e - s for s, e in blocks)
-    buf = torch.zeros((max(qmax, 1), RECORD_WIDTH), dtype=torch.float64, device=device)
+    buf = torch.zeros((max(qmax, 1), width), dtype=torch.float64, device=device)
     if local.shape[0]:
         buf[:local.shape[0]] = torch.from_numpy(local).to(buf.device)
-    out = torch.empty((world * buf.shape[0], RECORD_WIDTH), dtype=torch.float64, device=device)
+    out = torch.empty((world * buf.shape[0], width), dtype=torch.float64, device=device)
     dist.all_gather_into_tensor(out, buf)
-    out = out.cpu().numpy().reshape(world, buf.shape[0], RECORD_WIDTH)
+    out = out.cpu().numpy().reshape(world, buf.shape[0], width)
     return np.concatenate([out[r, :e - s] for r, (s, e) in enumerate(blocks)], axis=0)
 
 
@@ -222,4 +223,51 @@ def _device_statistics(model, samples, prior, params, z_edges, log_nhi_edges, dl
             proc.statistics_device(out, z_edges, log_nhi_edges, select=up(sel, np.uint8), sums=state["sums"],
                                    dla_log_nhi_min=dla_log_nhi_min, omega_m=omega_m)
         return state["sums"]
+    return compute
+
+
+def dla_posteriors_sharded(model: Dict, samples: Dict, spectra: Dict, prior: Dict, quantiles=None,
+                           log_nhi_threshold: float = None, params=None, batch_quasars: int = 4096,
+                           compute: Callable[[Dict], np.ndarray] = None, device=None) -> Dict:
+    """Per-quasar posterior summaries (``api.dla_posteriors``) of the whole catalogue on every rank.  Every rank calls
+    this with the FULL catalogue description; rank r runs its cost-balanced block through ``process_device`` and
+    ``posteriors_device`` in batches of ``batch_quasars``, and one ``all_gather`` of the fixed-width records follows.
+    ``compute(spectra) -> records`` replaces the CUDA path of one rank (tests inject a CPU stand-in).  Returns
+    ``records`` [Q x (7 + 2 P)] in catalogue order (``api.unpack_dla_posteriors``) and ``blocks``."""
+    import torch.distributed as dist
+    from . import params as P
+    from .api import DEFAULT_QUANTILES, dla_posteriors_width
+    quantiles = np.asarray(DEFAULT_QUANTILES if quantiles is None else quantiles, dtype=np.float64).ravel()
+    log_nhi_threshold = P.dla_log_nhi_min if log_nhi_threshold is None else log_nhi_threshold
+    rank, world = dist.get_rank(), dist.get_world_size()
+    blocks = partition_by_cost(quasar_costs(spectra), world)
+    s, e = blocks[rank]
+    width = dla_posteriors_width(quantiles.size)
+    if compute is None and e > s:
+        compute = _device_posteriors(model, samples, prior, params, quantiles, log_nhi_threshold)
+    step = max(int(batch_quasars), 1)
+    parts = [np.asarray(compute(slice_spectra(spectra, b0, min(e, b0 + step))), dtype=np.float64).reshape(-1, width)
+             for b0 in range(s, e, step)]
+    local = np.concatenate(parts, axis=0) if parts else np.zeros((0, width))
+    return dict(records=gather_records(local, blocks, device=device, width=width), blocks=blocks)
+
+
+def _device_posteriors(model, samples, prior, params, quantiles, log_nhi_threshold):
+    """The CUDA path of one rank: spectra -> process_device -> posteriors_device -> host records."""
+    import os
+    import torch
+    from .api import DLAProcessor, pad_spectra
+    from .params import DEFAULT
+    dev = int(os.environ.get("LOCAL_RANK", 0))
+    proc = DLAProcessor(model, samples, prior, params or DEFAULT, device=dev)
+
+    def compute(sp):
+        pad = pad_spectra(sp)
+        d = torch.device("cuda", dev)
+        up = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dtype=dt)).to(d)
+        out = proc.process_device(up(pad["wavelengths"], np.float64), up(pad["flux"], np.float64),
+                                  up(pad["noise_variance"], np.float64), up(pad["pixel_mask"], np.uint8),
+                                  up(pad["lengths"], np.int32), up(pad["z_qsos"], np.float64),
+                                  return_sample_log_likelihoods=True)
+        return proc.posteriors_device(out, quantiles, log_nhi_threshold).cpu().numpy()
     return compute

@@ -352,6 +352,50 @@ int gpdla_multi_dla_statistics_device(int64_t Q, int64_t S, int32_t max_dlas, co
                                       const double* log_nhi_edges, double dla_log_nhi_min, double omega_m,
                                       double* sums, void* stream);
 
+/* ---- Per-quasar summaries of the absorber posterior: error bars, effective sample size and the DLA-threshold mass
+ * that the point estimates (map_z_dlas, map_log_nhis, MAP_*) do not carry ----
+ * Single-DLA model.  Inputs as gpdla_dla_statistics takes them: sample_log_likelihoods_dla [Q x S] (gpdla_process_qsos
+ * output), min_z_dlas, max_z_dlas [Q], offset_samples, log_nhi_samples [S].  The sample posterior of quasar q is
+ * w_i = exp(ll_i - max ll) (NaN and -inf entries weigh 0); the samples are prior draws, so this is the DLA-model
+ * posterior over the sample set (process_qsos.m:203-210).  z_i = min_z + (max_z - min_z) * offset_i, each operation
+ * rounded, as map_z_dlas.  out [Q x (7 + 2 num_quantiles)], float64, per quasar:
+ *   ess                    Kish's effective sample size (sum w)^2 / sum w^2
+ *   z_mean, z_sd           posterior mean and standard deviation of z_DLA (two-pass central moments)
+ *   log_nhi_mean, log_nhi_sd, z_log_nhi_cov   the same of log10 N_HI, and the covariance of the two
+ *   mass_above_threshold   sum over log N_i >= log_nhi_threshold of w_i / sum w (p_dla times it: a DLA proper)
+ *   z_quantiles[P], log_nhi_quantiles[P]   the lower inverse CDF at quantiles[p]: the value of the first sample, in
+ *                          value order, whose cumulative weight reaches quantiles[p] * (the scan's total weight)
+ * A quasar with no finite weight, or with max_z_dlas <= min_z_dlas (or NaN), gets a NaN record.  Checks before any
+ * CUDA call, else GPDLA_ERR_INVALID: 0 <= Q < 2^31, 1 <= S < 2^31, 1 <= num_quantiles <= 16, every quantile inside
+ * (0, 1) (NaN is not), a finite log_nhi_threshold, no NULL array (the per-quasar ones may be NULL when Q == 0).
+ * No atomics: repeated calls give the same bits, and the host entry those of the _device entry, which takes device
+ * arrays (quantiles stays a host array) and is asynchronous on `stream`.  Context-free, on the current device. */
+int gpdla_dla_posteriors(int64_t Q, int64_t S, const double* sample_log_likelihoods_dla, const double* min_z_dlas,
+                         const double* max_z_dlas, const double* offset_samples, const double* log_nhi_samples,
+                         int32_t num_quantiles, const double* quantiles, double log_nhi_threshold, double* out);
+int gpdla_dla_posteriors_device(int64_t Q, int64_t S, const double* sample_log_likelihoods_dla,
+                                const double* min_z_dlas, const double* max_z_dlas, const double* offset_samples,
+                                const double* log_nhi_samples, int32_t num_quantiles, const double* quantiles,
+                                double log_nhi_threshold, double* out, void* stream);
+/* Multi-DLA model (Ho et al. 2021).  sample_log_likelihoods_dla [Q x max_dlas x S] and base_sample_inds
+ * [Q x (max_dlas - 1) x S] (0-based; may be NULL when max_dlas == 1) in the layout of gpdla_process_qsos_multi: sample
+ * i of level j places j absorbers, at samples i and base_sample_inds[0..j-2][i].  Per level j = 1..max_dlas, with
+ * w_ji = exp(ll_ji - max_i ll_ji): ess_j, and for the absorber of rank r < j in ascending z (ties broken by log N, then
+ * slot) the posterior mean and standard deviation of its z and log N (slots are exchangeable under the resampling,
+ * ranks are not).  out [Q x (J + 4 J (J + 1) / 2)], level-major: level j holds ess_j, then (z_mean, z_sd,
+ * log_nhi_mean, log_nhi_sd) of ranks 0..j-1 (44 doubles at J = 4).  A level with no finite weight, or whose partner
+ * rows hold an index outside [0, S), is NaN, the other levels are not; max_z_dlas <= min_z_dlas makes the record NaN.
+ * Quantiles are not computed: the ranks have no quasar-independent sample order, so they would need a per-quasar
+ * sort.  Checks as above plus 1 <= max_dlas <= 4; partner indices are not rejected (they make a level NaN).  No
+ * atomics; the host entry gives the bits of the _device entry, which is asynchronous on `stream`. */
+int gpdla_multi_dla_posteriors(int64_t Q, int64_t S, int32_t max_dlas, const double* sample_log_likelihoods_dla,
+                               const int32_t* base_sample_inds, const double* min_z_dlas, const double* max_z_dlas,
+                               const double* offset_samples, const double* log_nhi_samples, double* out);
+int gpdla_multi_dla_posteriors_device(int64_t Q, int64_t S, int32_t max_dlas, const double* sample_log_likelihoods_dla,
+                                      const int32_t* base_sample_inds, const double* min_z_dlas,
+                                      const double* max_z_dlas, const double* offset_samples,
+                                      const double* log_nhi_samples, double* out, void* stream);
+
 /* ---- The fitted model of each quasar under chosen absorbers: what CDDF_analysis/qso_loader.py:1654-1774
  * (plot_this_mu) draws, on the device, with the hot path's own model evaluation ----
  * Spectra as gpdla_process_qsos takes them.  absorber_z, absorber_nhi: [Q x num_absorbers] (N in cm^-2, as voigt and
