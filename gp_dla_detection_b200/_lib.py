@@ -145,6 +145,13 @@ SYMBOLS = {
     "gpdla_multi_dla_posteriors": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64, ctypes.c_int32] + [ctypes.c_void_p] * 7),
     "gpdla_multi_dla_posteriors_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64, ctypes.c_int32]
                                           + [ctypes.c_void_p] * 8),
+    "gpdla_multi_dla_posterior_quantiles": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64, ctypes.c_int32]
+                                            + [ctypes.c_void_p] * 6
+                                            + [ctypes.c_int32, c_double_p, ctypes.c_double, ctypes.c_void_p]),
+    "gpdla_multi_dla_posterior_quantiles_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64, ctypes.c_int32]
+                                                   + [ctypes.c_void_p] * 6
+                                                   + [ctypes.c_int32, c_double_p, ctypes.c_double, ctypes.c_void_p,
+                                                      ctypes.c_void_p]),
     "gpdla_reconstruct": (ctypes.c_int,[ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64] + [ctypes.c_void_p] * 6
                           + [ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p,
                              ctypes.POINTER(GpdlaReconstruction)]),

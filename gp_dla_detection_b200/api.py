@@ -418,17 +418,8 @@ class DLAProcessor:
         ``process_multi_device(..., return_samples=True)`` returned: a float64 CUDA tensor [Q, J + 2 J (J + 1)]
         (``unpack_multi_dla_posteriors``).  Asynchronous on torch's current stream."""
         import torch
-        ll = out.get("sample_log_likelihoods_dla")
-        if ll is None:
-            raise ValueError("multi_posteriors_device needs process_multi_device(..., return_samples=True)")
+        ll, part, (Q, J, S) = self._multi_posterior_inputs(out, "multi_posteriors_device")
         dev = ll.device
-        Q, J, S = ll.shape
-        part = out.get("base_sample_inds")
-        if J > 1 and (part is None or tuple(part.shape) != (Q, J - 1, S) or part.dtype != torch.int32
-                      or not part.is_contiguous()):
-            raise ValueError("base_sample_inds must be a contiguous int32 tensor [Q, max_dlas - 1, S]")
-        if not all(out[n].is_contiguous() for n in ("sample_log_likelihoods_dla", "min_z_dlas", "max_z_dlas")):
-            raise ValueError("the arrays of process_multi_device must be contiguous")
         off, lnhi, _ = self._device_samples(dev, S)
         rec = torch.empty((Q, multi_dla_posteriors_width(J)), dtype=torch.float64, device=dev)
         ptr = lambda t: None if t is None else ctypes.c_void_p(t.data_ptr())
@@ -438,6 +429,42 @@ class DLAProcessor:
                 Q, S, J, ptr(ll), ptr(part if J > 1 else None), ptr(out["min_z_dlas"]), ptr(out["max_z_dlas"]),
                 ptr(off), ptr(lnhi), ptr(rec), stream))
         return rec
+
+    def multi_posterior_quantiles_device(self, out: Dict, quantiles=DEFAULT_QUANTILES,
+                                         log_nhi_threshold: float = _params.dla_log_nhi_min):
+        """Credible intervals of every absorber of the multi-DLA model (``multi_dla_posterior_quantiles``) of what
+        ``process_multi_device(..., return_samples=True)`` returned: a float64 CUDA tensor
+        [Q, J (J + 1) / 2 (1 + 2 P)] (``unpack_multi_dla_posterior_quantiles``).  Asynchronous on torch's current
+        stream."""
+        import torch
+        ll, part, (Q, J, S) = self._multi_posterior_inputs(out, "multi_posterior_quantiles_device")
+        dev = ll.device
+        qs = _quantiles(quantiles)
+        off, lnhi, _ = self._device_samples(dev, S)
+        rec = torch.empty((Q, multi_dla_posterior_quantiles_width(J, qs.size)), dtype=torch.float64, device=dev)
+        ptr = lambda t: None if t is None else ctypes.c_void_p(t.data_ptr())
+        with torch.cuda.device(dev):
+            stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+            _lib.check(self._lib.gpdla_multi_dla_posterior_quantiles_device(
+                Q, S, J, ptr(ll), ptr(part if J > 1 else None), ptr(out["min_z_dlas"]), ptr(out["max_z_dlas"]),
+                ptr(off), ptr(lnhi), qs.size, _dp(qs), float(log_nhi_threshold), ptr(rec), stream))
+        return rec
+
+    @staticmethod
+    def _multi_posterior_inputs(out: Dict, name: str):
+        """The checked ``process_multi_device`` arrays of the multi-DLA posterior entries: (ll, partners, (Q, J, S))."""
+        import torch
+        ll = out.get("sample_log_likelihoods_dla")
+        if ll is None:
+            raise ValueError(name + " needs process_multi_device(..., return_samples=True)")
+        Q, J, S = ll.shape
+        part = out.get("base_sample_inds")
+        if J > 1 and (part is None or tuple(part.shape) != (Q, J - 1, S) or part.dtype != torch.int32
+                      or not part.is_contiguous()):
+            raise ValueError("base_sample_inds must be a contiguous int32 tensor [Q, max_dlas - 1, S]")
+        if not all(out[n].is_contiguous() for n in ("sample_log_likelihoods_dla", "min_z_dlas", "max_z_dlas")):
+            raise ValueError("the arrays of process_multi_device must be contiguous")
+        return ll, part, (Q, J, S)
 
     # ---------------------------------------------------------------- fitted model under chosen absorbers
     def _recon_operands(self, Q: int, absorber_z, absorber_nhi, to):
@@ -1291,10 +1318,49 @@ def multi_dla_posteriors(results: Dict, samples: Dict, device: int = 0) -> np.nd
     ``process_qsos_multiple_dlas_meanflux`` result in the reference layout -- ``sample_log_likelihoods_dla`` (Q, S, J),
     ``base_sample_inds`` (Q, S, J-1), 0-based.  Per level j, ess_j and the posterior means and standard deviations of
     z and log N of the absorber of rank r < j in ascending z (``unpack_multi_dla_posteriors``).  A level with no finite
-    weight or a partner index outside [0, S) is NaN.  Quantiles are not computed: the ranks have no quasar-independent
-    sample order."""
+    weight or a partner index outside [0, S) is NaN.  The quantiles of every rank and its mass above the DLA threshold
+    are ``multi_dla_posterior_quantiles``."""
     import torch
     lib = _lib.load()
+    Q, S, J, ll, part, zlo, zhi, off, lnhi = _multi_host_inputs(results, samples)
+    out = np.empty((Q, multi_dla_posteriors_width(J)))
+    vp = lambda a: None if a is None else ctypes.c_void_p(a.ctypes.data)
+    with torch.cuda.device(device):
+        _lib.check(lib.gpdla_multi_dla_posteriors(Q, S, J, vp(ll), vp(part), vp(zlo), vp(zhi), vp(off), vp(lnhi),
+                                                  vp(out)))
+    return out
+
+
+def multi_dla_posterior_quantiles_width(max_dlas: int, num_quantiles: int) -> int:
+    """Doubles per quasar of a multi-DLA quantile record: per (level j, rank r < j), the mass above the threshold
+    and P quantiles each of z and log N."""
+    J = int(max_dlas)
+    return J * (J + 1) // 2 * (1 + 2 * int(num_quantiles))
+
+
+def multi_dla_posterior_quantiles(results: Dict, samples: Dict, quantiles=DEFAULT_QUANTILES,
+                                  log_nhi_threshold: float = _params.dla_log_nhi_min, device: int = 0) -> np.ndarray:
+    """Credible intervals of every absorber of the multi-DLA model, computed on the GPU, from one result in the
+    reference layout (as ``multi_dla_posteriors`` takes it).  Per level j and rank r < j (ascending z), the posterior
+    mass of the rank-r absorber at log N >= ``log_nhi_threshold`` (a DLA proper rather than a sub-DLA) and the lower
+    inverse-CDF ``quantiles`` of its z and log N, from fixed-point weights: a quantile's cumulative weight is within
+    S 2^-F + 1e-12 of the target, F = 63 - ceil(log2 S).  Returns [Q, J (J + 1) / 2 (1 + 2 P)]
+    (``unpack_multi_dla_posterior_quantiles``); NaN as ``multi_dla_posteriors``."""
+    import torch
+    lib = _lib.load()
+    qs = _quantiles(quantiles)
+    Q, S, J, ll, part, zlo, zhi, off, lnhi = _multi_host_inputs(results, samples)
+    out = np.empty((Q, multi_dla_posterior_quantiles_width(J, qs.size)))
+    vp = lambda a: None if a is None else ctypes.c_void_p(a.ctypes.data)
+    with torch.cuda.device(device):
+        _lib.check(lib.gpdla_multi_dla_posterior_quantiles(Q, S, J, vp(ll), vp(part), vp(zlo), vp(zhi), vp(off),
+                                                           vp(lnhi), qs.size, _dp(qs), float(log_nhi_threshold),
+                                                           vp(out)))
+    return out
+
+
+def _multi_host_inputs(results: Dict, samples: Dict):
+    """A multi-DLA result in the reference layout -> Q, S, J and the contiguous C-layout host arrays."""
     sll = np.asarray(results["sample_log_likelihoods_dla"], dtype=np.float64)
     if sll.ndim != 3:
         raise ValueError("sample_log_likelihoods_dla must be (Q, S, max_dlas)")
@@ -1310,12 +1376,7 @@ def multi_dla_posteriors(results: Dict, samples: Dict, device: int = 0) -> np.nd
     off, lnhi = (_f64(samples[k]).ravel() for k in ("offset_samples", "log_nhi_samples"))
     if zlo.size != Q or zhi.size != Q or off.size != S or lnhi.size != S:
         raise ValueError("results need Q entries per quasar and the samples S entries each (Q, S = %d, %d)" % (Q, S))
-    out = np.empty((Q, multi_dla_posteriors_width(J)))
-    vp = lambda a: None if a is None else ctypes.c_void_p(a.ctypes.data)
-    with torch.cuda.device(device):
-        _lib.check(lib.gpdla_multi_dla_posteriors(Q, S, J, vp(ll), vp(part), vp(zlo), vp(zhi), vp(off), vp(lnhi),
-                                                  vp(out)))
-    return out
+    return Q, S, J, ll, part, zlo, zhi, off, lnhi
 
 
 def unpack_dla_posteriors(rec, num_quantiles: int, num_samples: Optional[int] = None, p_dlas=None) -> Dict[str, np.ndarray]:
@@ -1357,6 +1418,28 @@ def unpack_multi_dla_posteriors(rec, max_dlas: int) -> Dict[str, np.ndarray]:
         for i, n in enumerate(MULTI_POSTERIOR_FIELDS):
             out[n][:, j - 1, :j] = block[:, :, i]
         c += 1 + 4 * j
+    return out
+
+
+def unpack_multi_dla_posterior_quantiles(rec, max_dlas: int, num_quantiles: int) -> Dict[str, np.ndarray]:
+    """A multi-DLA quantile record [Q, J (J + 1) / 2 (1 + 2 P)] -> ``mass_above_threshold`` [Q, J, J] and
+    ``z_quantiles``, ``log_nhi_quantiles`` [Q, J, J, P], indexed (level - 1, rank); entries with rank >= level are
+    NaN."""
+    v = np.asarray(rec.cpu().numpy() if hasattr(rec, "cpu") else rec, dtype=np.float64)
+    J, P = int(max_dlas), int(num_quantiles)
+    W = multi_dla_posterior_quantiles_width(J, P)
+    if v.ndim != 2 or v.shape[1] != W:
+        raise ValueError("records must be [Q, %d] for max_dlas = %d and %d quantiles" % (W, J, P))
+    Q = v.shape[0]
+    out = dict(mass_above_threshold=np.full((Q, J, J), np.nan), z_quantiles=np.full((Q, J, J, P), np.nan),
+               log_nhi_quantiles=np.full((Q, J, J, P), np.nan))
+    c = 0
+    for j in range(1, J + 1):
+        block = v[:, c:c + j * (1 + 2 * P)].reshape(Q, j, 1 + 2 * P)
+        out["mass_above_threshold"][:, j - 1, :j] = block[:, :, 0]
+        out["z_quantiles"][:, j - 1, :j] = block[:, :, 1:1 + P]
+        out["log_nhi_quantiles"][:, j - 1, :j] = block[:, :, 1 + P:]
+        c += j * (1 + 2 * P)
     return out
 
 

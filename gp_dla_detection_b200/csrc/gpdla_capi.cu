@@ -2209,6 +2209,39 @@ static int post_check(const char* fn, int64_t Q, int64_t S, int32_t max_dlas, co
   return GPDLA_OK;
 }
 
+// the two sample orders of the posterior entries, with the statistics' counting rank and one class: by offset, and by
+// log N.  Takes post_order_bytes(S) of scratch at ptr (16-byte aligned pieces; ptr moves past them), launches on st.
+struct PostOrders {
+  double *z_offset, *z_lnhi, *n_lnhi;        // offset and log N in offset order; log N in log-N order
+  int32_t *z_perm, *z_rank, *n_perm, *n_rank;
+};
+static size_t post_order_bytes(int64_t S) { return (size_t)S * (3 * 8 + 8 + 4 + 4 * 4) + 10 * 16 + 16; }
+static PostOrders post_orders(int64_t S, const double* offset_samples, const double* log_nhi_samples, char*& ptr,
+                              cudaStream_t st) {
+  auto take = [&](size_t n) { char* r = ptr; ptr += (n + 15) / 16 * 16; return r; };
+  PostOrders o;
+  o.z_offset = (double*)take(S * 8); o.z_lnhi = (double*)take(S * 8); o.n_lnhi = (double*)take(S * 8);
+  uint64_t* key = (uint64_t*)take(S * 8);
+  int32_t* cls = (int32_t*)take(S * 4);
+  o.z_perm = (int32_t*)take(S * 4); o.z_rank = (int32_t*)take(S * 4);
+  o.n_perm = (int32_t*)take(S * 4); o.n_rank = (int32_t*)take(S * 4);
+  int32_t* class_start = (int32_t*)take(2 * 4);
+  const unsigned sblocks = (unsigned)((S + STAT_THREADS - 1) / STAT_THREADS);
+  StatsClassArgs ca;
+  ca.S = S; ca.nbound = 0; ca.cls = cls; ca.key = key;
+  ca.offset = offset_samples; ca.log_nhi = log_nhi_samples;
+  stats_class_kernel<<<sblocks, STAT_THREADS, 0, st>>>(ca);
+  stats_rank_kernel<<<sblocks, STAT_THREADS, 0, st>>>(cls, key, S, o.z_perm);
+  stats_gather_kernel<<<sblocks, STAT_THREADS, 0, st>>>(o.z_perm, cls, offset_samples, log_nhi_samples, S, 0, o.z_offset,
+                                                        o.z_lnhi, o.z_rank, class_start);
+  ca.offset = log_nhi_samples;                                  // the key of the second order
+  stats_class_kernel<<<sblocks, STAT_THREADS, 0, st>>>(ca);
+  stats_rank_kernel<<<sblocks, STAT_THREADS, 0, st>>>(cls, key, S, o.n_perm);
+  stats_gather_kernel<<<sblocks, STAT_THREADS, 0, st>>>(o.n_perm, cls, log_nhi_samples, log_nhi_samples, S, 0, o.n_lnhi,
+                                                        (double*)key, o.n_rank, class_start);   // key: ranked, unused
+  return o;
+}
+
 int gpdla_dla_posteriors_device(int64_t Q, int64_t S, const double* sample_log_likelihoods_dla,
                                 const double* min_z_dlas, const double* max_z_dlas, const double* offset_samples,
                                 const double* log_nhi_samples, int32_t num_quantiles, const double* quantiles,
@@ -2230,34 +2263,16 @@ int gpdla_dla_posteriors_device(int64_t Q, int64_t S, const double* sample_log_l
   CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev), g_err);
   const bool staged = (size_t)S * 8 + 4096 <= (size_t)optin;   // 4 KB: room for the static shared memory
   const size_t smem = staged ? (size_t)S * 8 : 0;
-  const size_t bytes = (size_t)S * (3 * 8 + 8 + 4 + 4 * 4) + (size_t)C * POST_THREADS * 4 + 8 * 64;
+  const size_t bytes = post_order_bytes(S) + (size_t)C * POST_THREADS * 4 + 8 * 64;
   char* base = nullptr;
   CUDA_TRY(cudaMallocAsync(&base, bytes, st), g_err);
   char* ptr = base;
   auto take = [&](size_t n) { char* r = ptr; ptr += (n + 15) / 16 * 16; return r; };
-  double* z_offset = (double*)take(S * 8); double* z_lnhi = (double*)take(S * 8); double* n_lnhi = (double*)take(S * 8);
-  uint64_t* key = (uint64_t*)take(S * 8);
-  int32_t* cls = (int32_t*)take(S * 4); int32_t* z_perm = (int32_t*)take(S * 4); int32_t* z_rank = (int32_t*)take(S * 4);
-  int32_t* n_perm = (int32_t*)take(S * 4); int32_t* n_rank = (int32_t*)take(S * 4);
-  int32_t* class_start = (int32_t*)take(2 * 4);
+  const PostOrders o = post_orders(S, offset_samples, log_nhi_samples, ptr, st);
   int32_t* n_chunk = (int32_t*)take((size_t)C * POST_THREADS * 4);
-  a.z_offset = z_offset; a.z_lnhi = z_lnhi; a.z_perm = z_perm; a.z_rank = z_rank; a.n_lnhi = n_lnhi; a.n_chunk = n_chunk;
-  // the two sample orders, with the statistics' counting rank and one class: by offset, and by log N
-  const unsigned sblocks = (unsigned)((S + STAT_THREADS - 1) / STAT_THREADS);
-  StatsClassArgs ca;
-  ca.S = S; ca.nbound = 0; ca.cls = cls; ca.key = key;
-  ca.offset = offset_samples; ca.log_nhi = log_nhi_samples;
-  stats_class_kernel<<<sblocks, STAT_THREADS, 0, st>>>(ca);
-  stats_rank_kernel<<<sblocks, STAT_THREADS, 0, st>>>(cls, key, S, z_perm);
-  stats_gather_kernel<<<sblocks, STAT_THREADS, 0, st>>>(z_perm, cls, offset_samples, log_nhi_samples, S, 0, z_offset,
-                                                        z_lnhi, z_rank, class_start);
-  ca.offset = log_nhi_samples;                                  // the key of the second order
-  stats_class_kernel<<<sblocks, STAT_THREADS, 0, st>>>(ca);
-  stats_rank_kernel<<<sblocks, STAT_THREADS, 0, st>>>(cls, key, S, n_perm);
-  stats_gather_kernel<<<sblocks, STAT_THREADS, 0, st>>>(n_perm, cls, log_nhi_samples, log_nhi_samples, S, 0, n_lnhi,
-                                                        (double*)key, n_rank, class_start);   // key: ranked, unused
-
-  posterior_chunk_kernel<<<(unsigned)((C * POST_THREADS + 255) / 256), 256, 0, st>>>(n_perm, z_rank, S, C, n_chunk);
+  a.z_offset = o.z_offset; a.z_lnhi = o.z_lnhi; a.z_perm = o.z_perm; a.z_rank = o.z_rank; a.n_lnhi = o.n_lnhi;
+  a.n_chunk = n_chunk;
+  posterior_chunk_kernel<<<(unsigned)((C * POST_THREADS + 255) / 256), 256, 0, st>>>(o.n_perm, o.z_rank, S, C, n_chunk);
   cudaError_t e = cudaGetLastError();
   if (e == cudaSuccess && staged)
     e = cudaFuncSetAttribute(dla_posterior_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -2350,6 +2365,114 @@ int gpdla_multi_dla_posteriors(int64_t Q, int64_t S, int32_t max_dlas, const dou
   if (e == cudaSuccess) {
     rc = gpdla_multi_dla_posteriors_device(Q, S, max_dlas, d_ll, d_part, d_zlo, d_zhi, d_off, d_lnhi, d_out, nullptr);
     if (rc == GPDLA_OK && W) e = cudaMemcpy(out, d_out, W * 8, cudaMemcpyDeviceToHost);
+  }
+  if (e != cudaSuccess) { g_err = std::string(fn) + ": " + cudaGetErrorString(e); rc = GPDLA_ERR_CUDA; }
+  cudaFree(base);
+  return rc;
+}
+
+int gpdla_multi_dla_posterior_quantiles_device(int64_t Q, int64_t S, int32_t max_dlas,
+                                               const double* sample_log_likelihoods_dla,
+                                               const int32_t* base_sample_inds, const double* min_z_dlas,
+                                               const double* max_z_dlas, const double* offset_samples,
+                                               const double* log_nhi_samples, int32_t num_quantiles,
+                                               const double* quantiles, double log_nhi_threshold, double* out,
+                                               void* stream) {
+  const char* fn = "gpdla_multi_dla_posterior_quantiles_device";
+  int rc = post_check(fn, Q, S, max_dlas, sample_log_likelihoods_dla, base_sample_inds, min_z_dlas, max_z_dlas,
+                      offset_samples, log_nhi_samples, 0, nullptr, 0.0, out);
+  if (!rc)                                                      // and the quantile checks of the single-DLA entries
+    rc = post_check(fn, Q, S, 0, sample_log_likelihoods_dla, nullptr, min_z_dlas, max_z_dlas, offset_samples,
+                    log_nhi_samples, num_quantiles, quantiles, log_nhi_threshold, out);
+  if (rc) return rc;
+  if (Q == 0) return GPDLA_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  MultiQuantArgs a;
+  a.m.ll = sample_log_likelihoods_dla; a.m.partners = max_dlas > 1 ? base_sample_inds : nullptr;
+  a.m.min_z_dlas = min_z_dlas; a.m.max_z_dlas = max_z_dlas; a.m.S = S; a.m.J = max_dlas;
+  a.m.offset = offset_samples; a.m.log_nhi = log_nhi_samples; a.m.out = out;
+  a.Q = Q; a.C = posterior_chunk(S); a.P = num_quantiles;
+  for (int p = 0; p < num_quantiles; ++p) a.prob[p] = quantiles[p];
+  a.threshold = log_nhi_threshold; a.scale = std::ldexp(1.0, multi_quantile_bits(S));
+  int dev = 0, optin = 0, sms = 0, per_sm = 0;
+  CUDA_TRY(cudaGetDevice(&dev), g_err);
+  CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev), g_err);
+  // both histograms in shared memory when they fit next to the static shared memory (4 KB), S <= 14 272 on a B200;
+  // otherwise each resident CTA gets 2 S bins of global scratch and steps over the quasars
+  const size_t smem = (size_t)S * 2 * 8;
+  const bool staged = smem + 4096 <= (size_t)optin;
+  int64_t grid = Q;
+  if (!staged) {
+    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev), g_err);
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, multi_dla_posterior_quantile_kernel<false>,
+                                                           POST_THREADS, 0), g_err);
+    grid = std::min<int64_t>(Q, (int64_t)std::max(per_sm, 1) * sms);
+  }
+  const size_t hist_bytes = staged ? 0 : (size_t)grid * smem;
+  char* base = nullptr;
+  CUDA_TRY(cudaMallocAsync(&base, post_order_bytes(S) + hist_bytes + 64, st), g_err);
+  char* ptr = base;
+  auto take = [&](size_t n) { char* r = ptr; ptr += (n + 15) / 16 * 16; return r; };
+  const PostOrders o = post_orders(S, offset_samples, log_nhi_samples, ptr, st);
+  a.z_rank = o.z_rank; a.n_rank = o.n_rank; a.z_offset = o.z_offset; a.n_lnhi = o.n_lnhi;
+  a.hist = staged ? nullptr : (uint64_t*)take(hist_bytes);
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess && staged)
+    e = cudaFuncSetAttribute(multi_dla_posterior_quantile_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)smem);
+  if (e == cudaSuccess) {
+    if (staged) multi_dla_posterior_quantile_kernel<true><<<(unsigned)grid, POST_THREADS, smem, st>>>(a);
+    else multi_dla_posterior_quantile_kernel<false><<<(unsigned)grid, POST_THREADS, 0, st>>>(a);
+    e = cudaGetLastError();
+  }
+  const cudaError_t ef = cudaFreeAsync(base, st);   // freed on the error path too
+  if (e == cudaSuccess) e = ef;
+  if (e != cudaSuccess) { g_err = std::string(fn) + ": " + cudaGetErrorString(e); return GPDLA_ERR_CUDA; }
+  return GPDLA_OK;
+}
+
+int gpdla_multi_dla_posterior_quantiles(int64_t Q, int64_t S, int32_t max_dlas, const double* sample_log_likelihoods_dla,
+                                        const int32_t* base_sample_inds, const double* min_z_dlas,
+                                        const double* max_z_dlas, const double* offset_samples,
+                                        const double* log_nhi_samples, int32_t num_quantiles, const double* quantiles,
+                                        double log_nhi_threshold, double* out) {
+  const char* fn = "gpdla_multi_dla_posterior_quantiles";
+  int rc = post_check(fn, Q, S, max_dlas, sample_log_likelihoods_dla, base_sample_inds, min_z_dlas, max_z_dlas,
+                      offset_samples, log_nhi_samples, 0, nullptr, 0.0, out);
+  if (!rc)
+    rc = post_check(fn, Q, S, 0, sample_log_likelihoods_dla, nullptr, min_z_dlas, max_z_dlas, offset_samples,
+                    log_nhi_samples, num_quantiles, quantiles, log_nhi_threshold, out);
+  if (rc) return rc;
+  const size_t J = (size_t)max_dlas, P = max_dlas > 1 ? (size_t)Q * (J - 1) * S : 0;
+  const size_t QJS = (size_t)Q * J * S, W = (size_t)Q * multi_quantile_width(max_dlas, num_quantiles);
+  const size_t Sb = (size_t)S * 8;
+  const size_t bytes = QJS * 8 + P * 4 + (size_t)Q * 2 * 8 + 2 * Sb + W * 8 + 7 * 64;
+  char* base = nullptr;
+  CUDA_TRY(cudaMalloc(&base, bytes), g_err);
+  char* ptr = base;
+  auto take = [&](size_t n) { char* r = ptr; ptr += (n + 15) / 16 * 16; return r; };
+  double* d_ll = (double*)take(QJS * 8); int32_t* d_part = P ? (int32_t*)take(P * 4) : nullptr;
+  double* d_zlo = (double*)take((size_t)Q * 8); double* d_zhi = (double*)take((size_t)Q * 8);
+  double* d_off = (double*)take(Sb); double* d_lnhi = (double*)take(Sb);
+  double* d_out = (double*)take(W * 8);
+  cudaError_t e = cudaSuccess;
+  auto copy = [&](void* d, const void* h, size_t n, cudaMemcpyKind k) {
+    if (e == cudaSuccess && n) e = cudaMemcpyAsync(d, h, n, k, nullptr);
+  };
+  copy(d_ll, sample_log_likelihoods_dla, QJS * 8, cudaMemcpyHostToDevice);
+  copy(d_part, base_sample_inds, P * 4, cudaMemcpyHostToDevice);
+  copy(d_zlo, min_z_dlas, (size_t)Q * 8, cudaMemcpyHostToDevice);
+  copy(d_zhi, max_z_dlas, (size_t)Q * 8, cudaMemcpyHostToDevice);
+  copy(d_off, offset_samples, Sb, cudaMemcpyHostToDevice);
+  copy(d_lnhi, log_nhi_samples, Sb, cudaMemcpyHostToDevice);
+  rc = GPDLA_ERR_CUDA;
+  if (e == cudaSuccess) {
+    rc = gpdla_multi_dla_posterior_quantiles_device(Q, S, max_dlas, d_ll, d_part, d_zlo, d_zhi, d_off, d_lnhi,
+                                                    num_quantiles, quantiles, log_nhi_threshold, d_out, nullptr);
+    if (rc == GPDLA_OK) {
+      copy(out, d_out, W * 8, cudaMemcpyDeviceToHost);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(nullptr);
+    }
   }
   if (e != cudaSuccess) { g_err = std::string(fn) + ": " + cudaGetErrorString(e); rc = GPDLA_ERR_CUDA; }
   cudaFree(base);

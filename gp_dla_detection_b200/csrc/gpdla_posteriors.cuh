@@ -7,11 +7,13 @@
 //                                quantiles of z and log N from fixed-order block scans of the weights
 //   multi_dla_posterior_kernel   one CTA per quasar of the multi-DLA model: per level j, its effective sample size and
 //                                the moments of the absorber of rank r (ascending z, then log N, then slot), r < j
+//   multi_dla_posterior_quantile_kernel<STAGED>   per level j and rank r < j: the mass at log N >= a threshold and
+//                                lower inverse-CDF quantiles of z and log N, from fixed-point histograms over the
+//                                positions of the absorbers' source samples in the two orders
 // No per-quasar sort: z_i = min_z + (max_z - min_z) * offset_i is monotone in offset_i (see gpdla_statistics.cuh) and
 // log N_i does not depend on the quasar, so one permutation by offset and one by log N (stats_rank_kernel with one
-// class) order every row.  Quantiles of the multi-DLA order statistics are not computed: the rank-r absorber of a
-// sample has no quasar-independent order, so they would need a per-quasar sort.  No atomics: repeated calls give the
-// same bits.
+// class) order every row, and every multi-DLA absorber is one of the samples.  No float atomics: repeated calls give
+// the same bits.
 #pragma once
 #include <stdint.h>
 #include <math.h>
@@ -217,33 +219,46 @@ struct MultiPostArgs {
   double* out;                               // [Q x multi_posterior_width(J)]
 };
 
-__device__ __forceinline__ void slot_exchange(double& za, double& na, int& sa, double& zb, double& nb, int& sb) {
+// SRC: the source samples ka, kb travel with their slots
+template <bool SRC>
+__device__ __forceinline__ void slot_exchange(double& za, double& na, int& sa, int& ka, double& zb, double& nb, int& sb,
+                                              int& kb) {
   if (za > zb || (za == zb && (na > nb || (na == nb && sa > sb)))) {
     double t = za; za = zb; zb = t;
     t = na; na = nb; nb = t;
     const int u = sa; sa = sb; sb = u;
+    if (SRC) { const int v = ka; ka = kb; kb = v; }
   }
 }
 
-// the j absorbers of sample i in ascending (z, log N, slot); entries j..3 are +inf
+// the j absorbers of sample i in ascending (z, log N, slot); entries j..3 are +inf.  SRC: src[r] = the sample the
+// absorber of rank r comes from (i or a partner), 0 past j
+template <bool SRC = false>
 __device__ __forceinline__ void sorted_slots(const MultiPostArgs& a, const int32_t* part, int64_t i, int j, double zlo,
-                                             double span, double z[MSTAT_MAX_DLAS], double n[MSTAT_MAX_DLAS]) {
-  int s[MSTAT_MAX_DLAS];
+                                             double span, double z[MSTAT_MAX_DLAS], double n[MSTAT_MAX_DLAS],
+                                             int src[MSTAT_MAX_DLAS] = nullptr) {
+  int s[MSTAT_MAX_DLAS], kk[MSTAT_MAX_DLAS];
 #pragma unroll
   for (int t = 0; t < MSTAT_MAX_DLAS; ++t) {
     s[t] = t;
+    kk[t] = 0;
     z[t] = n[t] = INFINITY;
     if (t < j) {
       const int64_t k = t == 0 ? i : (int64_t)part[(t - 1) * a.S + i];   // in [0, S): checked in pass 1
+      kk[t] = (int)k;
       z[t] = __dadd_rn(zlo, __dmul_rn(span, a.offset[k]));
       n[t] = a.log_nhi[k];
     }
   }
-  slot_exchange(z[0], n[0], s[0], z[1], n[1], s[1]);
-  slot_exchange(z[2], n[2], s[2], z[3], n[3], s[3]);
-  slot_exchange(z[0], n[0], s[0], z[2], n[2], s[2]);
-  slot_exchange(z[1], n[1], s[1], z[3], n[3], s[3]);
-  slot_exchange(z[1], n[1], s[1], z[2], n[2], s[2]);
+  slot_exchange<SRC>(z[0], n[0], s[0], kk[0], z[1], n[1], s[1], kk[1]);
+  slot_exchange<SRC>(z[2], n[2], s[2], kk[2], z[3], n[3], s[3], kk[3]);
+  slot_exchange<SRC>(z[0], n[0], s[0], kk[0], z[2], n[2], s[2], kk[2]);
+  slot_exchange<SRC>(z[1], n[1], s[1], kk[1], z[3], n[3], s[3], kk[3]);
+  slot_exchange<SRC>(z[1], n[1], s[1], kk[1], z[2], n[2], s[2], kk[2]);
+  if (SRC) {
+#pragma unroll
+    for (int t = 0; t < MSTAT_MAX_DLAS; ++t) src[t] = kk[t];
+  }
 }
 
 __global__ void __launch_bounds__(STAT_THREADS) multi_dla_posterior_kernel(const __grid_constant__ MultiPostArgs a) {
@@ -319,6 +334,147 @@ __global__ void __launch_bounds__(STAT_THREADS) multi_dla_posterior_kernel(const
         if (r < j) { lev[1 + 4 * r] = zm[r]; lev[2 + 4 * r] = sdz[r]; lev[3 + 4 * r] = nm[r]; lev[4 + 4 * r] = sdn[r]; }
     }
     lev += L;
+  }
+}
+
+// ---- credible intervals of every rank of the multi-DLA model.  The rank-r absorber of sample i of level j is a sample
+// k = src_r(i) (i or a partner), so its z and log N sit at positions z_rank[k] and n_rank[k] of the two sample orders
+// whatever the quasar: its weighted CDF is a histogram over S positions, bin z_rank[k] receiving w_ji, scanned in
+// order by posterior_quantiles.  The bins hold sum floor(w 2^F) as uint64, F = 63 - ceil(log2 S): the largest weight
+// is exactly 1, so the total lies in [2^F, 2^63], and integer atomics are associative, so the bins, and the record,
+// are the same bits on every call whatever the order the threads arrive in.
+// record: level-major, then rank; per (level j, rank r < j): mass_above_threshold, z_q[P], log_nhi_q[P]
+__host__ __device__ constexpr int64_t multi_quantile_width(int J, int P) {
+  return (int64_t)J * (J + 1) / 2 * (1 + 2 * (int64_t)P);
+}
+__host__ __device__ inline int multi_quantile_bits(int64_t S) {   // F
+  int c = 0;
+  while (((int64_t)1 << c) < S) ++c;
+  return 63 - c;
+}
+constexpr int MQ_UNROLL = 4;                         // samples per thread whose gathers are in flight together
+
+struct MultiQuantArgs {
+  MultiPostArgs m;                           // m.out: [Q x multi_quantile_width(J, P)]
+  int64_t Q, C;                              // C = posterior_chunk(S)
+  const int32_t* z_rank;                     // sample -> offset position
+  const int32_t* n_rank;                     // sample -> log-N position
+  const double* z_offset;                    // [S] offset_samples in offset order
+  const double* n_lnhi;                      // [S] log_nhi_samples in log-N order
+  uint64_t* hist;                            // [gridDim.x x 2 S] per-CTA bins when not STAGED
+  int P;
+  double prob[POST_MAX_P];
+  double threshold;
+  double scale;                              // 2^F
+};
+
+// A CTA steps over the quasars (STAGED: one each).  Pass 1 is multi_level_lse; then, per level j and rank r < j, one
+// pass over the samples fills both histograms (STAGED: in shared memory, otherwise the CTA's global scratch) and the
+// float sums of the mass, and two scans read the quantiles.  Lanes of a warp that hit one bin (crowded partners) are
+// added by the group's lowest lane, so a bin takes one atomic per warp and sample step.
+template <bool STAGED>
+__global__ void __launch_bounds__(POST_THREADS) multi_dla_posterior_quantile_kernel(const __grid_constant__ MultiQuantArgs a) {
+  extern __shared__ __align__(16) uint64_t mq_smem[];
+  __shared__ double red[POST_THREADS / 32 * MSTAT_MAX_DLAS * 2];
+  __shared__ int s_bad[POST_THREADS / 32];
+  __shared__ uint64_t s_fw[POST_THREADS];
+  __shared__ int s_pos[POST_MAX_P];
+  __shared__ double s_m[MSTAT_MAX_DLAS];
+  const int tid = threadIdx.x, lane = tid & 31;
+  const int64_t S = a.m.S, C = a.C;
+  const int J = a.m.J, P = a.P, B = 1 + 2 * P;
+  const int64_t W = multi_quantile_width(J, P);
+  uint64_t* hz = STAGED ? mq_smem : a.hist + (int64_t)blockIdx.x * 2 * S;   // [S] by z position, then [S] by log N
+  uint64_t* hn = hz + S;
+  uint64_t* fw_warp = s_fw + (tid & ~31);
+  bool use[MSTAT_MAX_DLAS];
+#pragma unroll
+  for (int j = 0; j < MSTAT_MAX_DLAS; ++j) use[j] = j < J;
+  auto scan = [&](const uint64_t* h) {                         // one instantiation of posterior_quantiles' statics
+    const uint64_t* hk = h + (int64_t)tid * C;
+    posterior_quantiles(S, C, P, a.prob, [&](int i) { return (double)(STAGED ? hk[i] : __ldcg(hk + i)); }, s_pos);
+  };
+  for (int64_t q = blockIdx.x; q < a.Q; q += gridDim.x) {
+    __syncthreads();                                           // the previous quasar's reads of red and s_bad are done
+    double* rec = a.m.out + q * W;
+    const double* ll = a.m.ll + q * J * S;
+    const int32_t* part = a.m.partners ? a.m.partners + q * (J - 1) * S : nullptr;
+    const double zlo = a.m.min_z_dlas[q], zhi = a.m.max_z_dlas[q];
+    if (!(zhi > zlo)) {
+      for (int64_t c = tid; c < W; c += POST_THREADS) rec[c] = NAN;
+      continue;
+    }
+    double m[MSTAT_MAX_DLAS], s[MSTAT_MAX_DLAS];
+    const int bad = multi_level_lse(ll, part, S, use, J - 1, red, s_bad, m, s);   // pass 1, as the moments kernel
+    if (tid < MSTAT_MAX_DLAS) s_m[tid] = tid == 0 ? m[0] : tid == 1 ? m[1] : tid == 2 ? m[2] : m[3];
+    __syncthreads();                                           // indexed by level from shared memory, not the stack
+    const double span = __dsub_rn(zhi, zlo);
+    double* lev = rec;
+    for (int j = 1; j <= J; ++j) {
+      const double mj = s_m[j - 1];
+      if (!isfinite(mj) || (bad & ((1 << (j - 1)) - 1))) {   // no finite weight, or a partner row outside [0, S)
+        for (int c = tid; c < j * B; c += POST_THREADS) lev[c] = NAN;
+        lev += j * B;
+        continue;
+      }
+      const double* row = ll + (int64_t)(j - 1) * S;
+      for (int r = 0; r < j; ++r, lev += B) {
+        for (int64_t k = tid; k < 2 * S; k += POST_THREADS) hz[k] = 0;
+        __syncthreads();
+        double s0 = 0.0, st = 0.0;
+        for (int64_t i0 = 0; i0 < S; i0 += POST_THREADS * MQ_UNROLL) {   // block-uniform: whole warps step together
+          uint64_t fw[MQ_UNROLL];
+          int zb[MQ_UNROLL], nb[MQ_UNROLL];
+#pragma unroll
+          for (int u = 0; u < MQ_UNROLL; ++u) {
+            const int64_t i = i0 + u * POST_THREADS + tid;
+            fw[u] = 0; zb[u] = nb[u] = -1;
+            const double v = i < S ? row[i] : -INFINITY;
+            const double w = v > -INFINITY ? exp(v - mj) : 0.0;
+            if (w > 0.0) {
+              double z[MSTAT_MAX_DLAS], n[MSTAT_MAX_DLAS];
+              int src[MSTAT_MAX_DLAS];
+              sorted_slots<true>(a.m, part, i, j, zlo, span, z, n, src);
+              int k = 0;
+              double nr = 0.0;
+#pragma unroll
+              for (int t = 0; t < MSTAT_MAX_DLAS; ++t)
+                if (t == r) { k = src[t]; nr = n[t]; }
+              s0 += w;
+              if (nr >= a.threshold) st += w;
+              fw[u] = __double2ull_rz(w * a.scale);          // w <= 1, so at most 2^F; exact product, floor
+              if (fw[u]) { zb[u] = a.z_rank[k]; nb[u] = a.n_rank[k]; }
+            }
+          }
+#pragma unroll
+          for (int u = 0; u < MQ_UNROLL; ++u) {
+            fw_warp[lane] = fw[u];
+            const unsigned gz = __match_any_sync(0xffffffffu, zb[u]);
+            const unsigned gn = __match_any_sync(0xffffffffu, nb[u]);
+            __syncwarp();
+            if (zb[u] >= 0 && lane == __ffs(gz) - 1) {
+              uint64_t t = 0;
+              for (unsigned g = gz; g; g &= g - 1) t += fw_warp[__ffs(g) - 1];
+              atomicAdd((unsigned long long*)(hz + zb[u]), (unsigned long long)t);
+            }
+            if (nb[u] >= 0 && lane == __ffs(gn) - 1) {
+              uint64_t t = 0;
+              for (unsigned g = gn; g; g &= g - 1) t += fw_warp[__ffs(g) - 1];
+              atomicAdd((unsigned long long*)(hn + nb[u]), (unsigned long long)t);
+            }
+            __syncwarp();
+          }
+        }
+        s0 = stats_block_sum(s0, red);                         // its barriers also end the pass's atomics
+        st = stats_block_sum(st, red);
+        scan(hz);
+        if (tid < P) lev[1 + tid] = __dadd_rn(zlo, __dmul_rn(span, a.z_offset[s_pos[tid]]));   // as sorted_slots
+        __syncthreads();                                       // s_pos is reused
+        scan(hn);
+        if (tid < P) lev[1 + P + tid] = a.n_lnhi[s_pos[tid]];
+        if (tid == 0) lev[0] = st / s0;
+      }
+    }
   }
 }
 

@@ -8,7 +8,8 @@ no data-path collective, and ONE ``all_gather`` of fixed-width per-quasar record
 NVLink on GPUs, gloo in CPU tests) reassembles the catalogue.  ``sample_log_likelihoods_dla``
 (80 KB/quasar) stays sharded; ``dla_statistics_sharded`` (and ``multi_dla_statistics_sharded`` for the multi-DLA
 model) reduces it to the population-statistics sums on the rank that produced it and gathers only those (a few KB);
-``dla_posteriors_sharded`` reduces it to one fixed-width posterior summary per quasar and gathers those.
+``dla_posteriors_sharded`` (and ``multi_dla_posteriors_sharded``) reduces it to fixed-width posterior summaries per
+quasar and gathers those.
 """
 from __future__ import annotations
 
@@ -270,4 +271,61 @@ def _device_posteriors(model, samples, prior, params, quantiles, log_nhi_thresho
                                   up(pad["lengths"], np.int32), up(pad["z_qsos"], np.float64),
                                   return_sample_log_likelihoods=True)
         return proc.posteriors_device(out, quantiles, log_nhi_threshold).cpu().numpy()
+    return compute
+
+
+def multi_dla_posteriors_sharded(model: Dict, samples: Dict, spectra: Dict, prior: Dict, quantiles=None,
+                                 log_nhi_threshold: float = None, params=None, max_dlas: int = 4,
+                                 batch_quasars: int = 4096,
+                                 compute: Callable[[Dict], Tuple[np.ndarray, np.ndarray]] = None,
+                                 device=None) -> Dict:
+    """``dla_posteriors_sharded`` for the multi-DLA model: rank r runs its cost-balanced block through
+    ``process_multi_device`` (up to ``max_dlas`` DLAs, sub-DLA model, mean flux; ``samples`` holds the sub-DLA samples)
+    in batches, then ``multi_posteriors_device`` and ``multi_posterior_quantiles_device``; one ``all_gather`` carries
+    both records of every quasar side by side.  ``compute(spectra) -> (records, quantile_records)`` replaces the CUDA
+    path of one rank.  Returns ``records`` [Q x (J + 2 J (J + 1))] (``api.unpack_multi_dla_posteriors``),
+    ``quantile_records`` [Q x J (J + 1) / 2 (1 + 2 P)] (``api.unpack_multi_dla_posterior_quantiles``), both in
+    catalogue order, and ``blocks``."""
+    import torch.distributed as dist
+    from . import params as P
+    from .api import DEFAULT_QUANTILES, multi_dla_posterior_quantiles_width, multi_dla_posteriors_width
+    quantiles = np.asarray(DEFAULT_QUANTILES if quantiles is None else quantiles, dtype=np.float64).ravel()
+    log_nhi_threshold = P.dla_log_nhi_min if log_nhi_threshold is None else log_nhi_threshold
+    rank, world = dist.get_rank(), dist.get_world_size()
+    blocks = partition_by_cost(quasar_costs(spectra), world)
+    s, e = blocks[rank]
+    w0, w1 = multi_dla_posteriors_width(max_dlas), multi_dla_posterior_quantiles_width(max_dlas, quantiles.size)
+    if compute is None and e > s:
+        compute = _device_multi_posteriors(model, samples, prior, params, max_dlas, quantiles, log_nhi_threshold)
+    step = max(int(batch_quasars), 1)
+    parts = []
+    for b0 in range(s, e, step):
+        rec, qrec = compute(slice_spectra(spectra, b0, min(e, b0 + step)))
+        parts.append(np.concatenate([np.asarray(rec, dtype=np.float64).reshape(-1, w0),
+                                     np.asarray(qrec, dtype=np.float64).reshape(-1, w1)], axis=1))
+    local = np.concatenate(parts, axis=0) if parts else np.zeros((0, w0 + w1))
+    both = gather_records(local, blocks, device=device, width=w0 + w1)
+    return dict(records=both[:, :w0].copy(), quantile_records=both[:, w0:].copy(), blocks=blocks)
+
+
+def _device_multi_posteriors(model, samples, prior, params, max_dlas, quantiles, log_nhi_threshold):
+    """The CUDA path of one rank: spectra -> process_multi_device -> multi_posteriors_device and
+    multi_posterior_quantiles_device -> host records."""
+    import os
+    import torch
+    from .api import DLAProcessor, pad_spectra
+    from .params import DEFAULT
+    dev = int(os.environ.get("LOCAL_RANK", 0))
+    proc = DLAProcessor(model, samples, prior, params or DEFAULT, device=dev)
+
+    def compute(sp):
+        pad = pad_spectra(sp)
+        d = torch.device("cuda", dev)
+        up = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dtype=dt)).to(d)
+        out = proc.process_multi_device(up(pad["wavelengths"], np.float64), up(pad["flux"], np.float64),
+                                        up(pad["noise_variance"], np.float64), up(pad["pixel_mask"], np.uint8),
+                                        up(pad["lengths"], np.int32), up(pad["z_qsos"], np.float64),
+                                        max_dlas=max_dlas, return_samples=True)
+        return (proc.multi_posteriors_device(out).cpu().numpy(),
+                proc.multi_posterior_quantiles_device(out, quantiles, log_nhi_threshold).cpu().numpy())
     return compute

@@ -385,9 +385,9 @@ int gpdla_dla_posteriors_device(int64_t Q, int64_t S, const double* sample_log_l
  * ranks are not).  out [Q x (J + 4 J (J + 1) / 2)], level-major: level j holds ess_j, then (z_mean, z_sd,
  * log_nhi_mean, log_nhi_sd) of ranks 0..j-1 (44 doubles at J = 4).  A level with no finite weight, or whose partner
  * rows hold an index outside [0, S), is NaN, the other levels are not; max_z_dlas <= min_z_dlas makes the record NaN.
- * Quantiles are not computed: the ranks have no quasar-independent sample order, so they would need a per-quasar
- * sort.  Checks as above plus 1 <= max_dlas <= 4; partner indices are not rejected (they make a level NaN).  No
- * atomics; the host entry gives the bits of the _device entry, which is asynchronous on `stream`. */
+ * Quantiles of the ranks and their DLA-threshold mass are gpdla_multi_dla_posterior_quantiles' record.  Checks as
+ * above plus 1 <= max_dlas <= 4; partner indices are not rejected (they make a level NaN).  No atomics; the host entry
+ * gives the bits of the _device entry, which is asynchronous on `stream`. */
 int gpdla_multi_dla_posteriors(int64_t Q, int64_t S, int32_t max_dlas, const double* sample_log_likelihoods_dla,
                                const int32_t* base_sample_inds, const double* min_z_dlas, const double* max_z_dlas,
                                const double* offset_samples, const double* log_nhi_samples, double* out);
@@ -395,6 +395,35 @@ int gpdla_multi_dla_posteriors_device(int64_t Q, int64_t S, int32_t max_dlas, co
                                       const int32_t* base_sample_inds, const double* min_z_dlas,
                                       const double* max_z_dlas, const double* offset_samples,
                                       const double* log_nhi_samples, double* out, void* stream);
+/* Credible intervals of every absorber of the multi-DLA model.  Arguments as gpdla_multi_dla_posteriors, plus
+ * num_quantiles, quantiles and log_nhi_threshold as gpdla_dla_posteriors.  Per level j = 1..max_dlas and rank r < j
+ * (the absorber of rank r in ascending z, ties by log N, then slot, as above), under w_ji = exp(ll_ji - max_i ll_ji):
+ *   mass_above_threshold   sum of w_ji over the samples whose rank-r absorber has log N >= log_nhi_threshold, / sum w
+ *   z_quantiles[P], log_nhi_quantiles[P]   the lower inverse CDF of the rank-r absorber's z and log N: the value at the
+ *                          first position, in value order, whose cumulative fixed-point weight reaches quantiles[p]
+ *                          times the scan's total
+ * out [Q x J (J + 1) / 2 x (1 + 2 num_quantiles)], level-major, then rank (110 doubles at J = 4, P = 5).  Every
+ * absorber is one of the samples, so its value order is the samples' order by offset (z) or by log N for every quasar,
+ * and the CDF is a histogram over the S sample positions.  Its bins hold sum floor(w 2^F) exactly, as uint64, with
+ * F = 63 - ceil(log2 S) (49 at S = 10^4, 46 at S = 10^5); the largest weight is 1, so each cumulative fraction is within
+ * S 2^-F of that of the float weights (1.8e-11 at S = 10^4, 1.4e-9 at S = 10^5): a reported quantile is a value whose
+ * cumulative float weight lies within S 2^-F + 1e-12 of quantiles[p] times the total.  The mass is a float sum, as in
+ * gpdla_dla_posteriors.  NaN as gpdla_multi_dla_posteriors: a level with no finite weight or a partner row outside
+ * [0, S) is NaN, the other levels keep their bits; max_z_dlas <= min_z_dlas makes the record NaN.  Checks before any
+ * CUDA call: those of both entries above.  Integer atomics only: repeated calls give the same bits, and the host
+ * entry those of the _device entry, which is asynchronous on `stream` (quantiles stays a host array). */
+int gpdla_multi_dla_posterior_quantiles(int64_t Q, int64_t S, int32_t max_dlas, const double* sample_log_likelihoods_dla,
+                                        const int32_t* base_sample_inds, const double* min_z_dlas,
+                                        const double* max_z_dlas, const double* offset_samples,
+                                        const double* log_nhi_samples, int32_t num_quantiles, const double* quantiles,
+                                        double log_nhi_threshold, double* out);
+int gpdla_multi_dla_posterior_quantiles_device(int64_t Q, int64_t S, int32_t max_dlas,
+                                               const double* sample_log_likelihoods_dla,
+                                               const int32_t* base_sample_inds, const double* min_z_dlas,
+                                               const double* max_z_dlas, const double* offset_samples,
+                                               const double* log_nhi_samples, int32_t num_quantiles,
+                                               const double* quantiles, double log_nhi_threshold, double* out,
+                                               void* stream);
 
 /* ---- The fitted model of each quasar under chosen absorbers: what CDDF_analysis/qso_loader.py:1654-1774
  * (plot_this_mu) draws, on the device, with the hot path's own model evaluation ----
