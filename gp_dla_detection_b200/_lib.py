@@ -61,6 +61,20 @@ class GpdlaReconstruction(ctypes.Structure):
     _fields_ = [(n, ctypes.c_void_p) for n in RECONSTRUCTION_FIELDS]
 
 
+class GpdlaDrawOptions(ctypes.Structure):
+    _fields_ = [("seed", ctypes.c_uint64), ("first_quasar", ctypes.c_int64), ("model", ctypes.c_int32),
+                ("max_dlas", ctypes.c_int32), ("inject", ctypes.c_int32), ("from_prior", ctypes.c_int32),
+                ("num_absorbers", ctypes.c_int32), ("reserved", ctypes.c_int32), ("absorber_z", ctypes.c_void_p),
+                ("absorber_nhi", ctypes.c_void_p)]
+
+
+DRAW_FIELDS = ["flux", "absorption", "truth_model", "truth_inds", "truth_z", "truth_log_nhi"]
+
+
+class GpdlaDrawOutputs(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_void_p) for n in DRAW_FIELDS]
+
+
 # every symbol include/gpdla.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "gpdla_default_parameters": (None, [ctypes.POINTER(GpdlaParams)]),
@@ -158,6 +172,11 @@ SYMBOLS = {
     "gpdla_reconstruct_device": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64] + [ctypes.c_void_p] * 6
                                  + [ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p,
                                     ctypes.POINTER(GpdlaReconstruction), ctypes.c_void_p]),
+    "gpdla_draw_spectra": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64] + [ctypes.c_void_p] * 6
+                           + [ctypes.POINTER(GpdlaDrawOptions), ctypes.POINTER(GpdlaDrawOutputs)]),
+    "gpdla_draw_spectra_device": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64] + [ctypes.c_void_p] * 6
+                                  + [ctypes.POINTER(GpdlaDrawOptions), ctypes.POINTER(GpdlaDrawOutputs),
+                                     ctypes.c_void_p]),
 }
 
 _lib = None

@@ -536,6 +536,104 @@ class DLAProcessor:
             ctypes.c_void_p(stream)), self._ctx)
         return out
 
+    # ---------------------------------------------------------------- draws from the model
+    def _draw_options(self, Q, seed, first_quasar, model, max_dlas, inject, absorber_z, absorber_nhi, to):
+        """(options, from_prior, truth width, given (z, N) operands) of a draw call."""
+        if model not in ("single", "multi"):
+            raise ValueError('model must be "single" or "multi"')
+        m = int(model == "multi")
+        from_prior = absorber_z is None and absorber_nhi is None
+        if from_prior and m and not self.has_lls:
+            raise ValueError("drawing from the multi-DLA prior needs lls_nhi_samples, Z_lls and Z_dla")
+        if m and not 1 <= int(max_dlas) <= 4:
+            raise ValueError("max_dlas must lie in [1, 4]")
+        if int(first_quasar) < 0:
+            raise ValueError("first_quasar must be >= 0")
+        A, az, an = (0, None, None) if from_prior else self._recon_operands(Q, absorber_z, absorber_nhi, to)
+        o = _lib.GpdlaDrawOptions()
+        o.seed = int(seed) & (2 ** 64 - 1)
+        o.first_quasar, o.model, o.max_dlas = int(first_quasar), m, int(max_dlas) if m else 1
+        o.inject, o.from_prior, o.num_absorbers = int(bool(inject)), int(from_prior), A
+        return o, from_prior, (o.max_dlas if from_prior else 0), az, an
+
+    def draw_spectra(self, spectra: Dict, seed: int, first_quasar: int = 0, model: str = "single", max_dlas: int = 4,
+                     inject: bool = False, absorber_z=None, absorber_nhi=None) -> Dict[str, np.ndarray]:
+        """Spectra drawn from the learned model on the observing setup of ``spectra`` (wavelengths, noise variance,
+        mask, lengths, z_qso; ragged or padded, as ``process`` takes them) -- ``gpdla_draw_spectra``.
+
+        ``model``: ``"single"`` (process_qsos.m's null model and DLA prior) or ``"multi"`` (the mean-flux null model and
+        the priors of no DLA, sub-DLA and 1..``max_dlas`` DLAs).  Absorbers: drawn from the model's prior over the
+        loaded samples when ``absorber_z`` / ``absorber_nhi`` are None, else the given [Q, 0..4] arrays (NaN z = none).
+        ``inject``: add the absorbers to the flux of ``spectra`` instead of drawing the whole spectrum.  ``seed`` and
+        ``first_quasar`` (the index of the first quasar in the whole catalogue) fix every random number, so shards of a
+        catalogue drawn with their offsets give the bits of the whole.  Returns the padded spectra with the new
+        ``flux`` (ready for ``process`` / ``process_multi``), ``absorption`` [Q, L_max] and, for prior draws,
+        ``truth_model`` [Q] (-2 no separated set, -1 no draw, 0 none, 1 sub-DLA, 1 + j: j DLAs), ``truth_inds``,
+        ``truth_z``, ``truth_log_nhi`` [Q, max_dlas] (multi) or [Q, 1] (single), absorbers in ascending z."""
+        sp = pad_spectra(spectra)
+        W, F, V = _f64(sp["wavelengths"]), _f64(sp["flux"]), _f64(sp["noise_variance"])
+        Mk = np.ascontiguousarray(sp["pixel_mask"], dtype=np.uint8)
+        lengths = np.ascontiguousarray(sp["lengths"], dtype=np.int32).ravel()
+        z = _f64(sp["z_qsos"]).ravel()
+        _check_planes(W, F, V, Mk, lengths, z)
+        Q, L_max = W.shape
+        o, from_prior, TW, az, an = self._draw_options(Q, seed, first_quasar, model, max_dlas, inject, absorber_z,
+                                                       absorber_nhi, _f64)
+        vp = lambda a: None if a is None else ctypes.c_void_p(a.ctypes.data)
+        o.absorber_z, o.absorber_nhi = vp(az), vp(an)
+        out = dict(wavelengths=W, noise_variance=V, pixel_mask=Mk, lengths=lengths, z_qsos=z,
+                   flux=np.empty((Q, L_max)), absorption=np.empty((Q, L_max)))
+        if from_prior:
+            out.update(truth_model=np.empty(Q, dtype=np.int32), truth_inds=np.empty((Q, TW), dtype=np.int64),
+                       truth_z=np.empty((Q, TW)), truth_log_nhi=np.empty((Q, TW)))
+        res = _lib.GpdlaDrawOutputs()
+        for n in _lib.DRAW_FIELDS:
+            setattr(res, n, out[n].ctypes.data if n in out and out[n].size else None)
+        _lib.check(self._lib.gpdla_draw_spectra(self._ctx, Q, L_max, vp(W), vp(F) if inject else None, vp(V), vp(Mk),
+                                                vp(lengths), vp(z), ctypes.byref(o), ctypes.byref(res)), self._ctx)
+        return out
+
+    def draw_spectra_device(self, wavelengths, flux, noise_variance, pixel_mask, lengths, z_qsos, seed: int,
+                            first_quasar: int = 0, model: str = "single", max_dlas: int = 4, inject: bool = False,
+                            absorber_z=None, absorber_nhi=None, return_absorption: bool = True) -> Dict:
+        """Device-resident ``draw_spectra``: the planes as ``process_device`` takes them (``flux`` is read only when
+        injecting and may be None otherwise), absorbers as CUDA tensors or host arrays; returns CUDA tensors ``flux``,
+        ``absorption`` (with ``return_absorption``) and, for prior draws, the truth arrays.  Asynchronous on torch's
+        current stream."""
+        import torch
+        Q, L_max = wavelengths.shape
+        dev = wavelengths.device
+        assert dev.type == "cuda" and dev.index == self.device
+        planes = [(wavelengths, torch.float64), (noise_variance, torch.float64), (pixel_mask, torch.uint8),
+                  (lengths, torch.int32), (z_qsos, torch.float64)]
+        if inject:
+            if flux is None:
+                raise ValueError("injecting needs the flux to inject into")
+            planes.append((flux, torch.float64))
+        for t, dt in planes:
+            assert t.is_cuda and t.dtype == dt and t.is_contiguous()
+        to = lambda a: torch.as_tensor(a, dtype=torch.float64, device=dev).contiguous()
+        o, from_prior, TW, az, an = self._draw_options(Q, seed, first_quasar, model, max_dlas, inject, absorber_z,
+                                                       absorber_nhi, to)
+        ptr = lambda t: None if t is None else ctypes.c_void_p(t.data_ptr())
+        o.absorber_z, o.absorber_nhi = ptr(az), ptr(an)
+        f64 = dict(dtype=torch.float64, device=dev)
+        out = dict(flux=torch.empty((Q, L_max), **f64))
+        if return_absorption:
+            out["absorption"] = torch.empty((Q, L_max), **f64)
+        if from_prior:
+            out.update(truth_model=torch.empty(Q, dtype=torch.int32, device=dev),
+                       truth_inds=torch.empty((Q, TW), dtype=torch.int64, device=dev),
+                       truth_z=torch.empty((Q, TW), **f64), truth_log_nhi=torch.empty((Q, TW), **f64))
+        res = _lib.GpdlaDrawOutputs()
+        for n in _lib.DRAW_FIELDS:
+            setattr(res, n, out[n].data_ptr() if n in out and out[n].numel() else None)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(self._lib.gpdla_draw_spectra_device(
+            self._ctx, Q, L_max, ptr(wavelengths), ptr(flux if inject else None), ptr(noise_variance), ptr(pixel_mask),
+            ptr(lengths), ptr(z_qsos), ctypes.byref(o), ctypes.byref(res), ctypes.c_void_p(stream)), self._ctx)
+        return out
+
 
 def process_qsos(model: Dict, samples: Dict, spectra: Dict, prior: Dict, params: Parameters = DEFAULT,
                  device: int = 0, return_sample_log_likelihoods: bool = True, gram_digits: int = 0,
@@ -648,6 +746,29 @@ def map_absorbers(results: Dict, samples: Dict, model="map"):
         if np.any(sel):
             zj, nj = level(j)
             zz[sel, :j], n[sel, :j] = zj[sel], nj[sel]
+    return zz, n
+
+
+def truth_absorbers(draw: Dict, samples: Dict):
+    """The drawn absorbers of a prior draw (``draw_spectra`` or ``draw_spectra_device`` output) as
+    ``DLAProcessor.reconstruct`` takes them: ``(absorber_z, absorber_nhi)``, [Q, width] NumPy arrays with z =
+    ``truth_z`` and N = ``nhi_samples[truth_inds]`` for DLAs, ``lls_nhi_samples[truth_inds]`` for a sub-DLA; NaN z for
+    an empty slot."""
+    if "truth_inds" not in draw:
+        raise ValueError("truth_absorbers needs a draw from the prior (no absorbers were given)")
+    ind = _host(draw["truth_inds"]).astype(np.int64)
+    code = _host(draw["truth_model"]).astype(np.int64)
+    zz = _host(draw["truth_z"]).astype(np.float64).copy()
+    nhi = _f64(samples["nhi_samples"]).ravel()
+    ok = ind >= 0
+    safe = np.where(ok, ind, 0)
+    n = np.where(ok, nhi[safe], np.nan)
+    sub = ok & (code[:, None] == 1)
+    if np.any(sub):
+        if "lls_nhi_samples" not in samples:
+            raise ValueError("a sub-DLA truth needs samples[\"lls_nhi_samples\"]")
+        n = np.where(sub, _f64(samples["lls_nhi_samples"]).ravel()[safe], n)
+    zz[~ok] = np.nan
     return zz, n
 
 

@@ -24,6 +24,7 @@
 #include "gpdla_statistics.cuh"
 #include "gpdla_posteriors.cuh"
 #include "gpdla_reconstruct.cuh"
+#include "gpdla_draw.cuh"
 #include "gpdla_rest_table.h"
 
 using namespace gpdla;
@@ -2479,6 +2480,33 @@ int gpdla_multi_dla_posterior_quantiles(int64_t Q, int64_t S, int32_t max_dlas, 
   return rc;
 }
 
+// ---- host entries over the context's staging buffer ----
+// One array of a host entry: copied in from host_in, or out to host_out, through a slice of c->d_stage set in *dev.
+struct StageItem { void** dev; const void* host_in; void* host_out; size_t bytes; };
+// grow the staging buffer to hold every item, point each at its slice and enqueue the copies in
+static int stage_in(gpdla_ctx* c, std::vector<StageItem>& items, cudaStream_t st) {
+  size_t bytes = 256;
+  for (auto& it : items) bytes += (it.bytes + 255) / 256 * 256;
+  if (c->st_bytes < bytes) {
+    cudaFree(c->d_stage); c->d_stage = nullptr; c->st_bytes = 0;
+    CUDA_TRY(cudaMalloc(&c->d_stage, bytes), c->err);
+    c->st_bytes = bytes;
+  }
+  char* p = (char*)c->d_stage;
+  for (auto& it : items) {
+    *it.dev = p; p += (it.bytes + 255) / 256 * 256;
+    if (it.host_in) CUDA_TRY(cudaMemcpyAsync(*it.dev, it.host_in, it.bytes, cudaMemcpyHostToDevice, st), c->err);
+  }
+  return GPDLA_OK;
+}
+// enqueue the copies out and wait for them
+static int stage_out(gpdla_ctx* c, const std::vector<StageItem>& items, cudaStream_t st) {
+  for (auto& it : items)
+    if (it.host_out) CUDA_TRY(cudaMemcpyAsync(it.host_out, *it.dev, it.bytes, cudaMemcpyDeviceToHost, st), c->err);
+  CUDA_TRY(cudaStreamSynchronize(st), c->err);
+  return GPDLA_OK;
+}
+
 // ---- the fitted model of each quasar under chosen absorbers (CDDF_analysis/qso_loader.py:1654-1774) ----
 
 // the checks both reconstruction entries make before any CUDA call
@@ -2577,13 +2605,12 @@ int gpdla_reconstruct(gpdla_ctx* c, int64_t Q, int64_t L_max, const double* wave
   }
   DeviceGuard guard(c->device);
   const size_t QL = (size_t)Q * L_max;
-  struct Item { void** dev; const void* host_in; void* host_out; size_t bytes; };
   double *d_w, *d_f, *d_v, *d_z, *d_az = nullptr, *d_an = nullptr;
   uint8_t* d_m;
   int32_t* d_len;
   gpdla_reconstruction dr;
   memset(&dr, 0, sizeof dr);
-  std::vector<Item> items = {
+  std::vector<StageItem> items = {
       {(void**)&d_w, wavelengths, nullptr, QL * 8}, {(void**)&d_f, flux, nullptr, QL * 8},
       {(void**)&d_v, noise_variance, nullptr, QL * 8}, {(void**)&d_z, z_qsos, nullptr, (size_t)Q * 8},
       {(void**)&d_len, lengths, nullptr, (size_t)Q * 4}, {(void**)&d_m, pixel_mask, nullptr, QL}};
@@ -2602,25 +2629,159 @@ int gpdla_reconstruct(gpdla_ctx* c, int64_t Q, int64_t L_max, const double* wave
   want((void**)&dr.chi2, out->chi2, (size_t)Q * 8);
   want((void**)&dr.log_likelihood, out->log_likelihood, (size_t)Q * 8);
   want((void**)&dr.num_pixels, out->num_pixels, (size_t)Q * 4);
-  size_t bytes = 256;
-  for (auto& it : items) bytes += (it.bytes + 255) / 256 * 256;
-  if (c->st_bytes < bytes) {
-    cudaFree(c->d_stage); c->d_stage = nullptr; c->st_bytes = 0;
-    CUDA_TRY(cudaMalloc(&c->d_stage, bytes), c->err);
-    c->st_bytes = bytes;
-  }
-  char* p = (char*)c->d_stage;
   cudaStream_t st = c->stream;
-  for (auto& it : items) {
-    *it.dev = p; p += (it.bytes + 255) / 256 * 256;
-    if (it.host_in) CUDA_TRY(cudaMemcpyAsync(*it.dev, it.host_in, it.bytes, cudaMemcpyHostToDevice, st), c->err);
-  }
+  if ((rc = stage_in(c, items, st))) return rc;
   rc = gpdla_reconstruct_device(c, Q, L_max, d_w, d_f, d_v, d_m, d_len, d_z, meanflux, num_absorbers, d_az, d_an, &dr, st);
   if (rc) return rc;
-  for (auto& it : items)
-    if (it.host_out) CUDA_TRY(cudaMemcpyAsync(it.host_out, *it.dev, it.bytes, cudaMemcpyDeviceToHost, st), c->err);
-  CUDA_TRY(cudaStreamSynchronize(st), c->err);
+  return stage_out(c, items, st);
+}
+
+
+// ---- draws from the learned model: prior-predictive spectra and injected absorbers, with their truth ----
+
+// the checks both draw entries make before any CUDA call
+static int draw_check(gpdla_ctx* c, const char* fn, int64_t Q, int64_t L_max, const double* wavelengths,
+                      const double* flux_in, const double* noise_variance, const uint8_t* pixel_mask,
+                      const int32_t* lengths, const double* z_qsos, const gpdla_draw_options* o,
+                      const gpdla_draw_outputs* out) {
+  if (!o || !out) {
+    c->err = std::string(fn) + ": options and outputs are required";
+    return GPDLA_ERR_INVALID;
+  }
+  // the spectra, model and absorber checks of gpdla_reconstruct; the flux is read only when injecting
+  gpdla_reconstruction none;
+  memset(&none, 0, sizeof none);
+  int rc = recon_check(c, fn, Q, L_max, wavelengths, o->inject ? flux_in : wavelengths, noise_variance, pixel_mask,
+                       lengths, z_qsos, o->model, o->num_absorbers, o->absorber_z, o->absorber_nhi, &none);
+  if (rc == GPDLA_ERR_INVALID) return rc;
+  const bool truth = out->truth_model && out->truth_inds && out->truth_z && out->truth_log_nhi;
+  if (!(o->inject == 0 || o->inject == 1) || !(o->from_prior == 0 || o->from_prior == 1) || o->first_quasar < 0 ||
+      (o->model == 1 && !(o->max_dlas >= 1 && o->max_dlas <= DRAW_MAX_ABSORBERS)) ||
+      (Q > 0 && !out->flux) || (Q > 0 && o->inject && !flux_in) || (o->from_prior && o->num_absorbers != 0) ||
+      (Q > 0 && o->from_prior && !truth)) {
+    c->err = std::string(fn) + ": invalid arguments (flux output required; flux_in when injecting; no given absorbers and "
+             "all four truth outputs with from_prior; first_quasar >= 0; model 1: 1 <= max_dlas <= 4)";
+    return GPDLA_ERR_INVALID;
+  }
+  if (rc) return rc;
+  if (o->from_prior && (!c->d_offset || c->n_prior < 0 || (o->model == 1 && (!c->d_lls_nhi || c->lls_S != c->S)))) {
+    c->err = std::string(fn) + ": drawing from the prior needs set_samples and set_prior (model 1: set_lls_samples)";
+    return GPDLA_ERR_STATE;
+  }
   return GPDLA_OK;
+}
+
+extern "C++" {
+template <int K>
+static int launch_draw(gpdla_ctx* c, const DrawArgs& da, int64_t Q, cudaStream_t st) {
+  const size_t smem = draw_smem_doubles<K>(da.L_max) * sizeof(double);
+  int optin = 0;
+  cudaFuncAttributes fa;
+  CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device), c->err);
+  CUDA_TRY(cudaFuncGetAttributes(&fa, draw_spectra_kernel<K>), c->err);
+  if (smem + fa.sharedSizeBytes > (size_t)optin) {
+    c->err = "gpdla_draw_spectra: L_max=" + std::to_string(da.L_max) + " does not fit one CTA's shared memory";
+    return GPDLA_ERR_UNSUPPORTED;
+  }
+  int rc = configure_smem(c->device, draw_spectra_kernel<K>, smem, c->err);
+  if (rc) return rc;
+  draw_spectra_kernel<K><<<(unsigned)Q, NTHREADS, smem, st>>>(da);
+  return GPDLA_OK;
+}
+}  // extern "C++"
+
+int gpdla_draw_spectra_device(gpdla_ctx* c, int64_t Q, int64_t L_max, const double* wavelengths, const double* flux_in,
+                              const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                              const double* z_qsos, const gpdla_draw_options* o, const gpdla_draw_outputs* out,
+                              void* stream) {
+  if (!c) return GPDLA_ERR_INVALID;
+  int rc = draw_check(c, "gpdla_draw_spectra_device", Q, L_max, wavelengths, flux_in, noise_variance, pixel_mask,
+                      lengths, z_qsos, o, out);
+  if (rc || Q == 0) return rc;
+  DeviceGuard guard(c->device);
+  DrawArgs da;
+  memset(&da, 0, sizeof da);
+  da.wavelengths = wavelengths; da.flux_in = flux_in; da.noise_variance = noise_variance; da.pixel_mask = pixel_mask;
+  da.lengths = lengths; da.z_qsos = z_qsos; da.L_max = L_max;
+  da.rest_wavelengths = c->d_rest; da.mu = c->d_mu; da.M = c->d_M; da.log_omega = c->d_log_omega; da.n_rest = c->n_rest;
+  da.c_0 = c->c_0; da.tau_0 = c->tau_0; da.beta = c->beta;
+  da.min_lambda = c->params.min_lambda; da.max_lambda = c->params.max_lambda;
+  da.lya_wavelength = c->params.lya_wavelength; da.lyman_limit = c->params.lyman_limit;
+  da.prior_z_qso_increase = c->params.prior_z_qso_increase; da.min_z_cut = c->params.min_z_cut;
+  da.max_z_cut = c->params.max_z_cut; da.pixel_spacing = c->params.pixel_spacing; da.num_lines = c->params.num_lines;
+  da.model = o->model; da.max_dlas = o->model == 1 ? o->max_dlas : 1;
+  da.inject = o->inject; da.from_prior = o->from_prior; da.seed = o->seed; da.first_quasar = o->first_quasar;
+  if (o->from_prior) {
+    da.prior_z_qsos = c->d_prior_z; da.prior_dla_ind = c->d_prior_dla; da.n_prior = c->n_prior;
+    da.offset_samples = c->d_offset; da.log_nhi_samples = c->d_log_nhi; da.nhi_samples = c->d_nhi;
+    da.lls_nhi_samples = c->d_lls_nhi; da.S = c->S; da.Z_lls = c->Z_lls; da.Z_dla = c->Z_dla;
+    da.min_z_separation = (3000.0 * 1000.0) / 299792458.0;   // kms_to_z(3000), ...meanflux.m:33
+  }
+  da.num_absorbers = o->num_absorbers; da.absorber_z = o->absorber_z; da.absorber_nhi = o->absorber_nhi;
+  da.flux = out->flux; da.absorption = out->absorption;
+  da.truth_model = out->truth_model; da.truth_inds = out->truth_inds; da.truth_z = out->truth_z;
+  da.truth_log_nhi = out->truth_log_nhi; da.truth_width = da.max_dlas;
+  switch (c->k) {
+    case 10: rc = launch_draw<10>(c, da, Q, (cudaStream_t)stream); break;
+    case 20: rc = launch_draw<20>(c, da, Q, (cudaStream_t)stream); break;
+    case 40: rc = launch_draw<40>(c, da, Q, (cudaStream_t)stream); break;
+    default: c->err = "gpdla_draw_spectra: rank not compiled in"; rc = GPDLA_ERR_UNSUPPORTED;
+  }
+  if (rc) return rc;
+  c->launches++;
+  CUDA_TRY(cudaGetLastError(), c->err);
+  return GPDLA_OK;
+}
+
+int gpdla_draw_spectra(gpdla_ctx* c, int64_t Q, int64_t L_max, const double* wavelengths, const double* flux_in,
+                       const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                       const double* z_qsos, const gpdla_draw_options* o, const gpdla_draw_outputs* out) {
+  if (!c) return GPDLA_ERR_INVALID;
+  int rc = draw_check(c, "gpdla_draw_spectra", Q, L_max, wavelengths, flux_in, noise_variance, pixel_mask, lengths,
+                      z_qsos, o, out);
+  if (rc || Q == 0) return rc;
+  const size_t QA = (size_t)Q * o->num_absorbers;
+  for (size_t i = 0; i < QA; ++i) {
+    const double z = o->absorber_z[i], N = o->absorber_nhi[i];
+    if (std::isnan(z)) continue;
+    if (!(std::isfinite(z) && z > -1.0 && std::isfinite(N) && N >= 0.0)) {
+      c->err = "gpdla_draw_spectra: absorber " + std::to_string(i) + " needs z > -1 and a finite N >= 0 (NaN z = none)";
+      return GPDLA_ERR_INVALID;
+    }
+  }
+  DeviceGuard guard(c->device);
+  const size_t QL = (size_t)Q * L_max;
+  const size_t TW = o->from_prior ? (size_t)(o->model == 1 ? o->max_dlas : 1) : 0;
+  double *d_w, *d_f = nullptr, *d_v, *d_z, *d_az = nullptr, *d_an = nullptr;
+  uint8_t* d_m;
+  int32_t* d_len;
+  gpdla_draw_outputs dout;
+  memset(&dout, 0, sizeof dout);
+  std::vector<StageItem> items = {
+      {(void**)&d_w, wavelengths, nullptr, QL * 8}, {(void**)&d_v, noise_variance, nullptr, QL * 8},
+      {(void**)&d_z, z_qsos, nullptr, (size_t)Q * 8}, {(void**)&d_len, lengths, nullptr, (size_t)Q * 4},
+      {(void**)&d_m, pixel_mask, nullptr, QL}};
+  if (o->inject) items.push_back({(void**)&d_f, flux_in, nullptr, QL * 8});
+  if (QA) {
+    items.push_back({(void**)&d_az, o->absorber_z, nullptr, QA * 8});
+    items.push_back({(void**)&d_an, o->absorber_nhi, nullptr, QA * 8});
+  }
+  auto want = [&](void** dev, void* host, size_t bytes) { if (host) items.push_back({dev, nullptr, host, bytes}); };
+  want((void**)&dout.flux, out->flux, QL * 8);
+  want((void**)&dout.absorption, out->absorption, QL * 8);
+  if (TW) {
+    want((void**)&dout.truth_model, out->truth_model, (size_t)Q * 4);
+    want((void**)&dout.truth_inds, out->truth_inds, (size_t)Q * TW * 8);
+    want((void**)&dout.truth_z, out->truth_z, (size_t)Q * TW * 8);
+    want((void**)&dout.truth_log_nhi, out->truth_log_nhi, (size_t)Q * TW * 8);
+  }
+  cudaStream_t st = c->stream;
+  if ((rc = stage_in(c, items, st))) return rc;
+  gpdla_draw_options dopt = *o;
+  dopt.absorber_z = d_az; dopt.absorber_nhi = d_an;
+  rc = gpdla_draw_spectra_device(c, Q, L_max, d_w, d_f, d_v, d_m, d_len, d_z, &dopt, &dout, st);
+  if (rc) return rc;
+  return stage_out(c, items, st);
 }
 
 }  // extern "C"

@@ -237,15 +237,21 @@ __device__ __forceinline__ double padded_wavelength(int p, int n_u, const double
   return exp10(ex);
 }
 
-__global__ void __launch_bounds__(NTHREADS) prepare_quasars_kernel(PrepArgs a) {
-  const int q = blockIdx.x, tid = threadIdx.x;
-  const int64_t L = min(max((int64_t)a.lengths[q], (int64_t)0), a.L_max);   // a length beyond the padded row is clamped
-  const double z_qso = a.z_qsos[q];
-  const double* wl = a.wavelengths + q * a.L_max;
-  const double* fl = a.flux + q * a.L_max;
-  const double* nv = a.noise_variance + q * a.L_max;
-  const uint8_t* pm = a.pixel_mask + q * a.L_max;
-
+// One quasar's window / used-pixel scan (process_qsos.m:102-110) and the prior-catalogue counts behind its DLA prior
+// (process_qsos.m:122-125), reduced over the CTA.  Every field is a min, a max or an integer count, so the result does
+// not depend on the order of the reduction.  All NTHREADS threads call it; every thread gets the result.
+// prepare_quasars_kernel and draw_spectra_kernel both scan through this function.
+struct WindowScan {
+  int first, n_u, n;              // first window pixel, window pixels (masked ones included), used pixels
+  double minw, maxw;              // extreme used wavelengths: the z range (set_parameters.m:65-73)
+  double minu, maxu;              // extreme window wavelengths: the padded grid (process_qsos.m:168-176)
+  int prior_num_quasars, prior_num_dlas;   // prior quasars below z_qso + prior_z_qso_increase, and their DLAs
+};
+__device__ __forceinline__ WindowScan scan_window(const double* wl, const uint8_t* pm, int64_t L, double z_qso,
+                                                  double min_lambda, double max_lambda, const double* prior_z_qsos,
+                                                  const uint8_t* prior_dla_ind, int64_t n_prior,
+                                                  double prior_z_qso_increase) {
+  const int tid = threadIdx.x;
   __shared__ int s_first, s_last, s_n, s_nq, s_nd;
   __shared__ double s_minw, s_maxw, s_minu, s_maxu;
   __shared__ double red_min[NTHREADS / 32], red_max[NTHREADS / 32];
@@ -258,7 +264,7 @@ __global__ void __launch_bounds__(NTHREADS) prepare_quasars_kernel(PrepArgs a) {
   for (int64_t i = tid; i < L; i += NTHREADS) {
     double w = wl[i];
     double rest = w / (1.0 + z_qso);
-    bool inwin = (rest >= a.min_lambda) && (rest <= a.max_lambda);
+    bool inwin = (rest >= min_lambda) && (rest <= max_lambda);
     if (inwin) {
       first = min(first, (int)i); last = max(last, (int)i);
       minu = fmin(minu, w); maxu = fmax(maxu, w);
@@ -267,10 +273,10 @@ __global__ void __launch_bounds__(NTHREADS) prepare_quasars_kernel(PrepArgs a) {
   }
   // DLA existence prior counts (process_qsos.m:122-125)
   int nq = 0, nd = 0;
-  const double zlim = z_qso + a.prior_z_qso_increase;
-  for (int64_t i = tid; i < a.n_prior; i += NTHREADS) {
-    bool less = a.prior_z_qsos[i] < zlim;
-    nq += less; nd += (less && a.prior_dla_ind[i]);
+  const double zlim = z_qso + prior_z_qso_increase;
+  for (int64_t i = tid; i < n_prior; i += NTHREADS) {
+    bool less = prior_z_qsos[i] < zlim;
+    nq += less; nd += (less && prior_dla_ind[i]);
   }
   atomicMin(&s_first, first); atomicMax(&s_last, last);
   atomicAdd(&s_n, n); atomicAdd(&s_nq, nq); atomicAdd(&s_nd, nd);
@@ -291,36 +297,79 @@ __global__ void __launch_bounds__(NTHREADS) prepare_quasars_kernel(PrepArgs a) {
   block_minmax(minw, maxw, s_minw, s_maxw);
   block_minmax(minu, maxu, s_minu, s_maxu);
   __syncthreads();
+  WindowScan ws;
+  ws.first = s_first; ws.n_u = s_last >= s_first ? s_last - s_first + 1 : 0; ws.n = s_n;
+  ws.minw = s_minw; ws.maxw = s_maxw; ws.minu = s_minu; ws.maxu = s_maxu;
+  ws.prior_num_quasars = s_nq; ws.prior_num_dlas = s_nd;
+  __syncthreads();   // the shared results are read before a later call may reset them
+  return ws;
+}
 
-  const int n_u = s_last >= s_first ? s_last - s_first + 1 : 0;
-  const int n_used = s_n;
+// The DLA redshift range of one quasar from its extreme used wavelengths (set_parameters.m:65-73)
+__device__ __forceinline__ void dla_z_range(double minw, double maxw, double z_qso, double lya_wavelength,
+                                            double lyman_limit, double min_z_cut, double max_z_cut, double& min_z,
+                                            double& max_z) {
+  max_z = (maxw / lya_wavelength - 1.0) - max_z_cut;
+  min_z = fmax(minw / lya_wavelength - 1.0, lyman_limit * (1.0 + z_qso) / lya_wavelength - 1.0 + min_z_cut);
+}
+
+// The single-DLA model priors from the prior-catalogue counts (process_qsos.m:128-131)
+__device__ __forceinline__ void single_dla_log_priors(int nq, int nd, double& log_prior_no_dla, double& log_prior_dla) {
+  log_prior_dla = log((double)nd) - log((double)nq);
+  log_prior_no_dla = log((double)(nq - nd)) - log((double)nq);
+}
+
+// The multi-DLA model priors (...meanflux.m:190-216): no DLA, sub-DLA and j = 1..max_dlas DLAs (log_prior_dla[j - 1])
+__device__ __forceinline__ void multi_dla_log_priors(int prior_num_quasars, int prior_num_dlas, double Z_lls,
+                                                     double Z_dla, int max_dlas, double& log_prior_no_dla,
+                                                     double& log_prior_lls, double* log_prior_dla) {
+  const double nq = (double)prior_num_quasars, nd = (double)prior_num_dlas;
+  const double p1 = nd / nq;
+  for (int j = 0; j < max_dlas; ++j) {
+    const double pj = pow(p1, (double)(j + 1));                                    // :194
+    log_prior_dla[j] = log(j < max_dlas - 1 ? pj - pow(p1, (double)(j + 2)) : pj); // :197-199, :204
+  }
+  log_prior_lls = log(nd) - log(nq) + log(Z_lls) - log(Z_dla);                     // :208-210
+  log_prior_no_dla = log(nq - nd - Z_lls * nd / Z_dla) - log(nq);                  // :214-216
+}
+
+__global__ void __launch_bounds__(NTHREADS) prepare_quasars_kernel(PrepArgs a) {
+  const int q = blockIdx.x, tid = threadIdx.x;
+  const int64_t L = min(max((int64_t)a.lengths[q], (int64_t)0), a.L_max);   // a length beyond the padded row is clamped
+  const double z_qso = a.z_qsos[q];
+  const double* wl = a.wavelengths + q * a.L_max;
+  const double* fl = a.flux + q * a.L_max;
+  const double* nv = a.noise_variance + q * a.L_max;
+  const uint8_t* pm = a.pixel_mask + q * a.L_max;
+
+  const WindowScan ws = scan_window(wl, pm, L, z_qso, a.min_lambda, a.max_lambda, a.prior_z_qsos, a.prior_dla_ind,
+                                    a.n_prior, a.prior_z_qso_increase);
+  const int n_u = ws.n_u;
+  const int n_used = ws.n;
   const int NPIX = a.NPIX;
   double* lam = a.lam_pad + (int64_t)q * (NPIX + 8);
   double* lamh = a.lamh + (int64_t)q * (NPIX + 8);
   double* pix = a.pix + (int64_t)q * NPIX * 4;
   double* Mq = a.Mq + (int64_t)q * NPIX * a.k;
   // first padded wavelength (same expression as p = 0 below)
-  const double lam_ref = n_used > 0 ? exp10(log10(s_minu) - 3 * a.pixel_spacing) : 1.0;
+  const double lam_ref = n_used > 0 ? exp10(log10(ws.minu) - 3 * a.pixel_spacing) : 1.0;
 
   if (tid == 0) {
     QuasarMeta m;
     m.lam_ref = lam_ref;
-    m.n_u = n_u; m.n = n_used; m.nchunks = (n_u + KC - 1) / KC; m.first = s_first;
-    // set_parameters.m:65-73
-    m.max_z_dla = (s_maxw / a.lya_wavelength - 1.0) - a.max_z_cut;
-    m.min_z_dla = fmax(s_minw / a.lya_wavelength - 1.0,
-                       a.lyman_limit * (1.0 + z_qso) / a.lya_wavelength - 1.0 + a.min_z_cut);
-    // process_qsos.m:128-131
-    m.log_prior_dla = log((double)s_nd) - log((double)s_nq);
-    m.prior_num_quasars = s_nq; m.prior_num_dlas = s_nd;
-    m.log_prior_no_dla = log((double)(s_nq - s_nd)) - log((double)s_nq);
+    m.n_u = n_u; m.n = n_used; m.nchunks = (n_u + KC - 1) / KC; m.first = ws.first;
+    dla_z_range(ws.minw, ws.maxw, z_qso, a.lya_wavelength, a.lyman_limit, a.min_z_cut, a.max_z_cut, m.min_z_dla,
+                m.max_z_dla);
+    single_dla_log_priors(ws.prior_num_quasars, ws.prior_num_dlas, m.log_prior_no_dla, m.log_prior_dla);
+    m.prior_num_quasars = ws.prior_num_quasars; m.prior_num_dlas = ws.prior_num_dlas;
     if (n_used == 0) { m.nchunks = 0; m.min_z_dla = NAN; m.max_z_dla = NAN; }
     a.meta[q] = m;
   }
   if (n_used == 0) return;
 
   // padded wavelength grid (process_qsos.m:168-176); pixels past the end continue the log grid
-  const double lo = log10(s_minu), hi = log10(s_maxu);
+  const double lo = log10(ws.minu), hi = log10(ws.maxu);
+  const int s_first = ws.first;
   for (int p = tid; p < NPIX + 8; p += NTHREADS) {
     const double v = padded_wavelength(p, n_u, wl + s_first, lo, hi, a.pixel_spacing);
     lam[p] = v;
@@ -1446,20 +1495,16 @@ __global__ void multi_posterior_kernel(MultiPosteriorArgs a) {
   if (q >= a.Q) return;
   const QuasarMeta meta = a.meta[q];
   const int MD = a.max_dlas;
-  const double nq = (double)meta.prior_num_quasars, nd = (double)meta.prior_num_dlas;
-  double pd[8];
-  const double p1 = nd / nq;
-  for (int j = 0; j < MD; ++j) pd[j] = pow(p1, (double)(j + 1));                   // :194
-  for (int j = 0; j < MD - 1; ++j) pd[j] = pd[j] - pd[j + 1];                      // :197-199
-  const double lp_lls_prior = log(nd) - log(nq) + log(a.Z_lls) - log(a.Z_dla);    // :208-210
-  const double lp_no_prior = log(nq - nd - a.Z_lls * nd / a.Z_dla) - log(nq);     // :214-216
+  double lp_no_prior, lp_lls_prior, lp_dla_prior[8];
+  multi_dla_log_priors(meta.prior_num_quasars, meta.prior_num_dlas, a.Z_lls, a.Z_dla, MD, lp_no_prior, lp_lls_prior,
+                       lp_dla_prior);
   a.min_z_dlas[q] = meta.min_z_dla; a.max_z_dlas[q] = meta.max_z_dla;
   a.log_priors_no_dla[q] = lp_no_prior; a.log_priors_lls[q] = lp_lls_prior;
   double lp[10];
   lp[0] = lp_no_prior + a.log_likelihoods_no_dla[q];                               // :300-301
   lp[1] = lp_lls_prior + a.log_likelihoods_lls[q];                                 // :428-430
   for (int j = 0; j < MD; ++j) {
-    const double pr = log(pd[j]);                                                  // :204
+    const double pr = lp_dla_prior[j];
     a.log_priors_dla[q * MD + j] = pr;
     lp[2 + j] = pr + a.log_likelihoods_dla[q * MD + j];                            // :411-413
     a.log_posteriors_dla[q * MD + j] = lp[2 + j];

@@ -46,6 +46,46 @@ struct ReconArgs {
   int32_t* num_pixels;
 };
 
+// The absorption of one quasar's window on the padded grid (process_qsos.m:168-188; ...meanflux.m:342-351): each
+// absorber's profile as voigt_batch_kernel computes it (num_lines lines, direct optical depth, exp_nonpos, 7-tap
+// instrument profile), the convolved profiles multiplied in the given order into s_a[0, n_u).  Absorber b is
+// (abs_z[b], abs_nhi[b]); a NaN z is no absorber.  s_raw holds NTHREADS + 6 doubles, s_mult MAX_LINES.  All NTHREADS
+// threads call it; s_a is complete when it returns.  reconstruct_kernel and draw_spectra_kernel both build it here.
+__device__ __forceinline__ void window_absorption(double* s_a, double* s_raw, double* s_mult, int n_u,
+                                                  const double* wl_first, double lo, double hi, double pixel_spacing,
+                                                  int num_lines, int num_absorbers, const double* abs_z,
+                                                  const double* abs_nhi) {
+  const int tid = threadIdx.x;
+  for (int i = tid; i < n_u; i += NTHREADS) s_a[i] = 1.0;
+  for (int b = 0; b < num_absorbers; ++b) {
+    const double z = abs_z[b];
+    if (z != z) continue;   // NaN: no absorber in this slot
+    const double N = abs_nhi[b];
+    __syncthreads();
+    if (tid < num_lines) s_mult[tid] = line_multiplier(tid, z);
+    for (int i0 = 0; i0 < n_u; i0 += NTHREADS) {
+      __syncthreads();
+      for (int t = tid; t < NTHREADS + 6; t += NTHREADS) {
+        const int p = i0 + t;
+        if (p < n_u + 6) {
+          const double tau = tau_sum_generic(padded_wavelength(p, n_u, wl_first, lo, hi, pixel_spacing), s_mult, 1,
+                                             num_lines);
+          s_raw[t] = exp_nonpos(-N * tau);                              // voigt.c:291
+        }
+      }
+      __syncthreads();
+      const int i = i0 + tid;
+      if (i < n_u) {
+        double acc = 0.0;
+#pragma unroll
+        for (int t = 0; t < 7; ++t) acc = fma(s_raw[tid + t], c_lines.ip[t], acc);   // voigt.c:297-299
+        s_a[i] = s_a[i] * acc;
+      }
+    }
+  }
+  __syncthreads();
+}
+
 // dynamic shared memory of reconstruct_kernel<K> for rows of L_max pixels
 template <int K>
 __host__ __device__ constexpr size_t reconstruct_smem_doubles(int64_t L_max) {
@@ -144,36 +184,9 @@ __global__ void __launch_bounds__(NTHREADS) reconstruct_kernel(const __grid_cons
   const double lo = s_lo, hi = s_hi;
   const double* wl_first = wl + first;
 
-  // 1. absorption on the padded grid (process_qsos.m:168-188; ...meanflux.m:342-351): each absorber's profile as
-  // voigt_batch_kernel computes it, the convolved profiles multiplied in the given order
-  for (int i = tid; i < n_u; i += NTHREADS) s_a[i] = 1.0;
-  for (int b = 0; b < a.num_absorbers; ++b) {
-    const double z = a.absorber_z[(int64_t)q * a.num_absorbers + b];
-    if (z != z) continue;   // NaN: no absorber in this slot
-    const double N = a.absorber_nhi[(int64_t)q * a.num_absorbers + b];
-    __syncthreads();
-    if (tid < a.num_lines) s_mult[tid] = line_multiplier(tid, z);
-    for (int i0 = 0; i0 < n_u; i0 += NTHREADS) {
-      __syncthreads();
-      for (int t = tid; t < NTHREADS + 6; t += NTHREADS) {
-        const int p = i0 + t;
-        if (p < n_u + 6) {
-          const double tau = tau_sum_generic(padded_wavelength(p, n_u, wl_first, lo, hi, a.pixel_spacing), s_mult, 1,
-                                             a.num_lines);
-          s_raw[t] = exp_nonpos(-N * tau);                              // voigt.c:291
-        }
-      }
-      __syncthreads();
-      const int i = i0 + tid;
-      if (i < n_u) {
-        double acc = 0.0;
-#pragma unroll
-        for (int t = 0; t < 7; ++t) acc = fma(s_raw[tid + t], c_lines.ip[t], acc);   // voigt.c:297-299
-        s_a[i] = s_a[i] * acc;
-      }
-    }
-  }
-  __syncthreads();
+  // 1. absorption on the padded grid
+  window_absorption(s_a, s_raw, s_mult, n_u, wl_first, lo, hi, a.pixel_spacing, a.num_lines, a.num_absorbers,
+                    a.absorber_z + (int64_t)q * a.num_absorbers, a.absorber_nhi + (int64_t)q * a.num_absorbers);
 
   // 2. the augmented Gram [B - I | g ; . | sum r^2/d] and sum log d.  Thread tid owns entries tid + NTHREADS m of the
   // augmented upper triangle (entry NAUG: sum log d) and walks the pixels in ascending order.

@@ -474,6 +474,88 @@ int gpdla_reconstruct_device(gpdla_ctx* ctx, int64_t Q, int64_t L_max, const dou
                              const double* z_qsos, int32_t meanflux, int32_t num_absorbers, const double* absorber_z,
                              const double* absorber_nhi, const gpdla_reconstruction* out, void* stream);
 
+/* ---- Draws from the learned model: mock spectra from the prior predictive, or absorbers injected into spectra,
+ * with the truth of every draw ----
+ * Spectra as gpdla_process_qsos takes them (flux_in is read only when injecting).  For quasar q, over the pixels of the
+ * modelled window (min_lambda <= lambda / (1 + z_qso) <= max_lambda, masked ones included), mu~, M~ and om2~ are the
+ * null model exactly as gpdla_reconstruct evaluates it (model 0: that of process_qsos.m, s = 1; model 1: the mean-flux
+ * null model of the multi-DLA path), and a is the product of the absorbers' instrument-convolved profiles on the
+ * padded window grid (params.num_lines lines, optical depth evaluated directly), bit-equal to gpdla_reconstruct's
+ * absorption plane for the same absorbers.  Modes:
+ *   draw    y = a (mu~ + M~ xi + om2~^(1/2) e1) + v^(1/2) e2,  xi ~ N(0, I_k) per quasar, e1, e2 ~ N(0, 1) per pixel:
+ *           an exact draw from the Gaussian whose density the hot path evaluates (log_mvnpdf_low_rank.m).  Pixels
+ *           outside the window are NaN (the model does not define them), pixels past lengths[q] are 0.
+ *   inject  y' = a y + ((1 - a^2) v)^(1/2) e2 on the caller's flux y (the noise variance stays v; where a^2 >= 1 the
+ *           noise term is 0): if y is a draw from the model, y' is one with the absorbers added.  Pixels outside the
+ *           window and past lengths[q] are copied.
+ * Absorbers are either given (from_prior = 0: absorber_z, absorber_nhi [Q x num_absorbers], 0 <= num_absorbers <= 4,
+ * NaN z = none; the conventions and checks of gpdla_reconstruct), or drawn from the model's own prior (from_prior = 1),
+ * discretised on the loaded samples exactly as the evidence integrates over them, with min_z, max_z the used-pixel
+ * range of processing (set_parameters.m:65-73) and z_i = min_z + (max_z - min_z) offset_i rounded as map_z_dlas:
+ *   model 0   one DLA with probability exp(log_prior_dla) (process_qsos.m:122-131, from the prior catalogue), at a
+ *             uniformly drawn sample i: (z_i, nhi_samples[i]).  Its z is bit-equal to the z processing gives sample i.
+ *   model 1   no DLA, sub-DLA or j = 1..max_dlas DLAs with the priors of ...meanflux.m:190-216.  A sub-DLA is a
+ *             uniform sample i at (z_i, lls_nhi_samples[i]); j DLAs are j i.i.d. uniform samples, the whole set
+ *             redrawn (up to 64 attempts) until every z gap is >= kms_to_z(3000), the separation filter of the level
+ *             evidence; after 64 failures the quasar is flagged (truth_model = -2), never silently changed.  The
+ *             multi-DLA evidence is an importance-sampled estimate (resampled partners, Occam terms), so its posterior
+ *             calibration against these draws is close to, not exactly, an identity.
+ * A quasar without a used pixel gets a NaN flux and absorption row (in both modes and with both sources); with the
+ * prior source so does one whose model probabilities are not finite (no prior quasar below its z), truth_model = -1.
+ * Truth (prior source only; TW = max_dlas for model 1, 1 for model 0):
+ *   truth_model [Q] int32      -2 no separated set, -1 no draw, 0 no absorber, 1 sub-DLA, 1 + j: j DLAs
+ *   truth_inds [Q x TW] int64  0-based sample indices in the caller's sample order, -1 for an empty slot
+ *   truth_z, truth_log_nhi [Q x TW]  NaN for an empty slot; log_nhi_samples[i] for a DLA, log10(lls_nhi_samples[i]) for
+ *                              a sub-DLA (the context holds no log copy of the sub-DLA samples)
+ * Absorbers are listed in ascending z (ties in slot order), the rank order of the multi-DLA posterior entries.
+ * Random numbers: Philox4x32-10 (10 rounds, multipliers 0xD2511F53 / 0xCD9E8D57, Weyl constants 0x9E3779B9 /
+ * 0xBB67AE85; the bits of curand_Philox4x32_10), key = seed (low word first), counter = (element, stream, g_lo, g_hi)
+ * with g = first_quasar + q, the quasar's index in the whole catalogue.  A draw therefore depends on (seed, g, stream,
+ * element) only -- not on the batch split, grid or GPU count: shards with their first_quasar draw the bits of the
+ * whole.  The output words r.x..r.w make W0 = r.y:r.x and W1 = r.w:r.z (64 bits each).  Layout:
+ *   stream 0, element 0                   the model choice u = ((W0 >> 11) + 0.5) 2^-53: the first model m with
+ *                                         u < sum_{<= m} p, else the last
+ *   stream 1, element 4 attempt + slot    a sample index __umul64hi(W0, S)
+ *   stream 2, element c                   latent xi_2c, xi_2c+1
+ *   stream 3, element i (pixel in row)    e1, e2
+ * Normals are Box-Muller on the uniforms of W0 and W1: r = sqrt(-2 log u0), r cospi(2 u1), r sinpi(2 u1).  This layout
+ * changes only together with the test oracle (oracle/draw_spectra_oracle.py).
+ * Options: model 0 or 1; max_dlas 1..4 (model 1); inject 0/1; from_prior 0/1; first_quasar >= 0.  Outputs: flux
+ * [Q x L_max] (required), absorption [Q x L_max] (nullable, NaN outside the window and past lengths[q]) and, with
+ * from_prior, the four truth arrays (required).  GPDLA_ERR_STATE without a model, and with from_prior also without
+ * samples and prior, and for model 1 without the sub-DLA samples.  GPDLA_ERR_INVALID: flux_in NULL when injecting,
+ * given absorbers with from_prior, first_quasar < 0, a truth pointer NULL with from_prior, and the checks of
+ * gpdla_reconstruct; all before any CUDA call.  k = 10, 20, 40 (else GPDLA_ERR_UNSUPPORTED), L_max bounded by one
+ * CTA's shared memory (about 20 000 pixels).  No atomics: repeated calls give the same bits, and the host entry those
+ * of the _device entry, which takes device arrays and is asynchronous on `stream`. */
+typedef struct {
+  uint64_t seed;
+  int64_t first_quasar;
+  int32_t model;
+  int32_t max_dlas;
+  int32_t inject;
+  int32_t from_prior;
+  int32_t num_absorbers;
+  int32_t reserved;
+  const double* absorber_z;
+  const double* absorber_nhi;
+} gpdla_draw_options;
+typedef struct {
+  double* flux;
+  double* absorption;
+  int32_t* truth_model;
+  int64_t* truth_inds;
+  double* truth_z;
+  double* truth_log_nhi;
+} gpdla_draw_outputs;
+int gpdla_draw_spectra(gpdla_ctx* ctx, int64_t Q, int64_t L_max, const double* wavelengths, const double* flux_in,
+                       const double* noise_variance, const uint8_t* pixel_mask, const int32_t* lengths,
+                       const double* z_qsos, const gpdla_draw_options* options, const gpdla_draw_outputs* out);
+int gpdla_draw_spectra_device(gpdla_ctx* ctx, int64_t Q, int64_t L_max, const double* wavelengths,
+                              const double* flux_in, const double* noise_variance, const uint8_t* pixel_mask,
+                              const int32_t* lengths, const double* z_qsos, const gpdla_draw_options* options,
+                              const gpdla_draw_outputs* out, void* stream);
+
 /* voigt.c:253-304: profile has num_points - 6 entries.  Host buffers; runs on the current device. */
 int gpdla_voigt(const double* lambdas, int64_t num_points, double z, double N, int32_t num_lines, double* profile);
 /* Batched, device buffers: profile[s, :] = voigt(lambdas, z[s], N[s], num_lines), [S x (num_points-6)] */
