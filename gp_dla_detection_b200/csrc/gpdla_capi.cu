@@ -1497,6 +1497,26 @@ int gpdla_preload_qsos(int64_t Q, int64_t L_in, const double* flux, const double
   return rc;
 }
 
+// objective_kernel keeps one spectrum's pixel arrays in shared memory, so the grid length is bounded by the device's
+// opt-in limit.  The check runs before any allocation, upload or launch, and reports P and the largest P that fits
+// instead of a failed cudaFuncSetAttribute.
+static int objective_fits(const char* fn, int32_t num_pixels, int32_t k) {
+  size_t smem = 0, smem0 = 0, smem1 = 0;
+  GPDLA_FOR_RANK(k, (smem = objective_smem_bytes<K>(num_pixels), smem0 = objective_smem_bytes<K>(0),
+                     smem1 = objective_smem_bytes<K>(1)));
+  int dev = 0, optin = 0;
+  CUDA_TRY(cudaGetDevice(&dev), g_err);
+  CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev), g_err);
+  if (smem > (size_t)optin) {
+    const size_t max_pixels = (size_t)optin > smem0 ? ((size_t)optin - smem0) / (smem1 - smem0) : 0;
+    g_err = std::string(fn) + ": num_pixels = " + std::to_string(num_pixels) + " needs " + std::to_string(smem) +
+            " bytes of shared memory at k = " + std::to_string(k) + ", more than the device's " + std::to_string(optin) +
+            " (at most " + std::to_string(max_pixels) + " pixels)";
+    return GPDLA_ERR_INVALID;
+  }
+  return GPDLA_OK;
+}
+
 int gpdla_objective_lyseries_device(int64_t num_quasars, int32_t num_pixels, int32_t k, const double* centered_rest_fluxes,
                                     const double* lya_1pzs, const double* rest_noise_variances, int32_t num_forest_lines,
                                     const double* all_transition_wavelengths, const double* all_oscillator_strengths,
@@ -1511,6 +1531,7 @@ int gpdla_objective_lyseries_device(int64_t num_quasars, int32_t num_pixels, int
     g_err = "gpdla_objective_device: rank k=" + std::to_string(k) + " not compiled in (available: 10, 20, 40)";
     return GPDLA_ERR_UNSUPPORTED;
   }
+  if (int rc = objective_fits("gpdla_objective_device", num_pixels, k)) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   ObjectiveArgs a;
   memset(&a, 0, sizeof a);
@@ -1537,6 +1558,8 @@ int gpdla_objective_lyseries(int64_t num_quasars, int32_t num_pixels, int32_t k,
                              const double* all_transition_wavelengths, const double* all_oscillator_strengths, const double* x,
                              double* f, double* g) {
   if (num_quasars < 0 || num_pixels < 1 || k < 1 || !x || !f || !g) { g_err = "gpdla_objective: invalid arguments"; return GPDLA_ERR_INVALID; }
+  if (rank_supported(k))                          // before the uploads (the device entry reports an unsupported rank)
+    if (int rc = objective_fits("gpdla_objective", num_pixels, k)) return rc;
   const size_t NP = (size_t)num_quasars * num_pixels, nx = (size_t)num_pixels * (k + 1) + 3;
   double* base = nullptr;
   CUDA_TRY(cudaMalloc(&base, (3 * NP + 2 * nx + 2) * sizeof(double)), g_err);

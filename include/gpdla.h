@@ -207,7 +207,9 @@ int gpdla_preload_qsos_device(int64_t Q, int64_t L_in, const double* flux, const
  * (objective.m:3-6), including the Kim et al. priors on tau_0 and beta (:59-71).  The three data matrices are
  * centered_rest_fluxes, lya_1pzs, rest_noise_variances of learn_qso_model.m:36-75, [num_quasars x num_pixels]
  * row-major, NaN in centered_rest_fluxes = pixel not observed (objective.m:42).  g has the layout of x.
- * Context-free; the _device entry (device pointers for data, x, f, g) is asynchronous on `stream`. */
+ * Context-free; the _device entry (device pointers for data, x, f, g) is asynchronous on `stream`.  A spectrum's pixel
+ * arrays live in shared memory (about 20 bytes per pixel): a num_pixels beyond the device's opt-in limit (near 9 700 at
+ * k = 40 on 227 KB) returns GPDLA_ERR_INVALID before anything is allocated or launched. */
 /* The Lyman-series variant the multi-DLA model is trained with: multi_dlas/objective_lyseries.m:13-87 +
  * multi_dlas/spectrum_loss_lyseries.m:14-91.  Same x, data matrices and outputs; the effective optical depth sums the
  * first num_forest_lines series members (all_transition_wavelengths, all_oscillator_strengths of
